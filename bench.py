@@ -2,6 +2,7 @@
 """Benchmark of the batched SATEnv hot path (BASELINE.json metric: SATEnv env-steps/s, uf100-430).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -29,6 +30,7 @@ from pathlib import Path
 ROOT = Path(__file__).resolve().parent
 if str(ROOT) not in sys.path:
     sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (it may be read-only)
 
 METRIC = "SATEnv env-steps/s, uf100-430, 1/2/4/8 B200; achieved HBM GB/s vs peak"
 UNIT = "env-steps/s"
@@ -44,6 +46,7 @@ WORKLOADS = {
 MAX_STEPS = 512          # configs/MAPPO_CONFIG.yaml:14
 SEED = 42                # configs/MAPPO_CONFIG.yaml:6
 ACTION_CYCLE = 64        # pre-generated action batches, cycled
+DUMP_BYTES = 60 * 10**6  # --dump-outputs: array bytes written, under 64 MB with the .npy headers
 
 
 def _load_synth():
@@ -290,6 +293,28 @@ def _time_steps(torch, fn, count):
     return e0.elapsed_time(e1)
 
 
+def dump_step_outputs(out, directory, row=None):
+    """Write the arrays one rollout step returned -- ``out`` of ``VecSATEnv.step``, or row ``row`` of the
+    ``[K, B, ...]`` outputs of ``VecSATEnv.steps`` -- as ``directory/<name>.npy`` in float32 (every value is
+    float32 or a small integer, so the cast is exact).  When they exceed DUMP_BYTES together, the same fixed,
+    seeded sample of env rows is taken from each; ``env_index.npy`` lists the rows written."""
+    import numpy as np
+    import torch
+    arrays = {k: (v if row is None else v[row]) for k, v in out.items()     # "_block": storage behind the views
+              if isinstance(v, torch.Tensor) and not k.startswith("_")}
+    B = arrays["reward"].shape[0]
+    bytes_per_env = sum(4 * a[0].numel() for a in arrays.values()) + 8
+    rows = np.arange(B)
+    if bytes_per_env * B > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(B, DUMP_BYTES // bytes_per_env, replace=False))
+    idx = torch.from_numpy(rows).to(arrays["reward"].device)
+    directory = Path(directory)
+    directory.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(directory / f"{name}.npy", a.index_select(0, idx).float().cpu().numpy())
+    np.save(directory / "env_index.npy", rows.astype(np.float64))
+
+
 def main_ours(args):
     import torch
     import torch.distributed as dist
@@ -366,12 +391,20 @@ def main_ours(args):
         sampler.start()
 
     # ---- device-resident throughput: `value` -------------------------------------------------
-    # bring the GPU to its steady clocks first (>= 60 ms of steps), then the W warm-up steps the caller asked for
+    # bring the GPU to its steady clocks first (>= 60 ms of steps), then the W warm-up steps the caller asked for.
+    # The clock warm-up runs as many steps as fit its wall-clock window, so the env state and the rng chain are
+    # put back afterwards (in place: the step binds their addresses): what the timed steps compute depends on
+    # the arguments alone.
+    state0, chain0, cur0 = vec.state.clone(), vec.keys._bufs.clone(), vec.keys._cur
     t_pre = time.perf_counter()
     while time.perf_counter() - t_pre < 0.06:
         for i in range(8):
             vec.step(actions[i])
         torch.cuda.synchronize()
+    vec.state.copy_(state0)
+    vec.keys._bufs.copy_(chain0)
+    vec.keys._cur = cur0
+    del state0, chain0
     for i in range(W):
         vec.step(actions[i % ACTION_CYCLE])
     torch.cuda.synchronize()
@@ -435,6 +468,11 @@ def main_ours(args):
     barrier()
     ms = ev0.elapsed_time(ev1)
     resets_timed = int(reset_counter.item())
+    if args.dump_outputs and rank == 0:
+        if mode == "multi":         # the last launch wrote rows 0 .. (K mod G or G) - 1
+            dump_step_outputs(multi_out, args.dump_outputs, row=(K % G or G) - 1)
+        else:
+            dump_step_outputs(vec.out, args.dump_outputs)
     launches = K if mode != "multi" else (K // G + (1 if K % G else 0))    # fused step launches in the timed region
 
     # ---- dominant kernel alone (roofline): K launches of the same fused step, back to back ---------------
@@ -906,7 +944,16 @@ def parse_args(argv=None):
                     help="debug: single process, but own the env shard of RANK out of WORLD")
     ap.add_argument("--watchdog", type=int, default=420,
                     help="seconds after which all thread stacks are dumped to stderr and the process exits")
-    return ap.parse_args(argv)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last one (obs, reward, done, solved, "
+                         "num_unsatisfied, episode_step; rank 0's envs) as DIR/<name>.npy in float32; above 64 MB "
+                         "a fixed, seeded sample of env rows, listed in DIR/env_index.npy")
+    args = ap.parse_args(argv)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
 
 
 def _guard_stdout():

@@ -1,7 +1,7 @@
 import sys
 from pathlib import Path
 import torch
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, str(Path(__file__).resolve().parent.parent))
 import marl_sat_b200 as M
 from marl_sat_b200 import _lib
 lib = _lib.load()
