@@ -107,6 +107,19 @@ int msat_reset(const msat_plan* plan, const void* bank, int32_t num_problems,
                const int32_t* problem_idx, const uint32_t* keys,
                uint32_t* state, int32_t* obs, int32_t num_envs, void* stream);
 
+/* Inverse of msat_export_state: packed states from reference-shaped leaves (env:13-24).
+ *   problem_idx int32[B] (clamped into [0, num_problems), as msat_reset does);
+ *   variable_assignments int32[B,n] (0/1; nonzero reads as 1);
+ *   step int32[B] (NULL = 0, stored verbatim); done uint8[B] (NULL = 0, nonzero = done)
+ * clauses_satisfied_status, num_unsatisfied (and an incremental plan's true-literal counts)
+ * are recomputed from the bank record; obs (NULL = skip) as msat_get_obs of the result.
+ * For warm starts, fixed starting assignments and resuming from a checkpoint: the reset path of
+ * the env kernel with the assignment read from memory instead of drawn from a key. */
+int msat_import_state(const msat_plan* plan, const void* bank, int32_t num_problems,
+                      const int32_t* problem_idx, const int32_t* variable_assignments,
+                      const int32_t* step, const uint8_t* done,
+                      uint32_t* state_out, int32_t* obs, int32_t num_envs, void* stream);
+
 /* Replaces `jax.vmap(SATEnv.step_env)` (env:225-284) and, with auto_reset != 0,
  * the reset-and-select of the rollout loop (learner:422-464) in the same launch.
  *   actions        int32 [B, A] (mode 0) or [B, A, V] (mode 1)

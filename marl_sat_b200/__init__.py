@@ -13,7 +13,8 @@ _lib.load()   # fail loudly when the CUDA library is missing
 from .env import FormulaBank, SATEnv, SATState, create_agent_groups   # noqa: E402
 from .gae import (advantage_stats, allreduce_stats, calculate_gae, mean_std_from_stats,  # noqa: E402
                   normalize_advantages)
-from .rollout import RolloutBuffer, RolloutKeys, VecSATEnv, derive_env_keys, prng_key, shard_range  # noqa: E402
+from .rollout import (RolloutBuffer, RolloutKeys, VecSATEnv, derive_env_keys, merge_state_dicts,  # noqa: E402
+                      prng_key, shard_range)
 from .wrapper import GNNWrapperState, SATDataWrapper  # noqa: E402
 from .features import (GNNInput, StaticGraph, dynamic_features, flip_gains, gnn_input_from_state,  # noqa: E402
                        static_graph)
@@ -22,7 +23,8 @@ from .evaluate import evaluate_policy  # noqa: E402
 from . import dimacs  # noqa: E402
 
 __all__ = ["SATEnv", "SATState", "FormulaBank", "create_agent_groups", "SATDataWrapper", "GNNWrapperState",
-           "VecSATEnv", "RolloutBuffer", "RolloutKeys", "derive_env_keys", "shard_range", "prng_key", "calculate_gae",
+           "VecSATEnv", "RolloutBuffer", "RolloutKeys", "derive_env_keys", "merge_state_dicts", "shard_range",
+           "prng_key", "calculate_gae",
            "advantage_stats", "normalize_advantages", "allreduce_stats", "mean_std_from_stats", "metrics_from_sums", "GNNInput", "StaticGraph", "static_graph", "dynamic_features",
            "gnn_input_from_state", "flip_gains", "rollout_metrics", "rollout_metric_sums", "evaluate_policy", "dimacs"]
 __version__ = "0.1.0"

@@ -41,6 +41,7 @@ SIGNATURES = {
     "msat_plan_dims": (C.c_int, [_p, C.POINTER(Dims)]),
     "msat_compile_bank": (C.c_int, [_p, _p, _i32, _p, _p]),
     "msat_reset": (C.c_int, [_p, _p, _i32, _p, _p, _p, _p, _i32, _p]),
+    "msat_import_state": (C.c_int, [_p, _p, _i32, _p, _p, _p, _p, _p, _p, _i32, _p]),
     "msat_plan_set_reward": (C.c_int, [_p, _i32, _f64, _f64, _f64]),
     "msat_tune": (C.c_int, [C.c_char_p, _i32]),
     "msat_plan_set_reset_counter": (C.c_int, [_p, _p]),

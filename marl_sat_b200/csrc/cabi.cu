@@ -284,6 +284,19 @@ int msat_reset(const msat_plan* plan, const void* bank, int32_t P, const int32_t
     return cuda_rc(launch_env(plan, MODE_RESET, a, (cudaStream_t)stream));
 }
 
+int msat_import_state(const msat_plan* plan, const void* bank, int32_t P, const int32_t* problem_idx,
+                      const int32_t* variable_assignments, const int32_t* step, const uint8_t* done, uint32_t* state_out,
+                      int32_t* obs, int32_t B, void* stream) {
+    if (!plan || B < 0 || P <= 0) return MSAT_EINVAL;
+    if (B > 0 && (!bank || !problem_idx || !variable_assignments || !state_out)) return MSAT_EINVAL;
+    if (!aligned(bank, 128) || !aligned(state_out, 16) || !aligned(obs, 16)) return MSAT_EALIGN;
+    EnvArgs a{};
+    a.bank = static_cast<const uint8_t*>(bank); a.P = P;
+    a.state_out = state_out; a.prob_idx = problem_idx; a.obs = obs; a.B = B;
+    a.assign_in = variable_assignments; a.step_in = step; a.done_in = done;
+    return cuda_rc(launch_env(plan, MODE_IMPORT, a, (cudaStream_t)stream));
+}
+
 int msat_step(const msat_plan* plan, const void* bank, int32_t P, const uint32_t* state_in, uint32_t* state_out,
               const int32_t* actions, int32_t auto_reset, const int32_t* new_problem_idx, const uint32_t* reset_keys,
               int32_t* obs, float* reward, int32_t reward_cols, uint8_t* done, int32_t done_cols, uint8_t* solved,

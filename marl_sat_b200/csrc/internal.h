@@ -102,9 +102,15 @@ struct EnvArgs {
     int32_t* newly_sat;         // optional int32[(K,) B]: clauses satisfied now that were not before the step
     unsigned long long* reset_count;   // optional device counter: += 1 for every auto-reset (msat_plan_set_reset_counter)
     int obs_i8;                 // `obs` points to int8 elements (msat_plan_set_obs_dtype)
+    // state import (msat_import_state): reference-shaped leaves in place of the reset's Threefry draw;
+    // assignment int32[B, n] (nonzero = 1), step int32[B] and done uint8[B] (NULL = 0)
+    const int32_t* assign_in;
+    const int32_t* step_in;
+    const uint8_t* done_in;
 };
 
-enum EnvMode { MODE_RESET = 0, MODE_STEP = 1, MODE_OBS = 2 };
+// MODE_IMPORT: the reset path with the assignment, step and done flag read from memory
+enum EnvMode { MODE_RESET = 0, MODE_STEP = 1, MODE_OBS = 2, MODE_IMPORT = 3 };
 
 extern int g_gae_force_plain;   // gae.cu; msat_tune("gae_plain", 1)
 extern int g_gae_variant;       // gae.cu; msat_tune("gae_variant", v)

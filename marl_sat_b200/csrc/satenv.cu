@@ -441,6 +441,32 @@ __device__ __forceinline__ void threefry_assign(const Dims& d, uint32_t k0, uint
     }
 }
 
+// State import: pack a given int32[n] assignment (nonzero reads as 1) into the assignment words.  Lane v % 32 (v % 16
+// in half-warp groups) loads variable v, so consecutive lanes read consecutive ints, and one ballot makes a word
+// (half a word for GS = 16, stored as a 16-bit piece: little endian, as the half-warp status words).  Every word,
+// including the bits past n, is written in full.
+template <int GS>
+__device__ __forceinline__ void load_assign(const Dims& d, const int32_t* __restrict__ src, uint32_t* assign, int gt) {
+    if constexpr (GS < 32) {
+        uint16_t* piece = reinterpret_cast<uint16_t*>(assign);
+        const uint32_t sh = subwarp_shift<16>();
+        const uint32_t mask = subwarp_mask<16>();
+        for (int r = 0; r < 2 * d.aw; ++r) {
+            const int v = 16 * r + gt;
+            const bool bit = v < d.n && src[v] != 0;
+            const uint32_t bits = (__ballot_sync(mask, bit) >> sh) & 0xFFFFu;
+            if (gt == 0) piece[r] = (uint16_t)bits;
+        }
+    } else {
+        const int lane = gt & 31;
+        for (int w = gt >> 5; w < d.aw; w += GS / 32) {
+            const int v = 32 * w + lane;
+            const uint32_t word = __ballot_sync(0xffffffffu, v < d.n && src[v] != 0);
+            if (lane == 0) assign[w] = word;
+        }
+    }
+}
+
 // Apply all agents' flips simultaneously (env:233-250) on the packed assignment in shared memory.
 // has_pre: the caller already holds act[gt] (mode 0) in `pre` (loaded early, next to the state record).
 template <int GS>
@@ -732,11 +758,13 @@ __device__ __forceinline__ void rng_advance(uint32_t& r0, uint32_t& r1) {
 // !OBS = literal block only (or, INCR, the CSR occurrence lists), optional GNN-input outputs.
 // MULTI = K steps per launch (msat_rollout_steps); INCR = incremental clause update (step launches of a plan
 // with MSAT_CLAUSES_INCREMENTAL that write no observations).
+// MODE_IMPORT (msat_import_state) is the reset with the assignment, step and done flag taken from memory.
 // =====================================================================================
 template <int GS, int MODE, bool OBS, bool MULTI, bool INCR>
 __global__ void __launch_bounds__(kCtaThreads, (MULTI || !OBS) ? 4 : 8) env_kernel(const Dims d, const EnvArgs a) {
     extern __shared__ __align__(128) uint8_t smem_raw[];
     constexpr int NG = kCtaThreads / GS;
+    constexpr bool FRESH = MODE == MODE_RESET || MODE == MODE_IMPORT;    // builds a state instead of reading one
     const int gid = threadIdx.x / GS, gt = threadIdx.x % GS;
     const int e = blockIdx.x * NG + gid;
     const GroupLayout& L = a.L;
@@ -792,11 +820,10 @@ __global__ void __launch_bounds__(kCtaThreads, (MULTI || !OBS) ? 4 : 8) env_kern
     // are issued back to back before anything consumes them, so their latencies overlap each other and the
     // shared-memory set-up below instead of adding up.
     // state records are multiples of 16 bytes (state_words % 4 == 0) in a 16-byte aligned array
-    const uint4* sin = (MODE == MODE_RESET) ? nullptr
-                                            : reinterpret_cast<const uint4*>(a.state_in + (size_t)e * d.state_words);
+    const uint4* sin = FRESH ? nullptr : reinterpret_cast<const uint4*>(a.state_in + (size_t)e * d.state_words);
     const int sw4 = d.state_words >> 2;
     uint4 s0 = make_uint4(0u, 0u, 0u, 0u);
-    if (MODE != MODE_RESET && gt < sw4) s0 = sin[gt];
+    if (!FRESH && gt < sw4) s0 = sin[gt];
     if constexpr (GS < 32) {            // issue-bound half-warp groups: no registers to spare for the overlap
         if (gt < sw4) reinterpret_cast<uint4*>(st)[gt] = s0;
     }
@@ -811,7 +838,7 @@ __global__ void __launch_bounds__(kCtaThreads, (MULTI || !OBS) ? 4 : 8) env_kern
     if constexpr (GS >= 32) {
         if (gt < sw4) reinterpret_cast<uint4*>(st)[gt] = s0;
     }
-    if (MODE != MODE_RESET) {
+    if (!FRESH) {
 #pragma unroll 1
         for (int i = gt + GS; i < sw4; i += GS) reinterpret_cast<uint4*>(st)[i] = sin[i];
     } else {
@@ -823,11 +850,14 @@ __global__ void __launch_bounds__(kCtaThreads, (MULTI || !OBS) ? 4 : 8) env_kern
     // Every thread keeps its own copy of the scalar state fields in registers from here on: thread 0 rewrites
     // them in shared memory only after the last step, and a warp that read `step` from shared memory after
     // such a write would disagree with the others about `done` and wait at a group barrier nobody else reaches.
-    int step_cur = (MODE == MODE_RESET) ? 0 : (int)st_tail[ST_STEP];
-    int nunsat_prev = (MODE == MODE_RESET) ? 0 : (int)st_tail[ST_NUNSAT];
-    uint32_t flags = (MODE == MODE_RESET) ? 0u : st_tail[ST_FLAGS];
+    // an imported step is stored verbatim: states exported after stepping past `done` carry step >= max_steps
+    int step_cur = (MODE == MODE_RESET) ? 0
+                 : (MODE == MODE_IMPORT) ? (a.step_in ? a.step_in[e] : 0) : (int)st_tail[ST_STEP];
+    int nunsat_prev = FRESH ? 0 : (int)st_tail[ST_NUNSAT];
+    uint32_t flags = (MODE == MODE_RESET) ? 0u
+                   : (MODE == MODE_IMPORT) ? ((a.done_in && a.done_in[e]) ? 1u : 0u) : st_tail[ST_FLAGS];
     int pidx;
-    if (MODE == MODE_RESET) pidx = a.prob_idx[e];
+    if (FRESH) pidx = a.prob_idx[e];
     else pidx = (int)st_tail[ST_PIDX];
     pidx = pidx < 0 ? 0 : (pidx >= a.P ? a.P - 1 : pidx);
     int loaded_pidx = -1;           // formula whose block sits in the record slot ...
@@ -876,6 +906,8 @@ __global__ void __launch_bounds__(kCtaThreads, (MULTI || !OBS) ? 4 : 8) env_kern
         // ---- new assignment while the record is in flight ----
         if (MODE == MODE_RESET) {
             threefry_assign<GS>(d, a.keys[2 * (size_t)e], a.keys[2 * (size_t)e + 1], st, gt);
+        } else if (MODE == MODE_IMPORT) {
+            load_assign<GS>(d, a.assign_in + (size_t)e * d.n, st, gt);
         } else if (MODE == MODE_STEP) {
             if (INCR) {
                 if (need_csr) {
@@ -1056,12 +1088,14 @@ static cudaError_t launch_env_gs(const msat_plan* plan, EnvMode mode, const EnvA
     const int groups = kCtaThreads / GS;
     const int grid = (a.B + groups - 1) / groups;
     if (grid == 0) return cudaSuccess;
+    // every instantiation a launch with this (GS, OBS) can select: the shared-memory opt-in below covers them all.
     // incremental clause update: step launches without observations on a plan that carries the counts
-    constexpr int kFns = OBS ? 4 : 6;
-    const void* fns[6] = {(const void*)env_kernel<GS, MODE_RESET, OBS, false, false>,
+    constexpr int kFns = OBS ? 5 : 7;
+    const void* fns[7] = {(const void*)env_kernel<GS, MODE_RESET, OBS, false, false>,
                           (const void*)env_kernel<GS, MODE_STEP, OBS, false, false>,
                           (const void*)env_kernel<GS, MODE_OBS, OBS, false, false>,
                           (const void*)env_kernel<GS, MODE_STEP, OBS, true, false>,
+                          (const void*)env_kernel<GS, MODE_IMPORT, OBS, false, false>,
                           OBS ? nullptr : (const void*)env_kernel<GS, MODE_STEP, false, false, true>,
                           OBS ? nullptr : (const void*)env_kernel<GS, MODE_STEP, false, true, true>};
     const bool multi = mode == MODE_STEP && a.num_steps > 1;
@@ -1081,7 +1115,8 @@ static cudaError_t launch_env_gs(const msat_plan* plan, EnvMode mode, const EnvA
             plan->prepared_devices.fetch_or(bit, std::memory_order_release);
         }
     }
-    const void* fn = incr ? fns[multi ? 5 : 4] : fns[multi ? 3 : (mode == MODE_RESET ? 0 : (mode == MODE_STEP ? 1 : 2))];
+    const void* fn = incr ? fns[multi ? 6 : 5]
+                          : fns[multi ? 3 : (mode == MODE_RESET ? 0 : (mode == MODE_STEP ? 1 : (mode == MODE_OBS ? 2 : 4)))];
     Dims d = plan->d;
     EnvArgs args = a;
     void* params[] = {&d, &args};

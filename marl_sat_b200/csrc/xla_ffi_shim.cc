@@ -49,6 +49,17 @@ ffi::Error Reset(cudaStream_t s, int64_t plan, int64_t num_problems, ffi::Buffer
                   "msat_reset");
 }
 
+// inverse of ExportState: packed states (+ observations) from reference-shaped leaves; step / done may be given as
+// zeros (msat_import_state treats them like NULL)
+ffi::Error ImportState(cudaStream_t s, int64_t plan, int64_t num_problems, ffi::Buffer<ffi::U8> bank,
+                       ffi::Buffer<ffi::S32> problem_idx, ffi::Buffer<ffi::S32> assignments, ffi::Buffer<ffi::S32> step,
+                       ffi::Buffer<ffi::U8> done, ffi::ResultBuffer<ffi::U32> state, ffi::ResultBuffer<ffi::S32> obs) {
+    return status(msat_import_state(plan_of(plan), bank.typed_data(), (int32_t)num_problems, problem_idx.typed_data(),
+                                    assignments.typed_data(), step.typed_data(), done.typed_data(), state->typed_data(),
+                                    obs->typed_data(), dim0(problem_idx.dimensions()), s),
+                  "msat_import_state");
+}
+
 ffi::Error Step(cudaStream_t s, int64_t plan, int64_t num_problems, int64_t auto_reset, ffi::Buffer<ffi::U8> bank,
                 ffi::Buffer<ffi::U32> state_in, ffi::Buffer<ffi::S32> actions, ffi::Buffer<ffi::S32> new_problem_idx,
                 ffi::Buffer<ffi::U32> reset_keys, ffi::ResultBuffer<ffi::U32> state, ffi::ResultBuffer<ffi::S32> obs,
@@ -222,6 +233,10 @@ XLA_FFI_DEFINE_HANDLER_SYMBOL(MsatCompileBank, CompileBank,
 XLA_FFI_DEFINE_HANDLER_SYMBOL(MsatReset, Reset,
     ffi::Ffi::Bind().Ctx<Stream>().Attr<int64_t>("plan").Attr<int64_t>("num_problems")
         .Arg<In<ffi::U8>>().Arg<In<ffi::S32>>().Arg<In<ffi::U32>>().Ret<Out<ffi::U32>>().Ret<Out<ffi::S32>>());
+XLA_FFI_DEFINE_HANDLER_SYMBOL(MsatImportState, ImportState,
+    ffi::Ffi::Bind().Ctx<Stream>().Attr<int64_t>("plan").Attr<int64_t>("num_problems")
+        .Arg<In<ffi::U8>>().Arg<In<ffi::S32>>().Arg<In<ffi::S32>>().Arg<In<ffi::S32>>().Arg<In<ffi::U8>>()
+        .Ret<Out<ffi::U32>>().Ret<Out<ffi::S32>>());
 XLA_FFI_DEFINE_HANDLER_SYMBOL(MsatStep, Step,
     ffi::Ffi::Bind().Ctx<Stream>().Attr<int64_t>("plan").Attr<int64_t>("num_problems").Attr<int64_t>("auto_reset")
         .Arg<In<ffi::U8>>().Arg<In<ffi::U32>>().Arg<In<ffi::S32>>().Arg<In<ffi::S32>>().Arg<In<ffi::U32>>()

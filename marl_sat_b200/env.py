@@ -354,6 +354,97 @@ class SATEnv:
                                         _ptr(keys), _ptr(packed), _ptr(obs), B, _stream_ptr(dev)), "msat_reset")
         return obs, SATState(self, bank, packed, True)
 
+    # ------------------------------------------------------------------ state import
+    def reset_with_assignment(self, problem_clauses: ArrayLike, variable_assignments: ArrayLike,
+                              step: Optional[ArrayLike] = None,
+                              done: Optional[ArrayLike] = None) -> Tuple[Dict[str, torch.Tensor], SATState]:
+        """Counterpart of ``reset(problem_clauses, key)`` (env:158-181) that starts from a given assignment instead
+        of a random one: ``(problem_clauses[m,k], variable_assignments[n])`` or the batched ``[B,m,k]`` / ``[B,n]``.
+        ``step`` / ``done`` (default 0 / False) as in ``import_state``."""
+        self._require_cuda()
+        cl = problem_clauses if isinstance(problem_clauses, torch.Tensor) else torch.as_tensor(np.asarray(problem_clauses))
+        batched = cl.dim() == 3
+        va = torch.as_tensor(np.asarray(variable_assignments)) if not isinstance(variable_assignments, torch.Tensor) \
+            else variable_assignments
+        if not batched:
+            cl, va = cl[None], va.reshape(1, -1)
+            if step is not None:
+                step = torch.as_tensor(step).reshape(1)
+            if done is not None:
+                done = torch.as_tensor(done)
+                done = done.reshape(1) if done.numel() == 1 else done.reshape(1, -1)
+        bank = FormulaBank(self, cl)
+        idx = torch.arange(bank.num_problems, dtype=torch.int32, device=self.device)
+        obs, state = self.import_state(bank, idx, va, step, done)
+        state.batched = batched
+        return self._obs_dict(obs, batched), state
+
+    def import_state(self, bank: FormulaBank, problem_idx: ArrayLike, variable_assignments: ArrayLike,
+                     step: Optional[ArrayLike] = None, done: Optional[ArrayLike] = None, *,
+                     state_out: Optional[torch.Tensor] = None, obs_out: Optional[torch.Tensor] = None,
+                     want_obs: bool = True, validate: bool = True) -> Tuple[Optional[torch.Tensor], SATState]:
+        """Inverse of the ``SATState`` export (``msat_import_state``): packed states of formulas resident in
+        ``bank`` built from reference-shaped leaves (env:13-24), and their observations ``[B,A,D]``.  Mirrors
+        ``reset_from_bank``.
+          variable_assignments  int32 / uint8 / bool ``[B, n]``, values 0 / 1
+          step                  int ``[B]``, default 0; stored as given, also at or past ``max_steps``
+          done                  ``[B]`` or the reference's per-agent ``[B, A]``, default False
+        Clause status, ``num_unsatisfied`` (and an incremental plan's per-clause counts) are recomputed on the
+        device.  ``validate=True`` checks on the host that assignments are 0 / 1, ``step >= 0``, problem indices
+        lie in ``[0, P)`` and ``[B, A]`` done rows are uniform (one device->host sync; ValueError / IndexError).
+        ``validate=False`` enqueues only and can be captured in a CUDA graph: the kernel then clamps problem indices
+        into ``[0, P)``, reads a nonzero assignment as 1 and takes agent 0's done flag."""
+        dev = self._require_cuda()
+        d = bank.plan.dims
+        idx = torch.as_tensor(problem_idx)
+        if idx.dim() != 1:
+            raise ValueError(f"problem_idx must be [B], got {tuple(idx.shape)}")
+        B = int(idx.shape[0])
+        idx = idx.to(device=dev, dtype=torch.int32).contiguous()
+        va = torch.as_tensor(variable_assignments)
+        if va.dtype not in (torch.int32, torch.uint8, torch.bool):
+            raise ValueError(f"variable_assignments must be int32, uint8 or bool, got {va.dtype}")
+        if tuple(va.shape) != (B, d.n):
+            raise ValueError(f"variable_assignments must be [{B}, {d.n}], got {tuple(va.shape)}")
+        va = va.to(device=dev, dtype=torch.int32).contiguous()
+        st = None
+        if step is not None:
+            st = torch.as_tensor(step)
+            if tuple(st.shape) != (B,):
+                raise ValueError(f"step must be [{B}], got {tuple(st.shape)}")
+            st = st.to(device=dev, dtype=torch.int32).contiguous()
+        dn = dn_rows = None
+        if done is not None:
+            dn_rows = torch.as_tensor(done).to(device=dev)
+            if tuple(dn_rows.shape) not in ((B,), (B, d.A)):
+                raise ValueError(f"done must be [{B}] or [{B}, {d.A}], got {tuple(dn_rows.shape)}")
+            dn = ((dn_rows[:, 0] if dn_rows.dim() == 2 else dn_rows) != 0).to(torch.uint8).contiguous()
+        if state_out is not None and tuple(state_out.shape) != (B, d.state_words):
+            raise ValueError(f"state_out must be [{B}, {d.state_words}], got {tuple(state_out.shape)}")
+        if validate and B:
+            zero = torch.zeros((), dtype=torch.int64, device=dev)
+            nz = dn_rows != 0 if dn_rows is not None and dn_rows.dim() == 2 else None
+            lo, hi, bad_assign, min_step, mixed_done = torch.stack([
+                idx.min().long(), idx.max().long(), ((va != 0) & (va != 1)).any().long(),
+                st.min().long() if st is not None else zero,
+                (nz.any(1) != nz.all(1)).any().long() if nz is not None else zero]).tolist()
+            if lo < 0 or hi >= bank.num_problems:
+                raise IndexError(f"problem_idx out of range [0, {bank.num_problems}): min {lo}, max {hi}")
+            if bad_assign:
+                raise ValueError("variable_assignments must hold 0 / 1 values only")
+            if min_step < 0:
+                raise ValueError(f"step must be >= 0, got min {min_step}")
+            if mixed_done:
+                raise ValueError("done [B, A]: every agent of an env must carry the same flag (env:260)")
+        packed = state_out if state_out is not None else torch.empty((B, d.state_words), dtype=torch.int32, device=dev)
+        obs = obs_out
+        if obs is None and want_obs:
+            obs = torch.empty((B, d.A, d.D), dtype=self.obs_dtype, device=dev)
+        _lib.check(self._lib.msat_import_state(bank.plan.handle, _ptr(bank.data), bank.num_problems, _ptr(idx),
+                                               _ptr(va), _ptr(st), _ptr(dn), _ptr(packed), _ptr(obs), B,
+                                               _stream_ptr(dev)), "msat_import_state")
+        return obs, SATState(self, bank, packed, True)
+
     # ------------------------------------------------------------------ step
     def _actions_tensor(self, actions, B: int, dev) -> torch.Tensor:
         if isinstance(actions, dict):                                         # learner:131

@@ -28,7 +28,8 @@ SHIM_PATH = Path(__file__).resolve().parent / "csrc" / "libmarlsat_b200_xla.so"
 
 # handler symbol -> FFI target name
 TARGETS = {
-    "MsatCompileBank": "msat_compile_bank", "MsatReset": "msat_reset", "MsatStep": "msat_step",
+    "MsatCompileBank": "msat_compile_bank", "MsatReset": "msat_reset", "MsatImportState": "msat_import_state",
+    "MsatStep": "msat_step",
     "MsatRolloutSteps": "msat_rollout_steps", "MsatRolloutStepsGnn": "msat_rollout_steps_gnn",
     "MsatGetObs": "msat_get_obs", "MsatExportState": "msat_export_state", "MsatRngChain": "msat_rng_chain",
     "MsatRngSplit2": "msat_rng_split2", "MsatEnvKeys": "msat_env_keys", "MsatGae": "msat_gae",
@@ -62,6 +63,23 @@ def reset(plan_handle: int, dims, bank, num_problems: int, problem_idx, keys):
     B = problem_idx.shape[0]
     call = jffi.ffi_call("msat_reset", (_sds((B, dims.state_words), jnp.uint32), _sds((B, dims.A, dims.D), jnp.int32)))
     return call(bank, problem_idx, keys, plan=np.int64(plan_handle), num_problems=np.int64(num_problems))
+
+
+def import_state(plan_handle: int, dims, bank, num_problems: int, problem_idx, variable_assignments, step=None,
+                 done=None):
+    """Inverse of ``MsatExportState``: packed states from reference-shaped ``SATState`` leaves (env:13-24), e.g. a
+    reference ``reset``'s, a checkpoint's or an edited assignment -> ``(state, obs)``.  ``variable_assignments``
+    [B, n] (0 / 1), ``step`` [B] (default 0, kept as given), ``done`` [B] or [B, A] (default False)."""
+    register()
+    B = problem_idx.shape[0]
+    step = jnp.zeros((B,), jnp.int32) if step is None else jnp.asarray(step, jnp.int32)
+    done = jnp.zeros((B,), jnp.uint8) if done is None else jnp.asarray(done)
+    if done.ndim == 2:
+        done = done[:, 0]
+    call = jffi.ffi_call("msat_import_state", (_sds((B, dims.state_words), jnp.uint32),
+                                               _sds((B, dims.A, dims.D), jnp.int32)))
+    return call(bank, jnp.asarray(problem_idx, jnp.int32), jnp.asarray(variable_assignments, jnp.int32), step,
+                done.astype(jnp.uint8), plan=np.int64(plan_handle), num_problems=np.int64(num_problems))
 
 
 def rollout_steps(plan_handle: int, dims, bank, num_problems: int, state, actions, rng, num_envs_global=None,

@@ -389,6 +389,82 @@ class VecSATEnv:
     def sat_state(self) -> SATState:
         return SATState(self.env, self.bank, self.state, True)
 
+    # ------------------------------------------------------------------ state import / checkpoints
+    def import_state(self, problem_idx, variable_assignments, step=None, done=None,
+                     validate: bool = True) -> Optional[torch.Tensor]:
+        """Put this shard's envs onto the given states (rows in shard order; leaves as ``SATEnv.import_state``) and
+        write the policy input this env emits: ``out["obs"]`` when it is allocated and, with ``gnn_outputs``, the
+        GNN assignment / clause features.  The rng chain is not touched."""
+        out = self.out
+        obs, _ = self.env.import_state(self.bank, problem_idx, variable_assignments, step, done, state_out=self.state,
+                                       obs_out=out["obs"], want_obs=out["obs"] is not None, validate=validate)
+        if self.gnn_outputs:
+            _lib.check(self.env._lib.msat_gnn_dynamic(
+                self.bank.plan.handle, _ptr(self.bank.data), self.bank.num_problems, _ptr(self.state), self.num_envs,
+                _ptr(out["gnn_assignment"]), _ptr(out["gnn_clause_features"]), _stream_ptr(self.state.device)),
+                "msat_gnn_dynamic")
+        return obs
+
+    def _signature(self) -> Dict[str, int]:
+        env = self.env
+        return {"num_vars": env.num_vars, "num_clauses": env.num_clauses, "k": self.bank.k,
+                "num_agents": env.num_agents, "num_problems": self.bank.num_problems}
+
+    def state_dict(self) -> Dict:
+        """Portable checkpoint of this shard (host tensors, ``torch.save``-able): its rows as reference-shaped
+        leaves (``variable_assignments`` [B,n], ``step`` [B], ``done`` [B,A], ``problem_idx`` [B]), the rollout rng
+        chain (``RolloutKeys.chain``, 10 words), ``env_offset``, ``num_envs_global`` and a shape ``signature``.
+        The packed layout never leaves the process, so the checkpoint loads into either clause-update mode, any
+        observation dtype and any later library version.  Synchronises the stream."""
+        st = self.sat_state()
+        return {"variable_assignments": st.variable_assignments.cpu(), "step": st.step.cpu(), "done": st.done.cpu(),
+                "problem_idx": st.problem_idx.cpu(), "rng_chain": self.keys.chain.cpu().clone(),
+                "env_offset": self.env_offset, "num_envs_global": self.num_envs_global, "signature": self._signature()}
+
+    def load_state_dict(self, sd: Dict) -> Optional[torch.Tensor]:
+        """Continue from a checkpoint of ``state_dict``: any dict with this env's signature and global batch size
+        whose rows cover this shard's global range ``[env_offset, env_offset + num_envs)``.  Problem indices and
+        reset keys depend only on (rng, global env index, global batch size) (DESIGN.md section 7), so a world-1
+        checkpoint loads into every rank of a world-N run, and rank checkpoints joined with
+        ``merge_state_dicts`` load into any world size, with the values of an uninterrupted single-device run.
+        Returns the policy input written by ``import_state``."""
+        sig = {k: int(v) for k, v in dict(sd["signature"]).items()}
+        if sig != self._signature():
+            raise ValueError(f"checkpoint signature {sig} does not match this env's {self._signature()}")
+        if int(sd["num_envs_global"]) != self.num_envs_global:
+            raise ValueError(f"checkpoint of {int(sd['num_envs_global'])} envs, this run has {self.num_envs_global}")
+        off, rows = int(sd["env_offset"]), int(sd["variable_assignments"].shape[0])
+        lo = self.env_offset - off
+        if lo < 0 or lo + self.num_envs > rows:
+            raise ValueError(f"checkpoint rows [{off}, {off + rows}) do not cover this shard's "
+                             f"[{self.env_offset}, {self.env_offset + self.num_envs})")
+        rows_of = lambda name: torch.as_tensor(sd[name])[lo:lo + self.num_envs]
+        obs = self.import_state(rows_of("problem_idx"), rows_of("variable_assignments"), rows_of("step"),
+                                rows_of("done"), validate=True)
+        self.keys.chain.copy_(as_u32_tensor(sd["rng_chain"], self.state.device).reshape(10))
+        return obs
+
+
+def merge_state_dicts(dicts) -> Dict:
+    """Join ``VecSATEnv.state_dict()`` checkpoints of adjacent shards of one run into one (rows in ``env_offset``
+    order), e.g. every rank's, which then loads into any world size."""
+    dicts = sorted(dicts, key=lambda sd: int(sd["env_offset"]))
+    first = dicts[0]
+    end = int(first["env_offset"])
+    for sd in dicts:
+        if int(sd["env_offset"]) != end:
+            raise ValueError(f"shards are not adjacent: a gap or overlap at env {end}")
+        if dict(sd["signature"]) != dict(first["signature"]) or int(sd["num_envs_global"]) != int(first["num_envs_global"]):
+            raise ValueError("checkpoints of different runs")
+        if not torch.equal(torch.as_tensor(sd["rng_chain"]), torch.as_tensor(first["rng_chain"])):
+            raise ValueError("checkpoints taken at different rollout steps (rng chains differ)")
+        end += int(sd["variable_assignments"].shape[0])
+    merged = {k: torch.cat([torch.as_tensor(sd[k]) for sd in dicts])
+              for k in ("variable_assignments", "step", "done", "problem_idx")}
+    merged.update(rng_chain=torch.as_tensor(first["rng_chain"]).clone(), env_offset=int(first["env_offset"]),
+                  num_envs_global=int(first["num_envs_global"]), signature=dict(first["signature"]))
+    return merged
+
 
 class RolloutBuffer:
     """``Transition`` storage (learner:358-369,467-478) for T steps of B envs, laid out ``[T, B, ...]`` so
