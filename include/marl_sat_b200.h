@@ -368,6 +368,46 @@ int msat_eval_track(const msat_plan* plan, const uint32_t* state, const uint8_t*
                     int32_t num_envs, uint8_t* ever_solved, int32_t* steps_to_solve, int32_t* solution,
                     void* stream);
 
+/* --- local search ------------------------------------------------------------------------------------ */
+
+/* Batched WalkSAT/SKC with noise p, in place on packed env states (a classical solver next to the env: labels
+ * for a bank, a local-search baseline at an RL flip budget, near-solution starts for msat_import_state).
+ *
+ * Algorithm contract (oracle/walksat.py restates it word for word).  The loop is per env.  Flip iteration t
+ * runs for t = 0 .. max_flips-1 and stops early as soon as num_unsat == 0; an env that is already satisfied on
+ * entry makes 0 flips.  Each iteration does the following:
+ *   1. Random bits.  c = flip_offset + t (uint32); (x0, x1) = threefry2x32(key[b], ctr = (c, 0)).
+ *   2. Clause choice.  U = num_unsat, r = umulhi(x0, U).  The picked clause is the r-th unsatisfied clause
+ *      (0-based) in increasing clause index.
+ *   3. Candidates.  The clause's non-padding literal columns j = 0..k-1, in column order; duplicates stay in
+ *      the list.  nc = their count.  If nc == 0 (an all-padding clause) nothing is flipped, but the iteration
+ *      still counts.
+ *   4. Break counts.  break(v) = the number of distinct clauses that are satisfied now and unsatisfied after
+ *      flipping v alone: a satisfied clause breaks iff all of its true literals are on v and it has no false
+ *      literal on v.  Literal 0 is never true (env:135-144).
+ *   5. Choice of variable.  If some candidate has break 0, the first such candidate (freebie).  Otherwise, if
+ *      (x1 >> 8) < thr with thr = llrint(noise * 2^24), a random walk: candidate ((x1 & 0xFF) * nc) >> 8.
+ *      Otherwise the first candidate with the minimum break.
+ *   6. Flip.  Flip the chosen variable and update the true-literal counts, the status and num_unsat.
+ * A call with max_flips = F1 + F2 gives the same result, bit for bit, as a call with F1 followed by a call with
+ * F2 and flip_offset = F1 on the returned state with the same keys.
+ *
+ *   state     uint32[B, state_words], read and written in place.  The problem index comes from each record
+ *             (clamped into [0, num_problems)).  The call rewrites the assignment words and num_unsatisfied
+ *             (plus the 4-bit true-literal counts on an MSAT_CLAUSES_INCREMENTAL plan); step, the problem index
+ *             and done are left unchanged.
+ *   keys      uint32[B, 2], one Threefry key per env
+ *   solved    uint8[B] (NULL = skip): num_unsat == 0 after the call
+ *   flips     int32[B] (NULL = skip): iterations this call used
+ * MSAT_EINVAL: missing pointers while B > 0, noise outside [0, 1] or NaN, negative max_flips / flip_offset or
+ * flip_offset + max_flips > 2^31 - 1.  MSAT_EALIGN as msat_import_state (bank 128 bytes, state 16 bytes).
+ * MSAT_EUNSUPPORTED: lits_per_clause > 32 or the per-env working set (literal block, var -> clause occurrence
+ * lists, counts and status bits) does not fit in shared memory.  B == 0 returns MSAT_OK without touching the
+ * device. */
+int msat_walksat(const msat_plan* plan, const void* bank, int32_t num_problems,
+                 uint32_t* state, const uint32_t* keys, int32_t max_flips, int32_t flip_offset,
+                 double noise, uint8_t* solved, int32_t* flips, int32_t num_envs, void* stream);
+
 /* Native DIMACS CNF reader (host only; replaces parse_cnf, src/utils/data_parser.py:8-42).  Parses `len`
  * bytes of `text`.  Call once with clauses == NULL to obtain clause_count (rows actually present) and
  * max_width (longest clause, terminating 0 excluded), then again with clauses int32[clause_count,

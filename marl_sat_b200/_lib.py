@@ -74,6 +74,7 @@ SIGNATURES = {
     "msat_dimacs_parse": (C.c_int, [C.c_char_p, C.c_size_t, _i32, C.POINTER(_i32), C.POINTER(_i32), C.POINTER(_i32),
                                     C.POINTER(_i32), _p, _i32]),
     "msat_eval_track": (C.c_int, [_p, _p, _p, _i32, _i32, _p, _p, _p, _p]),
+    "msat_walksat": (C.c_int, [_p, _p, _i32, _p, _p, _i32, _i32, _f64, _p, _p, _i32, _p]),
 }
 
 _lib = None

@@ -297,6 +297,23 @@ int msat_import_state(const msat_plan* plan, const void* bank, int32_t P, const 
     return cuda_rc(launch_env(plan, MODE_IMPORT, a, (cudaStream_t)stream));
 }
 
+int msat_walksat(const msat_plan* plan, const void* bank, int32_t P, uint32_t* state, const uint32_t* keys,
+                 int32_t max_flips, int32_t flip_offset, double noise, uint8_t* solved, int32_t* flips, int32_t B,
+                 void* stream) {
+    if (!plan || B < 0 || P <= 0) return MSAT_EINVAL;
+    if (!(noise >= 0.0 && noise <= 1.0)) return MSAT_EINVAL;          // also NaN
+    if (max_flips < 0 || flip_offset < 0 || (long long)flip_offset + max_flips > 2147483647LL) return MSAT_EINVAL;
+    if (B > 0 && (!bank || !state || !keys)) return MSAT_EINVAL;
+    if (!aligned(bank, 128) || !aligned(state, 16)) return MSAT_EALIGN;
+    if (walksat_warps(plan->d) == 0) return MSAT_EUNSUPPORTED;
+    WalksatArgs a{};
+    a.bank = static_cast<const uint8_t*>(bank); a.P = P; a.state = state; a.keys = keys;
+    a.max_flips = max_flips; a.flip_offset = flip_offset;
+    a.thr = (uint32_t)llrint(noise * 16777216.0);
+    a.solved = solved; a.flips = flips; a.B = B;
+    return cuda_rc(launch_walksat(plan, a, (cudaStream_t)stream));
+}
+
 int msat_step(const msat_plan* plan, const void* bank, int32_t P, const uint32_t* state_in, uint32_t* state_out,
               const int32_t* actions, int32_t auto_reset, const int32_t* new_problem_idx, const uint32_t* reset_keys,
               int32_t* obs, float* reward, int32_t reward_cols, uint8_t* done, int32_t done_cols, uint8_t* solved,

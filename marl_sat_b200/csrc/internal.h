@@ -59,6 +59,7 @@ struct msat_plan {
     // devices on which the > 48 KB dynamic shared memory opt-in of the env kernels has been made (bit = device
     // ordinal); set once per (plan, device) instead of once per launch
     mutable std::atomic<unsigned long long> prepared_devices{0};
+    mutable std::atomic<unsigned long long> prepared_walksat{0};   // the same opt-in for walksat_kernel
 };
 
 namespace msat {
@@ -133,6 +134,50 @@ struct ExportArgs {
     int32_t* l2a;
     int32_t* pidx;
 };
+
+// ---- WalkSAT (local_search.cu) ----------------------------------------------------------------------------
+// Shared-memory carve-up of one warp's env (byte offsets from the warp base): the staged literal block, the
+// var -> clause occurrence lists built from it, u8 true-literal counts, unsatisfied / repeated-variable clause bits,
+// the assignment and the per-candidate break counters.
+constexpr int kWalksatMaxK = 32;                   // one lane per literal column of the picked clause
+constexpr int kWalksatMaxWarps = 8;
+struct WalksatLayout {
+    int lits, occ, row, cnt, unsat, dup, assign, brk, bar, total;
+};
+inline WalksatLayout walksat_layout(const Dims& d) {
+    WalksatLayout L;
+    int o = 0;
+    L.lits = o;   o += (d.lits_bytes + 127) & ~127;          // TMA destination
+    L.occ = o;    o += (2 * d.m * d.k + 15) & ~15;           // u16 (clause << 1) | negated, grouped by variable
+    L.row = o;    o += (4 * d.n + 15) & ~15;                 // int: end of variable v's list (start = row[v - 1])
+    L.cnt = o;    o += (d.m + 15) & ~15;                     // u8 true-literal count per clause
+    L.unsat = o;  o += 4 * d.sw;
+    L.dup = o;    o += 4 * d.sw;                             // clause mentions a variable more than once
+    L.assign = o; o += 4 * d.aw;
+    L.brk = o;    o += 4 * kWalksatMaxK;
+    o = (o + 7) & ~7;
+    L.bar = o;    o += 8;
+    L.total = (o + 127) & ~127;
+    return L;
+}
+// warps (envs) per CTA; 0 = one env's working set does not fit in shared memory
+inline int walksat_warps(const Dims& d) {
+    if (d.k > kWalksatMaxK) return 0;
+    const int w = kMaxSmemOptin / walksat_layout(d).total;
+    return w < kWalksatMaxWarps ? w : kWalksatMaxWarps;
+}
+struct WalksatArgs {
+    const uint8_t* bank;
+    int P;
+    uint32_t* state;
+    const uint32_t* keys;
+    int max_flips, flip_offset;
+    uint32_t thr;               // random walk iff (x1 >> 8) < thr; llrint(noise * 2^24)
+    uint8_t* solved;
+    int32_t* flips;
+    int B;
+};
+cudaError_t launch_walksat(const msat_plan* plan, const WalksatArgs& a, cudaStream_t s);
 
 cudaError_t launch_compile_bank(const msat_plan* plan, const int32_t* clauses, int P, uint8_t* bank, cudaStream_t s);
 cudaError_t launch_env(const msat_plan* plan, EnvMode mode, const EnvArgs& a, cudaStream_t s);

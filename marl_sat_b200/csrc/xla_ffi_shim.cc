@@ -221,6 +221,18 @@ ffi::Error EvalTrack(cudaStream_t s, int64_t plan, int64_t t, ffi::Buffer<ffi::U
                   "msat_eval_track");
 }
 
+// ---- local search ----------------------------------------------------------------------------------------------
+// WalkSAT in place on the packed states (state_in is aliased to state); solved / flips per env
+ffi::Error Walksat(cudaStream_t s, int64_t plan, int64_t num_problems, int64_t max_flips, int64_t flip_offset,
+                   double noise, ffi::Buffer<ffi::U8> bank, ffi::Buffer<ffi::U32> state_in, ffi::Buffer<ffi::U32> keys,
+                   ffi::ResultBuffer<ffi::U32> state, ffi::ResultBuffer<ffi::U8> solved, ffi::ResultBuffer<ffi::S32> flips) {
+    (void)state_in;
+    return status(msat_walksat(plan_of(plan), bank.typed_data(), (int32_t)num_problems, state->typed_data(),
+                               keys.typed_data(), (int32_t)max_flips, (int32_t)flip_offset, noise, solved->typed_data(),
+                               flips->typed_data(), dim0(state->dimensions()), s),
+                  "msat_walksat");
+}
+
 template <ffi::DataType T> using In = ffi::Buffer<T>;
 template <ffi::DataType T> using Out = ffi::Buffer<T>;
 using Stream = ffi::PlatformStream<cudaStream_t>;
@@ -293,3 +305,7 @@ XLA_FFI_DEFINE_HANDLER_SYMBOL(MsatEvalTrack, EvalTrack,
     ffi::Ffi::Bind().Ctx<Stream>().Attr<int64_t>("plan").Attr<int64_t>("t")
         .Arg<In<ffi::U32>>().Arg<In<ffi::U8>>().Arg<In<ffi::U8>>().Arg<In<ffi::S32>>().Arg<In<ffi::S32>>()
         .Ret<Out<ffi::U8>>().Ret<Out<ffi::S32>>().Ret<Out<ffi::S32>>());
+XLA_FFI_DEFINE_HANDLER_SYMBOL(MsatWalksat, Walksat,
+    ffi::Ffi::Bind().Ctx<Stream>().Attr<int64_t>("plan").Attr<int64_t>("num_problems").Attr<int64_t>("max_flips")
+        .Attr<int64_t>("flip_offset").Attr<double>("noise").Arg<In<ffi::U8>>().Arg<In<ffi::U32>>().Arg<In<ffi::U32>>()
+        .Ret<Out<ffi::U32>>().Ret<Out<ffi::U8>>().Ret<Out<ffi::S32>>());

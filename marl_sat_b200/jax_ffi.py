@@ -35,7 +35,7 @@ TARGETS = {
     "MsatRngSplit2": "msat_rng_split2", "MsatEnvKeys": "msat_env_keys", "MsatGae": "msat_gae",
     "MsatAdvStats": "msat_adv_stats", "MsatAdvNormalize": "msat_adv_normalize", "MsatGnnStatic": "msat_gnn_static",
     "MsatGnnDynamic": "msat_gnn_dynamic", "MsatRolloutMetrics": "msat_rollout_metrics",
-    "MsatFlipGains": "msat_flip_gains", "MsatEvalTrack": "msat_eval_track",
+    "MsatFlipGains": "msat_flip_gains", "MsatEvalTrack": "msat_eval_track", "MsatWalksat": "msat_walksat",
 }
 _registered = False
 
@@ -80,6 +80,19 @@ def import_state(plan_handle: int, dims, bank, num_problems: int, problem_idx, v
                                                _sds((B, dims.A, dims.D), jnp.int32)))
     return call(bank, jnp.asarray(problem_idx, jnp.int32), jnp.asarray(variable_assignments, jnp.int32), step,
                 done.astype(jnp.uint8), plan=np.int64(plan_handle), num_problems=np.int64(num_problems))
+
+
+def walksat(plan_handle: int, bank, num_problems: int, state, keys, max_flips: int, noise: float = 0.5,
+            flip_offset: int = 0):
+    """WalkSAT/SKC on packed env states (``msat_walksat``; contract in include/marl_sat_b200.h).  ``state`` is
+    donated (searched in place); ``keys`` uint32 [B, 2].  Returns ``(state, solved uint8[B], flips int32[B])``."""
+    register()
+    B = state.shape[0]
+    call = jffi.ffi_call("msat_walksat", (_sds(state.shape, jnp.uint32), _sds((B,), jnp.uint8), _sds((B,), jnp.int32)),
+                         input_output_aliases={1: 0})
+    return call(bank, state, jnp.asarray(keys, jnp.uint32), plan=np.int64(plan_handle),
+                num_problems=np.int64(num_problems), max_flips=np.int64(max_flips), flip_offset=np.int64(flip_offset),
+                noise=np.float64(noise))
 
 
 def rollout_steps(plan_handle: int, dims, bank, num_problems: int, state, actions, rng, num_envs_global=None,
