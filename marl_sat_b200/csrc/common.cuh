@@ -36,6 +36,10 @@ __host__ __device__ __forceinline__ uint32_t lit_pad(const Dims& d) { return 2u 
 // shared-memory loads), and one aligned 32-bit load fetches the codes of two adjacent clauses.
 __host__ __device__ __forceinline__ int lit_index(int ms, int c, int j) { return j * ms + c; }
 
+// Problem index of an env as every kernel reads it: clamped into [0, P), so an index from outside (reset_from_bank,
+// import_state(validate=False)) or a corrupted state record never addresses past the bank.
+__device__ __forceinline__ int clamp_problem(int pidx, int P) { return pidx < 0 ? 0 : (pidx >= P ? P - 1 : pidx); }
+
 // ---- agent grouping (env:294-338; contiguous balanced split) --------------
 __host__ __device__ __forceinline__ int group_size(const Dims& d, int a) { return d.base + (a < d.rem ? 1 : 0); }
 __host__ __device__ __forceinline__ int group_start(const Dims& d, int a) { return a * d.base + (a < d.rem ? a : d.rem); }

@@ -49,8 +49,7 @@ __global__ void __launch_bounds__(128) gnn_dynamic_kernel(const Dims d, const ui
                                                           float* __restrict__ cf) {
     const int e = blockIdx.x, tid = threadIdx.x, nt = blockDim.x;
     const uint32_t* st = state + (size_t)e * d.state_words;
-    int pidx = (int)st[d.aw + ST_PIDX];
-    pidx = pidx < 0 ? 0 : (pidx >= P ? P - 1 : pidx);
+    const int pidx = clamp_problem((int)st[d.aw + ST_PIDX], P);
     const uint16_t* lits = reinterpret_cast<const uint16_t*>(bank + (size_t)pidx * d.rec_bytes);
     if (assign)
         for (int v = tid; v < d.n; v += nt) assign[(size_t)e * d.n + v] = (int)((st[v >> 5] >> (v & 31)) & 1u);
@@ -137,8 +136,7 @@ __global__ void __launch_bounds__(128) flip_gain_kernel(const Dims d, const uint
     extern __shared__ int gain[];                     // [n] break - make
     const int e = blockIdx.x, tid = threadIdx.x, nt = blockDim.x;
     const uint32_t* st = state + (size_t)e * d.state_words;
-    int pidx = (int)st[d.aw + ST_PIDX];
-    pidx = pidx < 0 ? 0 : (pidx >= P ? P - 1 : pidx);
+    const int pidx = clamp_problem((int)st[d.aw + ST_PIDX], P);
     const uint16_t* lits = reinterpret_cast<const uint16_t*>(bank + (size_t)pidx * d.rec_bytes);
     for (int v = tid; v < d.n; v += nt) gain[v] = 0;
     __syncthreads();

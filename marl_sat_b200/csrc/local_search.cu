@@ -77,8 +77,7 @@ __global__ void __launch_bounds__(kWalksatMaxWarps * 32) walksat_kernel(const Di
     uint32_t* st = a.state + (size_t)e * d.state_words;
     const uint32_t pad = lit_pad(d);
 
-    int pidx = (int)st[d.aw + ST_PIDX];
-    pidx = pidx < 0 ? 0 : (pidx >= a.P ? a.P - 1 : pidx);
+    const int pidx = clamp_problem((int)st[d.aw + ST_PIDX], a.P);
     if (lane == 0) {
         mbar_init(bar, 1);
         mbar_expect_tx(bar, (uint32_t)d.lits_bytes);

@@ -144,6 +144,15 @@ __device__ __forceinline__ void build_truth_table(const Dims& d, const uint32_t*
 // Clause truth via warp ballots (env:130-156): lane = clause, ballot word = 32 clause-status bits, __popc for
 // the number of (un)satisfied clauses; the evaluators follow the bulk-store helpers below.
 
+// Publish the number of unsatisfied clauses.  nsat: the satisfied clauses this thread's warp (sub-warp group for
+// GS < 32) evaluated, the same in each of its lanes.  A group of at most one warp stores m - nsat; the warps of a
+// wider group subtract their counts from *nunsat, which the caller set to m.
+template <int GS>
+__device__ __forceinline__ void publish_unsat(const Dims& d, int* nunsat, int nsat, int gt) {
+    if (GS <= 32) *nunsat = d.m - nsat;
+    else if ((gt & 31) == 0 && nsat) atomicAdd(nunsat, -nsat);
+}
+
 // ---- bulk (TMA) store shared -> global ----------------------------------------------------------------
 __device__ __forceinline__ void tma_store_1d(void* gmem_dst, const void* smem_src, uint32_t bytes) {
     asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gmem_dst), "r"(smem_u32(smem_src)),
@@ -153,6 +162,8 @@ __device__ __forceinline__ void tma_store_1d(void* gmem_dst, const void* smem_sr
 __device__ __forceinline__ void tma_store_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 // all committed bulk stores of this thread have finished READING their shared-memory source
 __device__ __forceinline__ void tma_store_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
+// all committed bulk stores of this thread have completed (their writes are done, not only their reads)
+__device__ __forceinline__ void tma_store_wait() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 
 // Clause evaluation for a GNN-style consumer (learner:165-195): besides status bits and the unsatisfied
 // count it emits clause_features float[m][3] = {is_sat, #true literals / 3.0, 1} -- the literal 3.0 of
@@ -176,7 +187,7 @@ __device__ __forceinline__ uint32_t true_literals(const Dims& d, const uint16_t*
 
 // cf01[t] = {t > 0 ? 1 : 0, t / 3.0} for t = 0..15: the first two clause features of a clause with t true literals
 // True-literal count of clause c for the evaluators below.  INCR: the 4-bit count carried in the state (kept
-// up to date by apply_actions_incr); otherwise from the staged literals, optionally packed into `cnt_store`
+// up to date by flip_and_update_counts); otherwise from the staged literals, optionally packed into `cnt_store`
 // (zeroed by the caller) so that a state of an incremental plan leaves every kernel with valid counts.
 template <bool K3, bool INCR, bool STORE = true>
 __device__ __forceinline__ uint32_t clause_count(const Dims& d, const uint16_t* lits, const uint8_t* tt,
@@ -247,9 +258,7 @@ __device__ __forceinline__ void eval_clauses_gnn(const Dims& d, const uint16_t* 
             if (mine) *reinterpret_cast<float*>(gdst + i) = *reinterpret_cast<const float*>(stage + phase16 + i);
         }
     }
-    // every lane of a warp holds the same count; one-warp groups need no shared accumulator
-    if (GS == 32) *nunsat = d.m - nsat;
-    else if (lane == 0 && nsat) atomicAdd(nunsat, -nsat);
+    publish_unsat<GS>(d, nunsat, nsat, gt);
 }
 
 // Paired evaluation for k == 3 in launches without observations: a lane owns two ADJACENT clauses, so one aligned
@@ -325,10 +334,7 @@ __device__ __forceinline__ void eval_clauses_pairs(const Dims& d, const uint16_t
         }
     }
     nsat = __reduce_add_sync(0xffffffffu, nsat);
-    if (nunsat) {
-        if (GS == 32) *nunsat = d.m - nsat;
-        else if ((gt & 31) == 0 && nsat) atomicAdd(nunsat, -nsat);
-    }
+    if (nunsat) publish_unsat<GS>(d, nunsat, nsat, gt);
 }
 
 // Plain evaluation (no clause features): status bits + number of unsatisfied clauses (optional).
@@ -363,7 +369,6 @@ __device__ __forceinline__ void eval_clauses_impl(const Dims& d, const uint16_t*
         }
         if (gt == 0)
             for (; r < (32 / GS) * d.sw; ++r) piece[r] = 0;      // rest of the last status word
-        if (nunsat) *nunsat = d.m - nsat;
     } else {
         for (int w = gt >> 5; w < d.sw; w += GS / 32) {
             const int c = w * 32 + lane;
@@ -372,11 +377,8 @@ __device__ __forceinline__ void eval_clauses_impl(const Dims& d, const uint16_t*
             nsat += __popc(word);
             if (lane == 0) satw[w] = word;
         }
-        if (nunsat) {
-            if (GS == 32) *nunsat = d.m - nsat;
-            else if (lane == 0 && nsat) atomicAdd(nunsat, -nsat);
-        }
     }
+    if (nunsat) publish_unsat<GS>(d, nunsat, nsat, gt);
 }
 // Half-warp groups, k == 3: a lane owns two ADJACENT clauses (one aligned 32-bit load per literal column fetches
 // both codes), so one trip of the 16 lanes covers a whole 32-bit status word: the ballots of the even and the odd
@@ -408,7 +410,7 @@ __device__ __forceinline__ void eval_clauses_pairs16(const Dims& d, const uint16
         nsat += __popc(word);
         if (gt == 0) satw[w] = word;
     }
-    if (nunsat) *nunsat = d.m - nsat;
+    if (nunsat) publish_unsat<16>(d, nunsat, nsat, gt);
 }
 
 template <int GS, bool K3, bool INCR>
@@ -467,11 +469,12 @@ __device__ __forceinline__ void load_assign(const Dims& d, const int32_t* __rest
     }
 }
 
-// Apply all agents' flips simultaneously (env:233-250) on the packed assignment in shared memory.
-// has_pre: the caller already holds act[gt] (mode 0) in `pre` (loaded early, next to the state record).
-template <int GS>
-__device__ __forceinline__ void apply_actions(const Dims& d, const int32_t* __restrict__ actions, int e,
-                                              uint32_t* assign, int gt, bool has_pre, int pre) {
+// Decode all agents' actions of env e (env:233-250) and call flip(v) once for every variable that flips; the flips
+// are simultaneous, so flip must commute (atomics).  has_pre: the caller already holds act[gt] (mode 0) in `pre`
+// (loaded early, next to the state record).
+template <int GS, typename F>
+__device__ __forceinline__ void for_each_flip(const Dims& d, const int32_t* __restrict__ actions, int e, int gt,
+                                              bool has_pre, int pre, F flip) {
     if (d.action_mode == 0) {
         const int32_t* act = actions + (size_t)e * d.A;
         for (int a = gt; a < d.A; a += GS) {
@@ -482,17 +485,14 @@ __device__ __forceinline__ void apply_actions(const Dims& d, const int32_t* __re
             if (idx < 0) idx += d.V;                       // JAX gather: wrap once, then clamp
             idx = idx < 0 ? 0 : (idx > d.V - 1 ? d.V - 1 : idx);
             if (idx >= size) continue;                     // landed on a -1 pad: one_hot(-1) = 0 (env:243)
-            const int v = group_start(d, a) + idx;
-            atomicXor(&assign[v >> 5], 1u << (v & 31));
+            flip(group_start(d, a) + idx);
         }
     } else {
         const int32_t* act = actions + (size_t)e * d.A * d.V;
         for (int i = gt; i < d.A * d.V; i += GS) {
             const int a = i / d.V, j = i - a * d.V;
-            if (j < group_size(d, a) && (act[i] & 1)) {    // env:246-250 (actions are 0/1)
-                const int v = group_start(d, a) + j;
-                atomicXor(&assign[v >> 5], 1u << (v & 31));
-            }
+            if (j < group_size(d, a) && (act[i] & 1))      // env:246-250 (actions are 0/1)
+                flip(group_start(d, a) + j);
         }
     }
 }
@@ -516,32 +516,6 @@ __device__ __forceinline__ void flip_and_update_counts(const Dims& d, const uint
         const uint32_t unit = 1u << (4 * (c & 7));
         if ((code & 1u) ^ now_true) atomicAdd(&cntw[c >> 3], unit);           // this literal became true
         else atomicSub(&cntw[c >> 3], unit);
-    }
-}
-
-template <int GS>
-__device__ __forceinline__ void apply_actions_incr(const Dims& d, const int32_t* __restrict__ actions, int e,
-                                                   const uint8_t* csr, uint32_t* assign, uint32_t* cntw,
-                                                   int gt) {
-    if (d.action_mode == 0) {
-        const int32_t* act = actions + (size_t)e * d.A;
-        for (int a = gt; a < d.A; a += GS) {
-            const int x = act[a];
-            const int size = group_size(d, a);
-            if (x >= size) continue;                       // env:236 no-op
-            int idx = x < size - 1 ? x : size - 1;         // env:238
-            if (idx < 0) idx += d.V;                       // JAX gather: wrap once, then clamp
-            idx = idx < 0 ? 0 : (idx > d.V - 1 ? d.V - 1 : idx);
-            if (idx >= size) continue;                     // landed on a -1 pad: one_hot(-1) = 0 (env:243)
-            flip_and_update_counts(d, csr, group_start(d, a) + idx, assign, cntw);
-        }
-    } else {
-        const int32_t* act = actions + (size_t)e * d.A * d.V;
-        for (int i = gt; i < d.A * d.V; i += GS) {
-            const int a = i / d.V, j = i - a * d.V;
-            if (j < group_size(d, a) && (act[i] & 1))      // env:246-250 (actions are 0/1)
-                flip_and_update_counts(d, csr, group_start(d, a) + j, assign, cntw);
-        }
     }
 }
 
@@ -859,7 +833,7 @@ __global__ void __launch_bounds__(kCtaThreads, (MULTI || !OBS) ? 4 : 8) env_kern
     int pidx;
     if (FRESH) pidx = a.prob_idx[e];
     else pidx = (int)st_tail[ST_PIDX];
-    pidx = pidx < 0 ? 0 : (pidx >= a.P ? a.P - 1 : pidx);
+    pidx = clamp_problem(pidx, a.P);
     int loaded_pidx = -1;           // formula whose block sits in the record slot ...
     bool loaded_csr = false;        // ... and whether that block is its occurrence lists (incremental steps) or its literals
     uint32_t phase = 0u;
@@ -916,10 +890,12 @@ __global__ void __launch_bounds__(kCtaThreads, (MULTI || !OBS) ? 4 : 8) env_kern
                     loaded_pidx = pidx;
                     loaded_csr = true;
                 }
-                apply_actions_incr<GS>(d, a.actions + (long long)j * a.act_step_stride, e, rec, st, cntw, gt);
+                for_each_flip<GS>(d, a.actions + (long long)j * a.act_step_stride, e, gt, false, 0,
+                                  [&](int v) { flip_and_update_counts(d, rec, v, st, cntw); });
+            } else {
+                for_each_flip<GS>(d, a.actions + (long long)j * a.act_step_stride, e, gt, act_pre_ok && j == 0, act_pre,
+                                  [&](int v) { atomicXor(&st[v >> 5], 1u << (v & 31)); });
             }
-            else apply_actions<GS>(d, a.actions + (long long)j * a.act_step_stride, e, st, gt,
-                                   act_pre_ok && j == 0, act_pre);
         }
         if (!INCR && cnt_store)
             for (int i = gt; i < d.cnt_words; i += GS) cnt_store[i] = 0u;
@@ -1008,7 +984,7 @@ __global__ void __launch_bounds__(kCtaThreads, (MULTI || !OBS) ? 4 : 8) env_kern
                     rk0 = a.keys[2 * (size_t)e];
                     rk1 = a.keys[2 * (size_t)e + 1];
                 }
-                pidx = pidx < 0 ? 0 : (pidx >= a.P ? a.P - 1 : pidx);
+                pidx = clamp_problem(pidx, a.P);
                 // the full evaluation of the new episode needs the literal block (an incremental step had the
                 // occurrence lists in the slot)
                 const bool need_lits = pidx != loaded_pidx || (INCR && loaded_csr);
@@ -1038,7 +1014,7 @@ __global__ void __launch_bounds__(kCtaThreads, (MULTI || !OBS) ? 4 : 8) env_kern
                 // the clause features of the finished episode are already on their way to the same rows: let
                 // those bulk stores complete before the new episode's features are sent after them
                 if (cf_row) {
-                    if (gt == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+                    if (gt == 0) tma_store_wait();
                     group_sync<GS>(gid);
                 }
                 run_eval<GS, false, OBS>(d, lits, tt, cnt_store, satw, &misc[0], cf01, stage, cf_row, pairs, gid, gt);
@@ -1089,13 +1065,14 @@ static cudaError_t launch_env_gs(const msat_plan* plan, EnvMode mode, const EnvA
     const int grid = (a.B + groups - 1) / groups;
     if (grid == 0) return cudaSuccess;
     // every instantiation a launch with this (GS, OBS) can select: the shared-memory opt-in below covers them all.
-    // incremental clause update: step launches without observations on a plan that carries the counts
+    // The single-step kernels sit at index `mode`, then the multi-step one, then the incremental clause update's
+    // single- and multi-step kernels (step launches without observations on a plan that carries the counts).
     constexpr int kFns = OBS ? 5 : 7;
     const void* fns[7] = {(const void*)env_kernel<GS, MODE_RESET, OBS, false, false>,
                           (const void*)env_kernel<GS, MODE_STEP, OBS, false, false>,
                           (const void*)env_kernel<GS, MODE_OBS, OBS, false, false>,
-                          (const void*)env_kernel<GS, MODE_STEP, OBS, true, false>,
                           (const void*)env_kernel<GS, MODE_IMPORT, OBS, false, false>,
+                          (const void*)env_kernel<GS, MODE_STEP, OBS, true, false>,
                           OBS ? nullptr : (const void*)env_kernel<GS, MODE_STEP, false, false, true>,
                           OBS ? nullptr : (const void*)env_kernel<GS, MODE_STEP, false, true, true>};
     const bool multi = mode == MODE_STEP && a.num_steps > 1;
@@ -1115,8 +1092,7 @@ static cudaError_t launch_env_gs(const msat_plan* plan, EnvMode mode, const EnvA
             plan->prepared_devices.fetch_or(bit, std::memory_order_release);
         }
     }
-    const void* fn = incr ? fns[multi ? 6 : 5]
-                          : fns[multi ? 3 : (mode == MODE_RESET ? 0 : (mode == MODE_STEP ? 1 : (mode == MODE_OBS ? 2 : 4)))];
+    const void* fn = fns[incr ? 5 + (int)multi : (multi ? 4 : (int)mode)];
     Dims d = plan->d;
     EnvArgs args = a;
     void* params[] = {&d, &args};
@@ -1169,8 +1145,7 @@ __global__ void __launch_bounds__(128) export_kernel(const Dims d, const ExportA
     const int e = blockIdx.x, tid = threadIdx.x, nt = blockDim.x;
     const uint32_t* st = a.state + (size_t)e * d.state_words;
     const uint32_t* tail = st + d.aw;
-    int pidx = (int)tail[ST_PIDX];
-    pidx = pidx < 0 ? 0 : (pidx >= a.P ? a.P - 1 : pidx);
+    const int pidx = clamp_problem((int)tail[ST_PIDX], a.P);
     const uint8_t* rec = a.bank + (size_t)pidx * d.rec_bytes;
     const uint16_t* lits = reinterpret_cast<const uint16_t*>(rec);
     const uint32_t* mflat = reinterpret_cast<const uint32_t*>(rec + d.lits_bytes);
