@@ -418,6 +418,25 @@ int msat_walksat(const msat_plan* plan, const void* bank, int32_t num_problems,
 int msat_dimacs_parse(const char* text, size_t len, int32_t strict, int32_t* num_vars, int32_t* num_clauses,
                       int32_t* clause_count, int32_t* max_width, int32_t* clauses, int32_t clause_stride);
 
+/* --- observation memory (host only) --------------------------------------------------------------------
+ * Device memory with the driver's generic data compression (CU_MEM_ALLOCATION_COMP_GENERIC), where the L2
+ * compresses lines on their way to DRAM and expands them on the way back.  Observation buffers hold only
+ * -1 / 0 / 1 and are most of a step's DRAM writes; in this memory the same bytes cost less DRAM traffic.
+ * Kernels, copies and torch ops see identical contents.  Unlike the enqueue calls above, these allocate and
+ * synchronise, and they are not bound in the XLA FFI layer (XLA allocates its custom calls' outputs).
+ *
+ * msat_obs_compression: *granted = 1 when `device` reports generic compression support and the driver
+ *   honours the compressible property for a probe allocation (and for every msat_obs_alloc on it since),
+ *   else 0.  MSAT_EINVAL for a NULL `granted`, a negative or unknown device.
+ * msat_obs_alloc / msat_obs_free: the allocation pair torch.cuda.memory.CUDAPluggableAllocator expects
+ *   (`stream` is a cudaStream_t and unused).  alloc maps `size` bytes rounded up to the driver's
+ *   recommended granularity on `device` and returns NULL when the driver refuses; free waits for the
+ *   device, unmaps and releases the memory.  Memory the driver hands back uncompressed is still returned
+ *   and turns msat_obs_compression off for the device. */
+int msat_obs_compression(int device, int* granted);
+void* msat_obs_alloc(size_t size, int device, void* stream);
+void msat_obs_free(void* ptr, size_t size, int device, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -75,6 +75,9 @@ SIGNATURES = {
                                     C.POINTER(_i32), _p, _i32]),
     "msat_eval_track": (C.c_int, [_p, _p, _p, _i32, _i32, _p, _p, _p, _p]),
     "msat_walksat": (C.c_int, [_p, _p, _i32, _p, _p, _i32, _i32, _f64, _p, _p, _i32, _p]),
+    "msat_obs_compression": (C.c_int, [C.c_int, C.POINTER(C.c_int)]),
+    "msat_obs_alloc": (_p, [C.c_size_t, C.c_int, _p]),
+    "msat_obs_free": (None, [_p, C.c_size_t, C.c_int, _p]),
 }
 
 _lib = None

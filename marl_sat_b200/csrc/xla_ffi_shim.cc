@@ -5,6 +5,9 @@
 // handler validates nothing itself, forwards to msat_* (enqueue only, no allocation, no synchronisation) and
 // maps a non-zero return code to an ffi::Error.
 //
+// The observation-memory calls msat_obs_compression(), msat_obs_alloc() and msat_obs_free() have no handler:
+// they allocate, and XLA allocates the outputs of a custom call itself.
+//
 // Built only where JAX ships the FFI headers (marl_sat_b200/build.py: `jax.ffi.include_dir()`); this image has
 // no JAX, so here the file is syntax-checked against tests/ffi_stub and otherwise unused.  Registration and the
 // `jax.ffi.ffi_call` wrappers live in marl_sat_b200/jax_ffi.py.

@@ -57,6 +57,35 @@ def u32_to_numpy(t: torch.Tensor) -> np.ndarray:
     return t.detach().cpu().contiguous().numpy().view(np.uint32)
 
 
+_OBS_POOLS: Dict[int, Optional["torch.cuda.MemPool"]] = {}
+
+
+def _obs_pool(device: torch.device) -> Optional["torch.cuda.MemPool"]:
+    """The device's pool of compressible memory (``msat_obs_alloc``), or None where the driver does not grant
+    generic compression.  Created on first use and kept for the life of the process."""
+    index = device.index if device.index is not None else torch.cuda.current_device()
+    if index not in _OBS_POOLS:
+        lib, granted = _lib.load(), C.c_int(0)
+        _lib.check(lib.msat_obs_compression(index, C.byref(granted)), "msat_obs_compression")
+        pool = None
+        if granted.value:
+            alloc = torch.cuda.memory.CUDAPluggableAllocator(str(_lib.lib_path()), "msat_obs_alloc", "msat_obs_free")
+            pool = torch.cuda.MemPool(alloc.allocator())
+        _OBS_POOLS[index] = pool
+    return _OBS_POOLS[index]
+
+
+def obs_empty(shape, dtype: torch.dtype, device: torch.device) -> torch.Tensor:
+    """``torch.empty`` for observation buffers.  Observations (-1 / 0 / 1 words) are most of a step's DRAM
+    writes; where the device grants generic compression they live in compressible memory, which DRAM stores in
+    fewer bytes.  Contents and every operation on the tensor are the same either way."""
+    pool = _obs_pool(device)
+    if pool is None:
+        return torch.empty(shape, dtype=dtype, device=device)
+    with torch.cuda.use_mem_pool(pool, device):
+        return torch.empty(shape, dtype=dtype, device=device)
+
+
 def create_agent_groups(num_vars: int, vars_per_agent: Optional[int], verbose: bool = True) -> Dict[str, List[int]]:
     """Reference grouping rule (env:294-338): ceil(n/vpa) agents when ``vars_per_agent`` is given, else
     n/4 agents if 4 divides n, else max(2, floor(sqrt(n))); contiguous ranges, the first ``n % A``
@@ -349,7 +378,7 @@ class SATEnv:
         packed = state_out if state_out is not None else torch.empty((B, d.state_words), dtype=torch.int32, device=dev)
         obs = obs_out
         if obs is None and want_obs:
-            obs = torch.empty((B, d.A, d.D), dtype=self.obs_dtype, device=dev)
+            obs = obs_empty((B, d.A, d.D), self.obs_dtype, dev)
         _lib.check(self._lib.msat_reset(bank.plan.handle, _ptr(bank.data), bank.num_problems, _ptr(problem_idx),
                                         _ptr(keys), _ptr(packed), _ptr(obs), B, _stream_ptr(dev)), "msat_reset")
         return obs, SATState(self, bank, packed, True)
@@ -439,7 +468,7 @@ class SATEnv:
         packed = state_out if state_out is not None else torch.empty((B, d.state_words), dtype=torch.int32, device=dev)
         obs = obs_out
         if obs is None and want_obs:
-            obs = torch.empty((B, d.A, d.D), dtype=self.obs_dtype, device=dev)
+            obs = obs_empty((B, d.A, d.D), self.obs_dtype, dev)
         _lib.check(self._lib.msat_import_state(bank.plan.handle, _ptr(bank.data), bank.num_problems, _ptr(idx),
                                                _ptr(va), _ptr(st), _ptr(dn), _ptr(packed), _ptr(obs), B,
                                                _stream_ptr(dev)), "msat_import_state")
@@ -501,7 +530,7 @@ class SATEnv:
         else:
             dev = self._require_cuda()
             block = torch.empty(B * (4 * rc + 8 + dc + 1), dtype=torch.uint8, device=dev)
-            obs = torch.empty((B, A, D), dtype=self.obs_dtype, device=dev) if want_obs else None
+            obs = obs_empty((B, A, D), self.obs_dtype, dev) if want_obs else None
         o0, o1, o2, o3 = 4 * rc * B, 4 * rc * B + 4 * B, 4 * rc * B + 8 * B, 4 * rc * B + 8 * B + dc * B
         newly = None
         if self.reward_mode == "shaped":
@@ -537,7 +566,7 @@ class SATEnv:
         dev = self._require_cuda()
         d = state.bank.plan.dims
         B = state.num_envs
-        obs = torch.empty((B, d.A, d.D), dtype=self.obs_dtype, device=dev)
+        obs = obs_empty((B, d.A, d.D), self.obs_dtype, dev)
         _lib.check(self._lib.msat_get_obs(state.bank.plan.handle, _ptr(state.bank.data), state.bank.num_problems,
                                           _ptr(state.packed), _ptr(obs), B, _stream_ptr(dev)), "msat_get_obs")
         return obs

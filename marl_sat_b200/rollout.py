@@ -26,7 +26,7 @@ from typing import Dict, Optional
 import torch
 
 from . import _lib
-from .env import FormulaBank, SATEnv, SATState, _ptr, _stream_ptr, as_u32_tensor
+from .env import FormulaBank, SATEnv, SATState, _ptr, _stream_ptr, as_u32_tensor, obs_empty
 
 
 def prng_key(seed: int):
@@ -236,7 +236,7 @@ class VecSATEnv:
             out["gnn_assignment"] = torch.empty(lead + (d.n,), dtype=torch.int32, device=dev)
             out["gnn_clause_features"] = torch.empty(lead + (d.m, 3), dtype=torch.float32, device=dev)
         elif self.out.get("obs") is not None:
-            out["obs"] = torch.empty(lead + (d.A, d.D), dtype=self.env.obs_dtype, device=dev)
+            out["obs"] = obs_empty(lead + (d.A, d.D), self.env.obs_dtype, dev)
         return out
 
     def steps(self, actions: torch.Tensor, out: Dict[str, torch.Tensor]) -> Dict[str, torch.Tensor]:
