@@ -10,6 +10,13 @@ PPO epochs on a small MLP actor/critic with DistributedDataParallel (NCCL gradie
 
 Rank 0 prints one JSON line: updates/s, env-steps/s of the whole cycle, the rollout / GAE / update split
 (max over ranks, CUDA events) and the bus bandwidth of a gradient-sized NCCL all-reduce.
+
+``--curriculum`` chooses which formulas auto-reset draws:
+  none      uniform over the bank (the default, the reference's randint);
+  unsolved  per-problem statistics of every rollout are accumulated (``RolloutBuffer.problem_stats``) and after each
+            update the weights become ``unsolved_weights`` of the totals;
+  walksat   one WalkSAT call over a reset of every bank formula labels the formulas it solves; only those are drawn.
+The JSON line then also reports the share of the bank solved at least once during the timed updates.
 Reference structure: src/learners/mappo_gnn_sat_learner.py:381-732, configs/MAPPO_CONFIG.yaml:27-48.
 """
 import argparse
@@ -28,6 +35,18 @@ from marl_sat_b200 import synth                                     # noqa: E402
 from marl_sat_b200.mappo import MAPPOTrainer, MLPActorCritic, PPOConfig    # noqa: E402
 
 
+def walksat_solvable(M, env, bank, max_flips, dev) -> torch.Tensor:
+    """bool [P]: the formulas one WalkSAT call (noise 0.5) solves from a reset of every bank formula."""
+    P = bank.num_problems
+    idx = torch.arange(P, dtype=torch.int32, device=dev)
+    keys = M.env.as_u32_tensor(torch.stack([torch.zeros(P, dtype=torch.int64), torch.arange(P)], 1), dev)
+    _, state = env.reset_from_bank(bank, idx, keys, want_obs=False)
+    solved = M.walksat(state, keys, max_flips).solved.cpu()
+    if not bool(solved.any()):
+        raise SystemExit(f"WalkSAT solved none of the {P} formulas in {max_flips} flips: nothing to train on")
+    return solved
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--n", type=int, default=250)
@@ -42,6 +61,9 @@ def main():
     ap.add_argument("--hidden", type=int, default=128)
     ap.add_argument("--obs-int8", action="store_true",
                     help="int8 observations (MSAT_OBS_INT8): same values, a quarter of the bytes the policy reads")
+    ap.add_argument("--curriculum", choices=("none", "unsolved", "walksat"), default="none",
+                    help="problem draw of auto-reset: uniform, weighted by unsolved rate, or WalkSAT-solved formulas only")
+    ap.add_argument("--walksat-flips", type=int, default=10000, help="flip budget of the walksat curriculum's labelling")
     args = ap.parse_args()
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -57,6 +79,10 @@ def main():
     problems = synth.uniform_ksat_torch(args.problems, args.n, args.m, 3, seed=20261018 + 4, device=dev)
     bank = env.make_bank(problems, validate=False)
     vec = M.VecSATEnv(env, bank, args.envs, M.prng_key(42), world_size=world, rank=rank, compact_outputs=True)
+    labelled = None
+    if args.curriculum == "walksat":
+        labelled = walksat_solvable(M, env, bank, args.walksat_flips, dev)
+        vec.set_problem_weights(labelled)           # identical on every rank: same bank, same keys
     vec.reset()
     torch.manual_seed(0)                       # identical initial weights on every rank
     net = MLPActorCritic(env, hidden=args.hidden)
@@ -70,8 +96,13 @@ def main():
     t0 = time.perf_counter()
     last = None
     split = torch.zeros(3, dtype=torch.float64, device=dev)
+    totals = torch.zeros((bank.num_problems, 4), dtype=torch.int64, device=dev)     # all-reduced per-problem stats
     for _ in range(args.updates):
         last = trainer.train_cycle()
+        if args.curriculum != "none":
+            trainer.buf.problem_stats(totals)   # this rollout's counters, summed over the ranks, added to the totals
+        if args.curriculum == "unsolved":
+            vec.set_problem_weights(M.unsolved_weights(totals))
         split += torch.tensor([last["rollout_ms"], last["gae_metrics_ms"], last["update_ms"]], dtype=torch.float64,
                               device=dev)
     torch.cuda.synchronize()
@@ -106,6 +137,10 @@ def main():
             "rollout_env_steps_per_s": args.steps * args.envs / (rollout_ms * 1e-3),
             "gradient_allreduce": bus, "replicas_in_sync": in_sync,
             "metrics_last_update": {k: v for k, v in last.items() if not k.endswith("_ms")},
+            "curriculum": args.curriculum,
+            "bank_share_solved_at_least_once": (None if args.curriculum == "none"
+                                                else float((totals[:, 1] > 0).double().mean())),
+            "bank_share_walksat_solved": None if labelled is None else float(labelled.double().mean()),
         }))
     if world > 1:
         dist.barrier()

@@ -309,6 +309,26 @@ int msat_env_keys(const uint32_t* prob_key, const uint32_t* reset_key,
                   int32_t num_envs_global, int32_t env_offset, int32_t num_envs_local,
                   int32_t num_problems, int32_t* problem_idx, uint32_t* reset_keys, void* stream);
 
+/* msat_env_keys with a weighted problem draw, for curricula that choose which formulas auto-reset lands on
+ * (train only on formulas a solver labelled satisfiable, weight by unsolved rate, ...).  Feed its outputs to
+ * msat_step(auto_reset = 1) after msat_rng_chain.
+ *
+ * Weighted draw contract (oracle/curriculum.py restates it word for word).  For global env g out of Bg:
+ *   - take the two 32-bit words randint already uses for that env: (k1, k2) = split(prob_key),
+ *     hi = bits32_at(k1, Bg, g), lo = bits32_at(k2, Bg, g); let u = hi * 2^32 + lo;
+ *   - cum_weights int64[P] holds inclusive prefix sums of non-negative integer weights; W = cum_weights[P-1];
+ *   - if W <= 0 the index is the uniform draw, equal to what msat_env_keys returns;
+ *   - otherwise r = floor(u * W / 2^64) (umulhi) and the index is the smallest p with cum_weights[p] > r;
+ *   - the index is always in [0, P), also when the table is not monotone: the binary search is bounded;
+ *   - reset_keys are identical to msat_env_keys' output.
+ * Each draw depends only on (prob_key, Bg, g, cum_weights), so any sharding yields the single-device values.
+ * A problem of weight 0 is never drawn while W > 0.  cum_weights must be 8-byte aligned (MSAT_EALIGN) and is read
+ * only when problem_idx != NULL. */
+int msat_env_keys_weighted(const uint32_t* prob_key, const uint32_t* reset_key,
+                           int32_t num_envs_global, int32_t env_offset, int32_t num_envs_local,
+                           const int64_t* cum_weights, int32_t num_problems,
+                           int32_t* problem_idx, uint32_t* reset_keys, void* stream);
+
 /* --- MAPPO advantage path (learner:504-532) ------------------------------------ */
 
 /* Reverse GAE scan.  reward: float, element (t,b) at reward[t*reward_stride_t +
@@ -351,6 +371,20 @@ int msat_rollout_metrics(const float* reward, int64_t reward_stride_t, int64_t r
                          const uint8_t* done, const uint8_t* solved, const int32_t* num_unsatisfied,
                          const int32_t* episode_step, int32_t num_steps, int32_t num_envs,
                          double* sums, void* stream);
+
+/* Per-problem rollout statistics over a [T,B] rollout: stats int64[P,4].  For every (t, b) with done[t,b] != 0 one
+ * episode is added to row p = clamp(problem_idx[t*pidx_stride_t + b*pidx_stride_b], 0, P-1); the columns are, in the
+ * order of msat_rollout_metrics' sums 1..4: #finished episodes, #solved at finish, sum of num_unsatisfied at finish,
+ * sum of episode_step over the episodes solved at finish.  Not cleared by the call (zero it first; shards can be
+ * all-reduced).  Strides count int32 elements, so a RolloutBuffer's state [T, B, state_words] can be passed as is,
+ * pointing at the problem-index word (word ceil(n/32) + 1, DESIGN.md section 3): the pre-step state of row t belongs
+ * to the episode that ends at t.  done, solved uint8 and num_unsatisfied, episode_step int32 are dense [T,B].
+ * stats must be 8-byte aligned (MSAT_EALIGN).  Rows of one problem are summed per warp and, for P <= 1024, per CTA in
+ * shared memory, so a hot problem (P = 1) does not serialise on one counter. */
+int msat_problem_stats(const int32_t* problem_idx, int64_t pidx_stride_t, int64_t pidx_stride_b,
+                       const uint8_t* done, const uint8_t* solved, const int32_t* num_unsatisfied,
+                       const int32_t* episode_step, int32_t num_steps, int32_t num_envs,
+                       int32_t num_problems, int64_t* stats, void* stream);
 
 /* Per-variable flip gains and the greedy expert labels of the BC pre-training
  * (src/runners/behavioral_cloning.py:54-100): delta_unsat int32[B,n] = change of the number of

@@ -21,11 +21,13 @@ from .features import (GNNInput, StaticGraph, dynamic_features, flip_gains, gnn_
 from .metrics import metrics_from_sums, rollout_metric_sums, rollout_metrics  # noqa: E402
 from .evaluate import evaluate_policy  # noqa: E402
 from .local_search import WalkSATResult, walksat  # noqa: E402
+from .curriculum import problem_stats, problem_weights, unsolved_weights  # noqa: E402
 from . import dimacs  # noqa: E402
 
 __all__ = ["SATEnv", "SATState", "FormulaBank", "create_agent_groups", "SATDataWrapper", "GNNWrapperState",
            "VecSATEnv", "RolloutBuffer", "RolloutKeys", "derive_env_keys", "merge_state_dicts", "shard_range",
            "prng_key", "calculate_gae",
            "advantage_stats", "normalize_advantages", "allreduce_stats", "mean_std_from_stats", "metrics_from_sums", "GNNInput", "StaticGraph", "static_graph", "dynamic_features",
-           "gnn_input_from_state", "flip_gains", "rollout_metrics", "rollout_metric_sums", "evaluate_policy", "walksat", "WalkSATResult", "dimacs"]
+           "gnn_input_from_state", "flip_gains", "rollout_metrics", "rollout_metric_sums", "evaluate_policy", "walksat", "WalkSATResult", "problem_stats",
+           "problem_weights", "unsolved_weights", "dimacs"]
 __version__ = "0.1.0"

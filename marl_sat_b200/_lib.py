@@ -64,6 +64,8 @@ SIGNATURES = {
     "msat_rng_chain": (C.c_int, [_p, _p, _p]),
     "msat_rng_split2": (C.c_int, [_p, _p, _p]),
     "msat_env_keys": (C.c_int, [_p, _p, _i32, _i32, _i32, _i32, _p, _p, _p]),
+    "msat_env_keys_weighted": (C.c_int, [_p, _p, _i32, _i32, _i32, _p, _i32, _p, _p, _p]),
+    "msat_problem_stats": (C.c_int, [_p, _i64, _i64, _p, _p, _p, _p, _i32, _i32, _i32, _p, _p]),
     "msat_gae": (C.c_int, [_p, _i64, _i64, _p, _p, _p, _f64, _f64, _p, _p, _p, _i32, _i32, _p]),
     "msat_adv_stats": (C.c_int, [_p, _i64, _p, _p]),
     "msat_adv_normalize": (C.c_int, [_p, _i64, _p, _p]),

@@ -625,7 +625,33 @@ int msat_env_keys(const uint32_t* prob_key, const uint32_t* reset_key, int32_t B
     if (problem_idx && (!prob_key || P <= 0)) return MSAT_EINVAL;
     if (reset_keys && !reset_key) return MSAT_EINVAL;
     if (Bg > (1 << 30)) return MSAT_EUNSUPPORTED;
-    return cuda_rc(launch_env_keys(prob_key, reset_key, Bg, off, Bl, P, problem_idx, reset_keys, (cudaStream_t)stream));
+    return cuda_rc(launch_env_keys(prob_key, reset_key, Bg, off, Bl, P, problem_idx, reset_keys, nullptr,
+                                   (cudaStream_t)stream));
+}
+
+int msat_env_keys_weighted(const uint32_t* prob_key, const uint32_t* reset_key, int32_t Bg, int32_t off, int32_t Bl,
+                           const int64_t* cum_weights, int32_t P, int32_t* problem_idx, uint32_t* reset_keys,
+                           void* stream) {
+    if (Bg < 0 || off < 0 || Bl < 0 || (long long)off + Bl > Bg) return MSAT_EINVAL;
+    if (problem_idx && (!prob_key || !cum_weights || P <= 0)) return MSAT_EINVAL;
+    if (reset_keys && !reset_key) return MSAT_EINVAL;
+    if (!aligned(cum_weights, 8)) return MSAT_EALIGN;
+    if (Bg > (1 << 30)) return MSAT_EUNSUPPORTED;
+    // without problem indices to draw, the call is msat_env_keys' reset-key half
+    const long long* cum = problem_idx ? reinterpret_cast<const long long*>(cum_weights) : nullptr;
+    return cuda_rc(launch_env_keys(prob_key, reset_key, Bg, off, Bl, P, problem_idx, reset_keys, cum,
+                                   (cudaStream_t)stream));
+}
+
+int msat_problem_stats(const int32_t* problem_idx, int64_t pidx_stride_t, int64_t pidx_stride_b, const uint8_t* done,
+                       const uint8_t* solved, const int32_t* num_unsatisfied, const int32_t* episode_step, int32_t T,
+                       int32_t B, int32_t P, int64_t* stats, void* stream) {
+    if (T < 0 || B < 0 || P <= 0 || !stats) return MSAT_EINVAL;
+    if (T > 0 && B > 0 && (!problem_idx || !done || !solved || !num_unsatisfied || !episode_step)) return MSAT_EINVAL;
+    if (!aligned(stats, 8)) return MSAT_EALIGN;
+    return cuda_rc(launch_problem_stats(problem_idx, pidx_stride_t, pidx_stride_b, done, solved, num_unsatisfied,
+                                        episode_step, T, B, P, reinterpret_cast<long long*>(stats),
+                                        (cudaStream_t)stream));
 }
 
 int msat_gae(const float* reward, int64_t rs_t, int64_t rs_b, const uint8_t* done, const float* value,

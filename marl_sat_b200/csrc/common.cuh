@@ -109,18 +109,31 @@ __host__ __device__ __forceinline__ void rng_chain_compute(uint32_t r0, uint32_t
     out[8] = y1; out[9] = z1;                   // reset_key
 }
 
-// problem index and reset key of global env g out of Bg (learner:430,434):
-//   randint(prob_key, (Bg,), 0, P)[g]  and  split(reset_key, Bg)[g]
-__host__ __device__ __forceinline__ uint32_t env_problem_index(uint32_t pk0, uint32_t pk1, uint32_t Bg, uint32_t g,
-                                                               uint32_t P) {
+// The two 32-bit draws of randint(prob_key, (Bg,), 0, P)[g] (learner:430): (k1, k2) = split(prob_key),
+// hi = bits32_at(k1, Bg, g), lo = bits32_at(k2, Bg, g).  The weighted draw (msat_env_keys_weighted) uses the same words.
+__host__ __device__ __forceinline__ void env_problem_bits(uint32_t pk0, uint32_t pk1, uint32_t Bg, uint32_t g,
+                                                          uint32_t& hi, uint32_t& lo) {
     uint32_t k1[2], k2[2];
     split2(pk0, pk1, k1, k2);
-    const uint32_t hi = bits32_at(k1[0], k1[1], Bg, g);
-    const uint32_t lo = bits32_at(k2[0], k2[1], Bg, g);
+    hi = bits32_at(k1[0], k1[1], Bg, g);
+    lo = bits32_at(k2[0], k2[1], Bg, g);
+}
+
+// jax._src.random._randint's combination of the two draws into [0, P)
+__host__ __device__ __forceinline__ uint32_t randint_from_bits(uint32_t hi, uint32_t lo, uint32_t P) {
     const uint32_t span = P > 0u ? P : 1u;
     uint32_t mult = 65536u % span;
     mult = (mult * mult) % span;
     return ((hi % span) * mult + (lo % span)) % span;
+}
+
+// problem index and reset key of global env g out of Bg (learner:430,434):
+//   randint(prob_key, (Bg,), 0, P)[g]  and  split(reset_key, Bg)[g]
+__host__ __device__ __forceinline__ uint32_t env_problem_index(uint32_t pk0, uint32_t pk1, uint32_t Bg, uint32_t g,
+                                                               uint32_t P) {
+    uint32_t hi, lo;
+    env_problem_bits(pk0, pk1, Bg, g, hi, lo);
+    return randint_from_bits(hi, lo, P);
 }
 __host__ __device__ __forceinline__ void env_reset_key(uint32_t rk0, uint32_t rk1, uint32_t Bg, uint32_t g,
                                                        uint32_t key[2]) {

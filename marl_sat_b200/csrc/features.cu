@@ -109,6 +109,67 @@ __global__ void __launch_bounds__(256) rollout_metrics_kernel(const float* __res
     }
 }
 
+// ---- per-problem statistics (msat_problem_stats) ------------------------------------------------------------
+// stats[p][0..3] += {#finished, #solved at finish, sum num_unsatisfied at finish, sum episode_step of solved-at-finish}
+// over the rows (t, b) with done != 0, p = the clamped problem index of the row.  A warp takes 32 consecutive rows; the
+// lanes whose rows end an episode of the same problem form one group (__match_any_sync) and its lowest lane adds the
+// group's sums, so a hot problem costs one update per warp instead of one per row.  kSmem: the CTA accumulates into
+// P * 4 shared counters and flushes each non-zero one with one global atomic.
+constexpr int kStatsSmemProblems = 1024;   // 32 KB of counters: six 256-thread CTAs still fit an SM's shared memory
+
+// exact sum of the int32 values of a lane group: the low 16 bits (unsigned) and the high 16 bits (signed) are reduced
+// separately, so neither 32-bit reduction can overflow
+__device__ __forceinline__ long long group_sum(unsigned grp, int v) {
+    return (long long)__reduce_add_sync(grp, v >> 16) * 65536LL + (long long)__reduce_add_sync(grp, (unsigned)v & 0xFFFFu);
+}
+
+template <bool kSmem>
+__global__ void __launch_bounds__(256) problem_stats_kernel(const int32_t* __restrict__ pidx, long long ps_t,
+                                                            long long ps_b, const uint8_t* __restrict__ done,
+                                                            const uint8_t* __restrict__ solved,
+                                                            const int32_t* __restrict__ num_unsat,
+                                                            const int32_t* __restrict__ episode_step, int T, int B,
+                                                            int P, unsigned long long* __restrict__ stats) {
+    extern __shared__ unsigned long long sacc[];          // [P][4] (kSmem)
+    if constexpr (kSmem) {
+        for (int i = threadIdx.x; i < 4 * P; i += blockDim.x) sacc[i] = 0ull;
+        __syncthreads();
+    }
+    unsigned long long* acc = kSmem ? sacc : stats;
+    const int lane = threadIdx.x & 31;
+    const long long N = (long long)T * B, stride = (long long)gridDim.x * blockDim.x;
+    // the warp's lanes share the trip count (the base is warp-aligned), so the full-warp votes below are legal
+    for (long long base = (long long)blockIdx.x * blockDim.x + (threadIdx.x & ~31); base < N; base += stride) {
+        const long long i = base + lane;
+        int p = -1, nu = 0, es = 0;
+        bool sol = false;
+        if (i < N && done[i]) {
+            const long long t = i / B, b = i - t * B;
+            p = clamp_problem(pidx[t * ps_t + b * ps_b], P);
+            sol = solved[i] != 0;
+            nu = num_unsat[i];
+            es = sol ? episode_step[i] : 0;
+        }
+        if (!__any_sync(0xffffffffu, p >= 0)) continue;
+        const unsigned sol_lanes = __ballot_sync(0xffffffffu, sol);
+        const unsigned grp = __match_any_sync(0xffffffffu, p);
+        if (p < 0) continue;
+        const unsigned nsol = __popc(grp & sol_lanes);
+        const long long snu = group_sum(grp, nu), ses = group_sum(grp, es);
+        if (lane != __ffs(grp) - 1) continue;
+        unsigned long long* row = acc + 4 * p;
+        atomicAdd(row + 0, (unsigned long long)__popc(grp));
+        if (nsol) atomicAdd(row + 1, (unsigned long long)nsol);
+        if (snu) atomicAdd(row + 2, (unsigned long long)snu);
+        if (ses) atomicAdd(row + 3, (unsigned long long)ses);
+    }
+    if constexpr (kSmem) {
+        __syncthreads();
+        for (int i = threadIdx.x; i < 4 * P; i += blockDim.x)
+            if (sacc[i]) atomicAdd(stats + i, sacc[i]);
+    }
+}
+
 // ---- greedy evaluation bookkeeping (runner:57-70) --------------------------------------------------------
 // After evaluation step t (0-based): envs that are solved for the first time record steps_to_solve = t+1
 // and a copy of their packed assignment.
@@ -209,6 +270,25 @@ cudaError_t launch_rollout_metrics(const float* reward, long long rs_t, long lon
     blocks = blocks > 148 * 8 ? 148 * 8 : (blocks < 1 ? 1 : blocks);
     rollout_metrics_kernel<<<(int)blocks, 256, 0, s>>>(reward, rs_t, rs_b, done, solved, num_unsat, episode_step, T, B,
                                                        sums);
+    return cudaGetLastError();
+}
+cudaError_t launch_problem_stats(const int32_t* pidx, long long ps_t, long long ps_b, const uint8_t* done,
+                                 const uint8_t* solved, const int32_t* num_unsat, const int32_t* episode_step, int T,
+                                 int B, int P, long long* stats, cudaStream_t s) {
+    const long long N = (long long)T * B;
+    if (N == 0) return cudaSuccess;
+    unsigned long long* out = reinterpret_cast<unsigned long long*>(stats);
+    long long blocks = (N + 256 * 8 - 1) / (256 * 8);
+    if (P <= kStatsSmemProblems) {
+        // every CTA flushes up to 4P counters: fewer, longer-lived CTAs (four per SM) keep that cost small
+        blocks = blocks > 148 * 4 ? 148 * 4 : blocks;
+        problem_stats_kernel<true><<<(int)blocks, 256, 4 * P * sizeof(unsigned long long), s>>>(
+            pidx, ps_t, ps_b, done, solved, num_unsat, episode_step, T, B, P, out);
+    } else {
+        blocks = blocks > 148 * 8 ? 148 * 8 : blocks;
+        problem_stats_kernel<false><<<(int)blocks, 256, 0, s>>>(pidx, ps_t, ps_b, done, solved, num_unsat,
+                                                                episode_step, T, B, P, out);
+    }
     return cudaGetLastError();
 }
 cudaError_t launch_eval_track(const msat_plan* plan, const uint32_t* state, const uint8_t* solved, int t, int B,

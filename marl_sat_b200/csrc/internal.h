@@ -184,8 +184,12 @@ cudaError_t launch_env(const msat_plan* plan, EnvMode mode, const EnvArgs& a, cu
 cudaError_t launch_export(const msat_plan* plan, const ExportArgs& a, cudaStream_t s);
 cudaError_t launch_rng_chain(const uint32_t* rng_in, uint32_t* chain_out, cudaStream_t s);
 cudaError_t launch_rng_split2(const uint32_t* key_in, uint32_t* out, cudaStream_t s);
+// cum_weights == NULL: the uniform randint draw; else the weighted draw of msat_env_keys_weighted
 cudaError_t launch_env_keys(const uint32_t* prob_key, const uint32_t* reset_key, int Bg, int off, int Bl, int P,
-                            int32_t* idx, uint32_t* keys, cudaStream_t s);
+                            int32_t* idx, uint32_t* keys, const long long* cum_weights, cudaStream_t s);
+cudaError_t launch_problem_stats(const int32_t* pidx, long long ps_t, long long ps_b, const uint8_t* done,
+                                 const uint8_t* solved, const int32_t* num_unsat, const int32_t* episode_step, int T,
+                                 int B, int P, long long* stats, cudaStream_t s);
 cudaError_t launch_gae(const float* reward, long long rs_t, long long rs_b, const uint8_t* done, const float* value,
                        const float* last_val, float gamma, float gamma_lambda, float* adv, float* targets, int T, int B,
                        double* stats, cudaStream_t s);

@@ -153,6 +153,17 @@ ffi::Error EnvKeys(cudaStream_t s, int64_t num_envs_global, int64_t env_offset, 
                   "msat_env_keys");
 }
 
+// weighted problem draw: cum_weights int64[P] are inclusive prefix sums of the problem weights
+ffi::Error EnvKeysWeighted(cudaStream_t s, int64_t num_envs_global, int64_t env_offset, ffi::Buffer<ffi::U32> prob_key,
+                           ffi::Buffer<ffi::U32> reset_key, ffi::Buffer<ffi::S64> cum_weights,
+                           ffi::ResultBuffer<ffi::S32> problem_idx, ffi::ResultBuffer<ffi::U32> reset_keys) {
+    return status(msat_env_keys_weighted(prob_key.typed_data(), reset_key.typed_data(), (int32_t)num_envs_global,
+                                         (int32_t)env_offset, dim0(problem_idx->dimensions()), cum_weights.typed_data(),
+                                         dim0(cum_weights.dimensions()), problem_idx->typed_data(),
+                                         reset_keys->typed_data(), s),
+                  "msat_env_keys_weighted");
+}
+
 // ---- MAPPO advantage path (learner:504-532) ---------------------------------------------------------------
 ffi::Error Gae(cudaStream_t s, double gamma, double gae_lambda, ffi::Buffer<ffi::F32> reward, ffi::Buffer<ffi::U8> done,
                ffi::Buffer<ffi::F32> value, ffi::Buffer<ffi::F32> last_val, ffi::Buffer<ffi::F64> stats_in,
@@ -205,6 +216,19 @@ ffi::Error RolloutMetrics(cudaStream_t s, ffi::Buffer<ffi::F32> reward, ffi::Buf
     return status(msat_rollout_metrics(reward.typed_data(), (int64_t)B * A, A, done.typed_data(), solved.typed_data(),
                                        num_unsatisfied.typed_data(), episode_step.typed_data(), T, B, sums->typed_data(), s),
                   "msat_rollout_metrics");
+}
+// per-problem statistics of a dense [T, B] rollout; stats_in (zeros or running totals) is aliased to stats
+ffi::Error ProblemStats(cudaStream_t s, ffi::Buffer<ffi::S32> problem_idx, ffi::Buffer<ffi::U8> done,
+                        ffi::Buffer<ffi::U8> solved, ffi::Buffer<ffi::S32> num_unsatisfied,
+                        ffi::Buffer<ffi::S32> episode_step, ffi::Buffer<ffi::S64> stats_in,
+                        ffi::ResultBuffer<ffi::S64> stats) {
+    const ffi::Dimensions dd = done.dimensions();
+    const int32_t T = dim0(dd), B = last_dim(dd);
+    (void)stats_in;
+    return status(msat_problem_stats(problem_idx.typed_data(), B, 1, done.typed_data(), solved.typed_data(),
+                                     num_unsatisfied.typed_data(), episode_step.typed_data(), T, B,
+                                     dim0(stats->dimensions()), stats->typed_data(), s),
+                  "msat_problem_stats");
 }
 ffi::Error FlipGains(cudaStream_t s, int64_t plan, int64_t num_problems, double tau, ffi::Buffer<ffi::U8> bank,
                      ffi::Buffer<ffi::U32> state, ffi::ResultBuffer<ffi::S32> delta_unsat,
@@ -284,6 +308,9 @@ XLA_FFI_DEFINE_HANDLER_SYMBOL(MsatRngSplit2, RngSplit2,
 XLA_FFI_DEFINE_HANDLER_SYMBOL(MsatEnvKeys, EnvKeys,
     ffi::Ffi::Bind().Ctx<Stream>().Attr<int64_t>("num_envs_global").Attr<int64_t>("env_offset")
         .Attr<int64_t>("num_problems").Arg<In<ffi::U32>>().Arg<In<ffi::U32>>().Ret<Out<ffi::S32>>().Ret<Out<ffi::U32>>());
+XLA_FFI_DEFINE_HANDLER_SYMBOL(MsatEnvKeysWeighted, EnvKeysWeighted,
+    ffi::Ffi::Bind().Ctx<Stream>().Attr<int64_t>("num_envs_global").Attr<int64_t>("env_offset")
+        .Arg<In<ffi::U32>>().Arg<In<ffi::U32>>().Arg<In<ffi::S64>>().Ret<Out<ffi::S32>>().Ret<Out<ffi::U32>>());
 XLA_FFI_DEFINE_HANDLER_SYMBOL(MsatGae, Gae,
     ffi::Ffi::Bind().Ctx<Stream>().Attr<double>("gamma").Attr<double>("gae_lambda")
         .Arg<In<ffi::F32>>().Arg<In<ffi::U8>>().Arg<In<ffi::F32>>().Arg<In<ffi::F32>>().Arg<In<ffi::F64>>()
@@ -301,6 +328,9 @@ XLA_FFI_DEFINE_HANDLER_SYMBOL(MsatGnnDynamic, GnnDynamic,
 XLA_FFI_DEFINE_HANDLER_SYMBOL(MsatRolloutMetrics, RolloutMetrics,
     ffi::Ffi::Bind().Ctx<Stream>().Arg<In<ffi::F32>>().Arg<In<ffi::U8>>().Arg<In<ffi::U8>>().Arg<In<ffi::S32>>()
         .Arg<In<ffi::S32>>().Arg<In<ffi::F64>>().Ret<Out<ffi::F64>>());
+XLA_FFI_DEFINE_HANDLER_SYMBOL(MsatProblemStats, ProblemStats,
+    ffi::Ffi::Bind().Ctx<Stream>().Arg<In<ffi::S32>>().Arg<In<ffi::U8>>().Arg<In<ffi::U8>>().Arg<In<ffi::S32>>()
+        .Arg<In<ffi::S32>>().Arg<In<ffi::S64>>().Ret<Out<ffi::S64>>());
 XLA_FFI_DEFINE_HANDLER_SYMBOL(MsatFlipGains, FlipGains,
     ffi::Ffi::Bind().Ctx<Stream>().Attr<int64_t>("plan").Attr<int64_t>("num_problems").Attr<double>("tau")
         .Arg<In<ffi::U8>>().Arg<In<ffi::U32>>().Ret<Out<ffi::S32>>().Ret<Out<ffi::S32>>());

@@ -32,7 +32,8 @@ TARGETS = {
     "MsatStep": "msat_step",
     "MsatRolloutSteps": "msat_rollout_steps", "MsatRolloutStepsGnn": "msat_rollout_steps_gnn",
     "MsatGetObs": "msat_get_obs", "MsatExportState": "msat_export_state", "MsatRngChain": "msat_rng_chain",
-    "MsatRngSplit2": "msat_rng_split2", "MsatEnvKeys": "msat_env_keys", "MsatGae": "msat_gae",
+    "MsatRngSplit2": "msat_rng_split2", "MsatEnvKeys": "msat_env_keys",
+    "MsatEnvKeysWeighted": "msat_env_keys_weighted", "MsatProblemStats": "msat_problem_stats", "MsatGae": "msat_gae",
     "MsatAdvStats": "msat_adv_stats", "MsatAdvNormalize": "msat_adv_normalize", "MsatGnnStatic": "msat_gnn_static",
     "MsatGnnDynamic": "msat_gnn_dynamic", "MsatRolloutMetrics": "msat_rollout_metrics",
     "MsatFlipGains": "msat_flip_gains", "MsatEvalTrack": "msat_eval_track", "MsatWalksat": "msat_walksat",
@@ -110,6 +111,29 @@ def rollout_steps(plan_handle: int, dims, bank, num_problems: int, state, action
     return call(bank, state, actions, rng, plan=np.int64(plan_handle), num_problems=np.int64(num_problems),
                 num_steps=np.int64(K), num_envs_global=np.int64(num_envs_global or B), env_offset=np.int64(env_offset),
                 emit_every_step=np.int64(1 if emit_every_step else 0))
+
+
+def env_keys_weighted(prob_key, reset_key, cum_weights, num_envs_local: int, num_envs_global=None,
+                      env_offset: int = 0):
+    """Per-env problem indices drawn with the weights whose inclusive prefix sums are ``cum_weights`` (int64 [P]) and
+    the reset keys of ``msat_env_keys``, for the shard ``[env_offset, env_offset + num_envs_local)`` -> ``(idx, keys)``.
+    The draw contract is in include/marl_sat_b200.h; int64 buffers need ``jax_enable_x64``."""
+    register()
+    B = int(num_envs_local)
+    call = jffi.ffi_call("msat_env_keys_weighted", (_sds((B,), jnp.int32), _sds((B, 2), jnp.uint32)))
+    return call(prob_key, reset_key, jnp.asarray(cum_weights, jnp.int64),
+                num_envs_global=np.int64(num_envs_global or B), env_offset=np.int64(env_offset))
+
+
+def problem_stats(problem_idx, done, solved, num_unsatisfied, episode_step, num_problems: int, stats=None):
+    """int64 ``[P, 4]`` per-problem statistics of a dense ``[T, B]`` rollout (``msat_problem_stats``), added to
+    ``stats`` (default zeros).  Needs ``jax_enable_x64``."""
+    register()
+    P = int(num_problems)
+    stats = jnp.zeros((P, 4), jnp.int64) if stats is None else stats
+    call = jffi.ffi_call("msat_problem_stats", _sds((P, 4), jnp.int64), input_output_aliases={5: 0})
+    return call(jnp.asarray(problem_idx, jnp.int32), done.astype(jnp.uint8), solved.astype(jnp.uint8),
+                jnp.asarray(num_unsatisfied, jnp.int32), jnp.asarray(episode_step, jnp.int32), stats)
 
 
 def calculate_gae(reward, done, value, last_val, gamma: float, gae_lambda: float):

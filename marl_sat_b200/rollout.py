@@ -26,7 +26,8 @@ from typing import Dict, Optional
 import torch
 
 from . import _lib
-from .env import FormulaBank, SATEnv, SATState, _ptr, _stream_ptr, as_u32_tensor, obs_empty
+from .curriculum import problem_stats, problem_weights
+from .env import ArrayLike, FormulaBank, SATEnv, SATState, _ptr, _stream_ptr, as_u32_tensor, obs_empty
 
 
 def prng_key(seed: int):
@@ -97,13 +98,24 @@ class RolloutKeys:
 
 def derive_env_keys(prob_key: Optional[torch.Tensor], reset_key: Optional[torch.Tensor], num_envs_global: int,
                     env_offset: int, num_envs_local: int, num_problems: int,
-                    problem_idx: Optional[torch.Tensor], reset_keys: Optional[torch.Tensor]) -> None:
-    """``randint(prob_key, (Bg,), 0, P)`` and ``split(reset_key, Bg)`` restricted to a shard."""
+                    problem_idx: Optional[torch.Tensor], reset_keys: Optional[torch.Tensor],
+                    cum_weights: Optional[torch.Tensor] = None) -> None:
+    """``randint(prob_key, (Bg,), 0, P)`` and ``split(reset_key, Bg)`` restricted to a shard.  With ``cum_weights``
+    (int64 ``[P]`` device tensor, inclusive prefix sums of ``curriculum.problem_weights``) the problem indices come
+    from the weighted draw of ``msat_env_keys_weighted`` instead; the reset keys are the same."""
     lib = _lib.load()
     dev = (problem_idx if problem_idx is not None else reset_keys).device
-    _lib.check(lib.msat_env_keys(_ptr(prob_key), _ptr(reset_key), num_envs_global, env_offset, num_envs_local,
-                                 num_problems, _ptr(problem_idx), _ptr(reset_keys), _stream_ptr(dev)),
-               "msat_env_keys")
+    if cum_weights is None:
+        _lib.check(lib.msat_env_keys(_ptr(prob_key), _ptr(reset_key), num_envs_global, env_offset, num_envs_local,
+                                     num_problems, _ptr(problem_idx), _ptr(reset_keys), _stream_ptr(dev)),
+                   "msat_env_keys")
+        return
+    if cum_weights.dtype != torch.int64 or tuple(cum_weights.shape) != (num_problems,) or cum_weights.device != dev:
+        raise ValueError(f"cum_weights must be an int64 [{num_problems}] tensor on {dev}")
+    _lib.check(lib.msat_env_keys_weighted(_ptr(prob_key), _ptr(reset_key), num_envs_global, env_offset,
+                                          num_envs_local, _ptr(cum_weights.contiguous()), num_problems,
+                                          _ptr(problem_idx), _ptr(reset_keys), _stream_ptr(dev)),
+               "msat_env_keys_weighted")
 
 
 class VecSATEnv:
@@ -135,6 +147,39 @@ class VecSATEnv:
         if gnn_outputs:
             self.out["gnn_assignment"] = torch.empty((B, d.n), dtype=torch.int32, device=dev)
             self.out["gnn_clause_features"] = torch.empty((B, d.m, 3), dtype=torch.float32, device=dev)
+        self._weights: Optional[torch.Tensor] = None        # quantised problem weights (host), None = uniform draw
+        self._cum_weights: Optional[torch.Tensor] = None    # their inclusive prefix sums on the device
+
+    # ------------------------------------------------------------------ weighted problem draw
+    @property
+    def problem_weights(self) -> Optional[torch.Tensor]:
+        """The quantised weights of ``set_problem_weights`` (int64 ``[P]``, host), or None for the uniform draw."""
+        return self._weights
+
+    def set_problem_weights(self, weights: Optional[ArrayLike]) -> None:
+        """Draw the problems of ``reset`` and of every auto-reset with probability proportional to ``weights``
+        (``[P]``, non-negative, not all zero; quantised by ``curriculum.problem_weights``) instead of uniformly.
+        ``None`` restores the uniform draw and the fused one-launch step.  Every rank must pass the same weights:
+        each env's draw depends only on the rng, its global index and the weights, which keeps sharded runs equal to
+        the single-device run.  The weights are validated on the host and copied into a device buffer that this env
+        allocates once, so changing them between replays of a captured CUDA graph needs no re-capture.  While
+        weights are set, ``step`` runs ``msat_rng_chain`` -> ``msat_env_keys_weighted`` -> ``msat_step`` (three
+        launches), and ``steps``, ``step_host`` and ``step_host_async`` raise ``ValueError``."""
+        if weights is None:
+            self._weights = None
+            return
+        self._install_weights(problem_weights(weights, self.bank.num_problems))
+
+    def _install_weights(self, q: torch.Tensor) -> None:
+        if self._cum_weights is None:
+            self._cum_weights = torch.empty((self.bank.num_problems,), dtype=torch.int64, device=self.state.device)
+        self._cum_weights.copy_(torch.cumsum(q, 0))
+        self._weights = q
+
+    def _require_uniform(self, what: str) -> None:
+        if self._weights is not None:
+            raise ValueError(f"{what} draws problem indices inside its fused kernel and cannot apply problem weights; "
+                             f"use step(), or set_problem_weights(None) first")
 
     # runner:289-295 -- key,_rng = split(key); idx = randint(_rng,...); reset_keys = split(_rng, B)
     def reset(self) -> Optional[torch.Tensor]:
@@ -143,7 +188,7 @@ class VecSATEnv:
         self.keys.chain[0:2].copy_(self._split_tmp[0:2])     # key
         rng = self._split_tmp[2:4]                           # _rng, used for both draws (runner:291,294)
         derive_env_keys(rng, rng, self.num_envs_global, self.env_offset, self.num_envs, self.bank.num_problems,
-                        self.new_problem_idx, self.reset_keys)
+                        self.new_problem_idx, self.reset_keys, None if self._weights is None else self._cum_weights)
         obs, _ = self.env.reset_from_bank(self.bank, self.new_problem_idx, self.reset_keys, state_out=self.state,
                                           obs_out=self.out["obs"], want_obs=self.out["obs"] is not None)
         return obs
@@ -152,12 +197,13 @@ class VecSATEnv:
         """One rollout step (learner:397-464) for this shard.  ``actions`` int32 ``[B, A]`` (mode 0) or
         ``[B, A, V]`` (mode 1) on the device.  Returns the output dict (obs of the state to continue
         from; reward/done/info are the pre-reset values, learner:467-478)."""
-        if self.gnn_outputs:
+        weighted = self._weights is not None
+        if self.gnn_outputs and not weighted:
             return self._step_gnn(actions)
-        if out is None and self.fused_keys:
+        if out is None and self.fused_keys and not weighted:
             return self._step_fast(actions)
-        out = self.out if out is None else out
-        if self.fused_keys:
+        out = self.out if out is None or self.gnn_outputs else out
+        if self.fused_keys and not weighted:
             # one launch: rng chain + per-env key derivation + step + auto-reset (msat_rollout_step)
             done, reward = out.get("done"), out.get("reward")
             _lib.check(self.env._lib.msat_rollout_step(
@@ -170,11 +216,18 @@ class VecSATEnv:
                 _stream_ptr(self.state.device)), "msat_rollout_step")
             self.keys.flip()
             return out
+        # separate launches: rng chain, per-env problem indices (weighted while weights are set) and reset keys, step
         self.keys.advance()
         derive_env_keys(self.keys.prob_key, self.keys.reset_key, self.num_envs_global, self.env_offset, self.num_envs,
-                        self.bank.num_problems, self.new_problem_idx, self.reset_keys)
-        self.env.step_into(self.bank, self.state, self.state, actions, out, auto_reset=True,
-                           new_problem_idx=self.new_problem_idx, reset_keys=self.reset_keys)
+                        self.bank.num_problems, self.new_problem_idx, self.reset_keys,
+                        self._cum_weights if weighted else None)
+        self.env.step_into(self.bank, self.state, self.state, actions, dict(out, obs=None) if self.gnn_outputs else out,
+                           auto_reset=True, new_problem_idx=self.new_problem_idx, reset_keys=self.reset_keys)
+        if self.gnn_outputs:          # the GNN input of the state to continue from, as msat_rollout_step_gnn emits it
+            _lib.check(self.env._lib.msat_gnn_dynamic(
+                self.bank.plan.handle, _ptr(self.bank.data), self.bank.num_problems, _ptr(self.state), self.num_envs,
+                _ptr(out["gnn_assignment"]), _ptr(out["gnn_clause_features"]), _stream_ptr(self.state.device)),
+                "msat_gnn_dynamic")
         return out
 
     def _step_gnn(self, actions: torch.Tensor) -> Dict[str, torch.Tensor]:
@@ -243,6 +296,7 @@ class VecSATEnv:
         """K rollout steps in ONE launch (``msat_rollout_steps``) for an action table ``[K, B, A(, V)]`` that
         does not depend on the intermediate observations (replay, open-loop evaluation, launch-bound small
         batches).  Identical results to K calls of ``step``; ``out`` from ``alloc_multi_step_outputs``."""
+        self._require_uniform("steps()")
         K = int(actions.shape[0])
         done, reward = out["done"], out["reward"]
         _lib.check(self.env._lib.msat_rollout_steps(
@@ -279,6 +333,7 @@ class VecSATEnv:
         synchronised.  Observations stay in HBM (``self.out['obs']``) where the policy consumes them.
         With ``compact_outputs`` the per-agent reward / done values (identical for all agents, env:196,260)
         travel once per env; ``host_views`` expands them without copying."""
+        self._require_uniform("step_host()")
         out, dev = self.out, self.state.device
         if actions_dev is None:
             if not hasattr(self, "_actions_dev"):
@@ -328,6 +383,7 @@ class VecSATEnv:
         action upload, the fused step and the result download of this call overlap the neighbouring steps'.
         ``actions_host`` (pinned; default ``slot['host']['actions']``) must stay untouched until the step's
         kernel has run; read the results from ``slot['host']`` after ``host_wait(slot_idx)``."""
+        self._require_uniform("step_host_async()")
         host, dev = slot["host"], self.state.device
         acts = host["actions"] if actions_host is None else actions_host
         k, cur = self.keys, self.keys._cur
@@ -415,11 +471,15 @@ class VecSATEnv:
         leaves (``variable_assignments`` [B,n], ``step`` [B], ``done`` [B,A], ``problem_idx`` [B]), the rollout rng
         chain (``RolloutKeys.chain``, 10 words), ``env_offset``, ``num_envs_global`` and a shape ``signature``.
         The packed layout never leaves the process, so the checkpoint loads into either clause-update mode, any
-        observation dtype and any later library version.  Synchronises the stream."""
+        observation dtype and any later library version.  While problem weights are set, their quantised values are
+        stored under ``problem_weights``.  Synchronises the stream."""
         st = self.sat_state()
-        return {"variable_assignments": st.variable_assignments.cpu(), "step": st.step.cpu(), "done": st.done.cpu(),
-                "problem_idx": st.problem_idx.cpu(), "rng_chain": self.keys.chain.cpu().clone(),
-                "env_offset": self.env_offset, "num_envs_global": self.num_envs_global, "signature": self._signature()}
+        sd = {"variable_assignments": st.variable_assignments.cpu(), "step": st.step.cpu(), "done": st.done.cpu(),
+              "problem_idx": st.problem_idx.cpu(), "rng_chain": self.keys.chain.cpu().clone(),
+              "env_offset": self.env_offset, "num_envs_global": self.num_envs_global, "signature": self._signature()}
+        if self._weights is not None:
+            sd["problem_weights"] = self._weights.clone()
+        return sd
 
     def load_state_dict(self, sd: Dict) -> Optional[torch.Tensor]:
         """Continue from a checkpoint of ``state_dict``: any dict with this env's signature and global batch size
@@ -427,7 +487,8 @@ class VecSATEnv:
         reset keys depend only on (rng, global env index, global batch size) (DESIGN.md section 7), so a world-1
         checkpoint loads into every rank of a world-N run, and rank checkpoints joined with
         ``merge_state_dicts`` load into any world size, with the values of an uninterrupted single-device run.
-        Returns the policy input written by ``import_state``."""
+        The problem weights are restored too: those of the checkpoint, or the uniform draw for a checkpoint without
+        them.  Returns the policy input written by ``import_state``."""
         sig = {k: int(v) for k, v in dict(sd["signature"]).items()}
         if sig != self._signature():
             raise ValueError(f"checkpoint signature {sig} does not match this env's {self._signature()}")
@@ -438,19 +499,29 @@ class VecSATEnv:
         if lo < 0 or lo + self.num_envs > rows:
             raise ValueError(f"checkpoint rows [{off}, {off + rows}) do not cover this shard's "
                              f"[{self.env_offset}, {self.env_offset + self.num_envs})")
+        weights = sd.get("problem_weights")
+        q = None if weights is None else problem_weights(weights, self.bank.num_problems)
+        if q is not None and not torch.equal(q, torch.as_tensor(weights, dtype=torch.int64)):
+            raise ValueError("checkpoint problem_weights are not quantised weights (problem_weights)")
         rows_of = lambda name: torch.as_tensor(sd[name])[lo:lo + self.num_envs]
         obs = self.import_state(rows_of("problem_idx"), rows_of("variable_assignments"), rows_of("step"),
                                 rows_of("done"), validate=True)
         self.keys.chain.copy_(as_u32_tensor(sd["rng_chain"], self.state.device).reshape(10))
+        if q is None:
+            self._weights = None
+        else:
+            self._install_weights(q)
         return obs
 
 
 def merge_state_dicts(dicts) -> Dict:
     """Join ``VecSATEnv.state_dict()`` checkpoints of adjacent shards of one run into one (rows in ``env_offset``
-    order), e.g. every rank's, which then loads into any world size."""
+    order), e.g. every rank's, which then loads into any world size.  Shards must agree on the problem weights
+    (all without, or all with equal ``problem_weights``)."""
     dicts = sorted(dicts, key=lambda sd: int(sd["env_offset"]))
     first = dicts[0]
     end = int(first["env_offset"])
+    weights = first.get("problem_weights")
     for sd in dicts:
         if int(sd["env_offset"]) != end:
             raise ValueError(f"shards are not adjacent: a gap or overlap at env {end}")
@@ -458,11 +529,17 @@ def merge_state_dicts(dicts) -> Dict:
             raise ValueError("checkpoints of different runs")
         if not torch.equal(torch.as_tensor(sd["rng_chain"]), torch.as_tensor(first["rng_chain"])):
             raise ValueError("checkpoints taken at different rollout steps (rng chains differ)")
+        w = sd.get("problem_weights")
+        if (w is None) != (weights is None) or (w is not None and not torch.equal(torch.as_tensor(w),
+                                                                                   torch.as_tensor(weights))):
+            raise ValueError("shards have different problem weights")
         end += int(sd["variable_assignments"].shape[0])
     merged = {k: torch.cat([torch.as_tensor(sd[k]) for sd in dicts])
               for k in ("variable_assignments", "step", "done", "problem_idx")}
     merged.update(rng_chain=torch.as_tensor(first["rng_chain"]).clone(), env_offset=int(first["env_offset"]),
                   num_envs_global=int(first["num_envs_global"]), signature=dict(first["signature"]))
+    if weights is not None:
+        merged["problem_weights"] = torch.as_tensor(weights).clone()
     return merged
 
 
@@ -508,6 +585,14 @@ class RolloutBuffer:
         """``Transition.info`` (learner:475; env:278-282), ``[T, B]`` each."""
         return {"solved": self.solved.view(torch.bool), "num_unsatisfied": self.num_unsatisfied,
                 "episode_step": self.episode_step}
+
+    def problem_stats(self, stats: Optional[torch.Tensor] = None, group=None) -> torch.Tensor:
+        """``curriculum.problem_stats`` of this rollout, with each row's problem read from the problem-index word of
+        its pre-step state (the episode that ends at step t started on that problem) through strides, without a
+        copy.  int64 ``[P, 4]``; added to ``stats`` when given; summed over ranks under ``torch.distributed``."""
+        pidx = self.state[:, :, (self.env.num_vars + 31) // 32 + 1]      # state words: assignment, step, problem index
+        return problem_stats(pidx, self.global_done, self.solved, self.num_unsatisfied, self.episode_step,
+                             self.bank.num_problems, stats, group)
 
     def pre_step_state(self, t: int) -> SATState:
         """The state the policy acted on at step t (source of ``Transition.local_obs`` / ``global_state`` /
