@@ -64,6 +64,9 @@ def main():
     ap.add_argument("--curriculum", choices=("none", "unsolved", "walksat"), default="none",
                     help="problem draw of auto-reset: uniform, weighted by unsolved rate, or WalkSAT-solved formulas only")
     ap.add_argument("--walksat-flips", type=int, default=10000, help="flip budget of the walksat curriculum's labelling")
+    ap.add_argument("--act-key-sampling", action="store_true",
+                    help="draw actions on the device with each step's act_key (msat_sample_actions): trajectories "
+                         "independent of the world size")
     args = ap.parse_args()
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -87,7 +90,7 @@ def main():
     torch.manual_seed(0)                       # identical initial weights on every rank
     net = MLPActorCritic(env, hidden=args.hidden)
     cfg = PPOConfig(num_steps=args.steps, update_epochs=args.epochs, minibatch_size=args.minibatch)
-    trainer = MAPPOTrainer(vec, net, cfg, seed=1)
+    trainer = MAPPOTrainer(vec, net, cfg, seed=1, act_key_sampling=args.act_key_sampling)
 
     trainer.train_cycle()                      # warm-up cycle (allocator, cuBLAS handles, NCCL channels)
     if world > 1:

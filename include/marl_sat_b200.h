@@ -329,6 +329,47 @@ int msat_env_keys_weighted(const uint32_t* prob_key, const uint32_t* reset_key,
                            const int64_t* cum_weights, int32_t num_problems,
                            int32_t* problem_idx, uint32_t* reset_keys, void* stream);
 
+/* --- policy sampling (learner:397-403) ---------------------------------------------- */
+
+/* The joint action of one rollout step, drawn on the device with the step's act_key
+ * (`rng, act_key = split(rng); action = pi.sample(seed=act_key)`, learner:397-403).
+ *
+ * Sampling contract (oracle/sampling.py restates it word for word).
+ *   - logits float32 [num_rows, C] (C = num_classes) are rows [row_offset, row_offset + num_rows) of a global
+ *     [num_rows_global, C] table: action mode 0 [B, A, V+1] is A rows per env, mode 1 [B, A, V, 2] is A*V rows.
+ *   - Key: act_key = split(rng_in)[1], the key msat_rng_chain and msat_rollout_step(s) write to chain_out[2:4]
+ *     when they advance the same rng_in.  Pass the rollout rng that the next step will advance.
+ *   - For element e = (row_offset + r) * C + c and N = num_rows_global * C:
+ *       bits_e = threefry_2x32(act_key, arange(N))[e]                      (bits32_at in csrc/common.cuh)
+ *       f_e    = bitcast_f32((bits_e >> 9) | 0x3F800000) - 1
+ *       u_e    = max(FLT_MIN, f_e * (1 - FLT_MIN) + FLT_MIN) in float32      (f_e, or FLT_MIN when f_e == 0:
+ *                jax.random.uniform(minval=finfo.tiny, maxval=1))
+ *       g_e    = -log(-log(u_e))                                             (jax.random.gumbel)
+ *   - Per row: z = log_softmax(l): M = max l, z_c = (l_c - M) - log(sum_c exp(l_c - M)) (distrax normalises the
+ *     logits of a Categorical); action = the smallest c that maximises g_c + z_c (jnp.argmax); log_prob = z_action.
+ *   - Invalid rows: a row with a NaN or +inf logit, or with every logit -inf, gets action = -1 and
+ *     log_prob = -inf (distrax's _sample_n returns -1 for such rows, and log_prob of an out-of-domain value is
+ *     -inf; the env applies -1 with the reference's gather semantics).  A -inf entry of an otherwise valid row
+ *     is never drawn.
+ *   - Floating point: bits, f and u are exact; log / exp are CUDA's accurate logf / expf, so g, z and log_prob
+ *     may differ from XLA's values in the last bits and the action only where the two best scores are within a
+ *     few ulps.
+ *   - Each output depends only on (rng_in, num_rows_global, global row, C, that row's logits): any sharding
+ *     reproduces the single-call outputs bit for bit.
+ * The JAX 0.4.29 categorical / gumbel / uniform and distrax 0.1.5 Categorical details above are restated from
+ * the published sources without JAX at hand and cannot be confirmed against it here (as SURVEY.md App. B says of
+ * Threefry); the Threefry bits (known-answer tests) and the key (the reference fixtures' act_keys) are pinned.
+ *
+ *   actions   int32 [num_rows]
+ *   log_prob  float32 [num_rows] (NULL = skip)
+ * MSAT_EINVAL: NULL logits / rng_in / actions while num_rows > 0, C < 1, a negative count or offset,
+ * row_offset + num_rows > num_rows_global.  MSAT_EALIGN: logits or log_prob not 4-byte aligned.
+ * MSAT_EUNSUPPORTED: N >= 2^32 - 1 (beyond JAX's single-block counter path).  num_rows == 0 returns MSAT_OK
+ * without touching the device. */
+int msat_sample_actions(const float* logits, int64_t num_rows_global, int64_t row_offset, int32_t num_rows,
+                        int32_t num_classes, const uint32_t* rng_in, int32_t* actions, float* log_prob,
+                        void* stream);
+
 /* --- MAPPO advantage path (learner:504-532) ------------------------------------ */
 
 /* Reverse GAE scan.  reward: float, element (t,b) at reward[t*reward_stride_t +

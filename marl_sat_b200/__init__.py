@@ -22,6 +22,7 @@ from .metrics import metrics_from_sums, rollout_metric_sums, rollout_metrics  # 
 from .evaluate import evaluate_policy  # noqa: E402
 from .local_search import WalkSATResult, walksat  # noqa: E402
 from .curriculum import problem_stats, problem_weights, unsolved_weights  # noqa: E402
+from .sampling import sample_actions  # noqa: E402
 from . import dimacs  # noqa: E402
 
 __all__ = ["SATEnv", "SATState", "FormulaBank", "create_agent_groups", "SATDataWrapper", "GNNWrapperState",
@@ -29,5 +30,5 @@ __all__ = ["SATEnv", "SATState", "FormulaBank", "create_agent_groups", "SATDataW
            "prng_key", "calculate_gae",
            "advantage_stats", "normalize_advantages", "allreduce_stats", "mean_std_from_stats", "metrics_from_sums", "GNNInput", "StaticGraph", "static_graph", "dynamic_features",
            "gnn_input_from_state", "flip_gains", "rollout_metrics", "rollout_metric_sums", "evaluate_policy", "walksat", "WalkSATResult", "problem_stats",
-           "problem_weights", "unsolved_weights", "dimacs"]
+           "problem_weights", "unsolved_weights", "sample_actions", "dimacs"]
 __version__ = "0.1.0"

@@ -14,7 +14,8 @@ from pathlib import Path
 
 CSRC = Path(__file__).resolve().parent / "csrc"
 LIB_PATH = CSRC / "libmarlsat_b200.so"
-SOURCES = ["cabi.cu", "satenv.cu", "keys.cu", "gae.cu", "features.cu", "local_search.cu", "obs_memory.cu", "dimacs.cpp"]
+SOURCES = ["cabi.cu", "satenv.cu", "keys.cu", "gae.cu", "features.cu", "local_search.cu", "obs_memory.cu", "sampling.cu",
+           "dimacs.cpp"]
 HEADERS = ["common.cuh", "internal.h", "../../include/marl_sat_b200.h"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-shared", "-Xcompiler", "-fPIC"]

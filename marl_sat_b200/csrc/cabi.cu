@@ -643,6 +643,21 @@ int msat_env_keys_weighted(const uint32_t* prob_key, const uint32_t* reset_key, 
                                    (cudaStream_t)stream));
 }
 
+int msat_sample_actions(const float* logits, int64_t num_rows_global, int64_t row_offset, int32_t num_rows,
+                        int32_t num_classes, const uint32_t* rng_in, int32_t* actions, float* log_prob, void* stream) {
+    if (num_classes < 1 || num_rows < 0 || num_rows_global < 0 || row_offset < 0) return MSAT_EINVAL;
+    if (row_offset > num_rows_global - num_rows) return MSAT_EINVAL;
+    if (num_rows > 0 && (!logits || !rng_in || !actions)) return MSAT_EINVAL;
+    if (!aligned(logits, 4) || !aligned(log_prob, 4)) return MSAT_EALIGN;
+    // one Threefry call over the whole table (JAX's single-block counter path): N + 1 must fit in 32 bits
+    if (num_rows_global >= 0xFFFFFFFFll || (unsigned long long)num_rows_global * (unsigned)num_classes >= 0xFFFFFFFFull)
+        return MSAT_EUNSUPPORTED;
+    if (num_rows == 0) return MSAT_OK;
+    const uint32_t N = (uint32_t)(num_rows_global * num_classes);
+    return cuda_rc(launch_sample_actions(logits, N, (uint32_t)row_offset, num_rows, num_classes, rng_in, actions,
+                                         log_prob, (cudaStream_t)stream));
+}
+
 int msat_problem_stats(const int32_t* problem_idx, int64_t pidx_stride_t, int64_t pidx_stride_b, const uint8_t* done,
                        const uint8_t* solved, const int32_t* num_unsatisfied, const int32_t* episode_step, int32_t T,
                        int32_t B, int32_t P, int64_t* stats, void* stream) {

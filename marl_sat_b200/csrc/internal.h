@@ -187,6 +187,9 @@ cudaError_t launch_rng_split2(const uint32_t* key_in, uint32_t* out, cudaStream_
 // cum_weights == NULL: the uniform randint draw; else the weighted draw of msat_env_keys_weighted
 cudaError_t launch_env_keys(const uint32_t* prob_key, const uint32_t* reset_key, int Bg, int off, int Bl, int P,
                             int32_t* idx, uint32_t* keys, const long long* cum_weights, cudaStream_t s);
+// N = global element count (< 2^32 - 1), C >= 1, num_rows > 0
+cudaError_t launch_sample_actions(const float* logits, uint32_t N, uint32_t row_offset, int num_rows, int C,
+                                  const uint32_t* rng_in, int32_t* actions, float* log_prob, cudaStream_t s);
 cudaError_t launch_problem_stats(const int32_t* pidx, long long ps_t, long long ps_b, const uint8_t* done,
                                  const uint8_t* solved, const int32_t* num_unsat, const int32_t* episode_step, int T,
                                  int B, int P, long long* stats, cudaStream_t s);

@@ -164,6 +164,17 @@ ffi::Error EnvKeysWeighted(cudaStream_t s, int64_t num_envs_global, int64_t env_
                   "msat_env_keys_weighted");
 }
 
+// ---- policy sampling (learner:397-403) --------------------------------------------------------------------
+// logits F32[rows, C] are rows [row_offset, row_offset + rows) of a global table of num_rows_global rows
+ffi::Error SampleActions(cudaStream_t s, int64_t num_rows_global, int64_t row_offset, ffi::Buffer<ffi::F32> logits,
+                         ffi::Buffer<ffi::U32> rng_in, ffi::ResultBuffer<ffi::S32> actions,
+                         ffi::ResultBuffer<ffi::F32> log_prob) {
+    return status(msat_sample_actions(logits.typed_data(), num_rows_global, row_offset, dim0(logits.dimensions()),
+                                      last_dim(logits.dimensions()), rng_in.typed_data(), actions->typed_data(),
+                                      log_prob->typed_data(), s),
+                  "msat_sample_actions");
+}
+
 // ---- MAPPO advantage path (learner:504-532) ---------------------------------------------------------------
 ffi::Error Gae(cudaStream_t s, double gamma, double gae_lambda, ffi::Buffer<ffi::F32> reward, ffi::Buffer<ffi::U8> done,
                ffi::Buffer<ffi::F32> value, ffi::Buffer<ffi::F32> last_val, ffi::Buffer<ffi::F64> stats_in,
@@ -311,6 +322,9 @@ XLA_FFI_DEFINE_HANDLER_SYMBOL(MsatEnvKeys, EnvKeys,
 XLA_FFI_DEFINE_HANDLER_SYMBOL(MsatEnvKeysWeighted, EnvKeysWeighted,
     ffi::Ffi::Bind().Ctx<Stream>().Attr<int64_t>("num_envs_global").Attr<int64_t>("env_offset")
         .Arg<In<ffi::U32>>().Arg<In<ffi::U32>>().Arg<In<ffi::S64>>().Ret<Out<ffi::S32>>().Ret<Out<ffi::U32>>());
+XLA_FFI_DEFINE_HANDLER_SYMBOL(MsatSampleActions, SampleActions,
+    ffi::Ffi::Bind().Ctx<Stream>().Attr<int64_t>("num_rows_global").Attr<int64_t>("row_offset")
+        .Arg<In<ffi::F32>>().Arg<In<ffi::U32>>().Ret<Out<ffi::S32>>().Ret<Out<ffi::F32>>());
 XLA_FFI_DEFINE_HANDLER_SYMBOL(MsatGae, Gae,
     ffi::Ffi::Bind().Ctx<Stream>().Attr<double>("gamma").Attr<double>("gae_lambda")
         .Arg<In<ffi::F32>>().Arg<In<ffi::U8>>().Arg<In<ffi::F32>>().Arg<In<ffi::F32>>().Arg<In<ffi::F64>>()

@@ -33,7 +33,8 @@ TARGETS = {
     "MsatRolloutSteps": "msat_rollout_steps", "MsatRolloutStepsGnn": "msat_rollout_steps_gnn",
     "MsatGetObs": "msat_get_obs", "MsatExportState": "msat_export_state", "MsatRngChain": "msat_rng_chain",
     "MsatRngSplit2": "msat_rng_split2", "MsatEnvKeys": "msat_env_keys",
-    "MsatEnvKeysWeighted": "msat_env_keys_weighted", "MsatProblemStats": "msat_problem_stats", "MsatGae": "msat_gae",
+    "MsatEnvKeysWeighted": "msat_env_keys_weighted", "MsatSampleActions": "msat_sample_actions",
+    "MsatProblemStats": "msat_problem_stats", "MsatGae": "msat_gae",
     "MsatAdvStats": "msat_adv_stats", "MsatAdvNormalize": "msat_adv_normalize", "MsatGnnStatic": "msat_gnn_static",
     "MsatGnnDynamic": "msat_gnn_dynamic", "MsatRolloutMetrics": "msat_rollout_metrics",
     "MsatFlipGains": "msat_flip_gains", "MsatEvalTrack": "msat_eval_track", "MsatWalksat": "msat_walksat",
@@ -123,6 +124,20 @@ def env_keys_weighted(prob_key, reset_key, cum_weights, num_envs_local: int, num
     call = jffi.ffi_call("msat_env_keys_weighted", (_sds((B,), jnp.int32), _sds((B, 2), jnp.uint32)))
     return call(prob_key, reset_key, jnp.asarray(cum_weights, jnp.int64),
                 num_envs_global=np.int64(num_envs_global or B), env_offset=np.int64(env_offset))
+
+
+def sample_actions(logits, rng, num_rows_global=None, row_offset: int = 0):
+    """``pi.sample(seed=act_key)`` after ``rng, act_key = split(rng)`` (learner:397-403) on the device: ``logits``
+    float32 ``[..., C]`` (rows ``[row_offset, row_offset + rows)`` of a global table of ``num_rows_global`` rows),
+    ``rng`` the rollout rng that the next ``rollout_steps`` call advances -> ``(actions int32, log_prob float32)`` of
+    shape ``logits.shape[:-1]``.  The draw contract is in include/marl_sat_b200.h."""
+    register()
+    shape, C = logits.shape[:-1], logits.shape[-1]
+    rows = int(np.prod(shape, dtype=np.int64))
+    call = jffi.ffi_call("msat_sample_actions", (_sds((rows,), jnp.int32), _sds((rows,), jnp.float32)))
+    actions, log_prob = call(jnp.asarray(logits, jnp.float32).reshape(rows, C), jnp.asarray(rng, jnp.uint32),
+                             num_rows_global=np.int64(num_rows_global or rows), row_offset=np.int64(row_offset))
+    return actions.reshape(shape), log_prob.reshape(shape)
 
 
 def problem_stats(problem_idx, done, solved, num_unsatisfied, episode_step, num_problems: int, stats=None):

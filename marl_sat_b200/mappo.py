@@ -108,9 +108,15 @@ def ppo_loss(logits: torch.Tensor, value: torch.Tensor, action: torch.Tensor, ol
 
 class MAPPOTrainer:
     """One process per GPU.  ``vec`` is this rank's shard of the env batch; ``net`` is wrapped in
-    ``DistributedDataParallel`` when ``torch.distributed`` is initialised with more than one rank."""
+    ``DistributedDataParallel`` when ``torch.distributed`` is initialised with more than one rank.
 
-    def __init__(self, vec: VecSATEnv, net: MLPActorCritic, cfg: PPOConfig, seed: int = 0, autocast: bool = True):
+    ``act_key_sampling=True`` draws the rollout's actions on the device with each step's act_key
+    (``VecSATEnv.sample_actions``, learner:397-403): the trajectories then depend only on the seed key, the network
+    and the global batch, not on the world size, and a run resumed from ``VecSATEnv.state_dict`` continues exactly.
+    The default draws with ``torch.multinomial`` and a per-rank generator."""
+
+    def __init__(self, vec: VecSATEnv, net: MLPActorCritic, cfg: PPOConfig, seed: int = 0, autocast: bool = True,
+                 act_key_sampling: bool = False):
         self.vec, self.cfg = vec, cfg
         self.env = vec.env
         self.device = vec.state.device
@@ -124,6 +130,7 @@ class MAPPOTrainer:
         self.buf = RolloutBuffer(self.env, vec.bank, cfg.num_steps, vec.num_envs)
         self.gen = torch.Generator(device=self.device).manual_seed(seed + 7919 * vec.env_offset)
         self.autocast = autocast
+        self.act_key_sampling = act_key_sampling
 
     # -- the critic's global input from a packed state -------------------------------------------------------
     def _global_features(self, state: SATState):
@@ -136,6 +143,9 @@ class MAPPOTrainer:
             logits = self.raw_net.actor_logits(vec.out["obs"])
             assignment, sat = self._global_features(vec.sat_state())
             value = self.raw_net.value(assignment, sat)
+        if self.act_key_sampling:
+            action, log_prob = vec.sample_actions(logits)
+            return action, value, log_prob
         probs = torch.softmax(logits, dim=-1)
         action = torch.multinomial(probs.reshape(-1, probs.shape[-1]), 1, generator=self.gen).reshape(probs.shape[:-1])
         log_prob = torch.log(torch.gather(probs, -1, action[..., None]).squeeze(-1).clamp_min(1e-30))

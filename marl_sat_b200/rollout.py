@@ -28,6 +28,7 @@ import torch
 from . import _lib
 from .curriculum import problem_stats, problem_weights
 from .env import ArrayLike, FormulaBank, SATEnv, SATState, _ptr, _stream_ptr, as_u32_tensor, obs_empty
+from .sampling import sample_actions
 
 
 def prng_key(seed: int):
@@ -229,6 +230,26 @@ class VecSATEnv:
                 _ptr(out["gnn_assignment"]), _ptr(out["gnn_clause_features"]), _stream_ptr(self.state.device)),
                 "msat_gnn_dynamic")
         return out
+
+    def sample_actions(self, logits: torch.Tensor, actions: Optional[torch.Tensor] = None,
+                       log_prob: Optional[torch.Tensor] = None):
+        """The joint action of the next ``step`` drawn on the device with that step's act_key (learner:397-403):
+        ``logits`` float32 ``[B, A, V+1]`` (action mode 0) or ``[B, A, V, 2]`` (mode 1) for this shard's envs ->
+        ``(actions, log_prob)`` of shape ``[B, A]`` / ``[B, A, V]``, ready for ``step``.  Rows are indexed in the global
+        batch, so every sharding draws the single-device actions, and a run resumed from ``state_dict`` draws what
+        the uninterrupted run would have drawn.  Contract: ``sampling.sample_actions``."""
+        env, B = self.env, self.num_envs
+        A, V = env.num_agents, env.max_vars_per_agent
+        shape = (B, A, V + 1) if env.action_mode == 0 else (B, A, V, 2)
+        if not isinstance(logits, torch.Tensor) or tuple(logits.shape) != shape:
+            got = tuple(logits.shape) if isinstance(logits, torch.Tensor) else type(logits).__name__
+            raise ValueError(f"logits must be {shape} for action mode {env.action_mode}, got {got}")
+        if logits.device != self.state.device:
+            raise ValueError(f"logits must be on {self.state.device}, got {logits.device}")
+        rows_per_env = A if env.action_mode == 0 else A * V
+        # the rng this env's next step advances: act_key = split(rng)[1] (msat_rng_chain's chain_out[2:4])
+        return sample_actions(logits, self.keys.chain[0:2], self.num_envs_global * rows_per_env,
+                              self.env_offset * rows_per_env, actions, log_prob)
 
     def _step_gnn(self, actions: torch.Tensor) -> Dict[str, torch.Tensor]:
         """Rollout step that emits the dynamic GNN input instead of local observations
