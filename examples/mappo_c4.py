@@ -16,7 +16,12 @@ Rank 0 prints one JSON line: updates/s, env-steps/s of the whole cycle, the roll
   unsolved  per-problem statistics of every rollout are accumulated (``RolloutBuffer.problem_stats``) and after each
             update the weights become ``unsolved_weights`` of the totals;
   walksat   one WalkSAT call over a reset of every bank formula labels the formulas it solves; only those are drawn.
-The JSON line then also reports the share of the bank solved at least once during the timed updates.
+  reverse   the walksat draw, and every episode starts at its formula's WalkSAT solution with each bit flipped with
+            probability q (``set_start_states``; q starts at --start-flip-prob).  After every update
+            ``adapt_flip_prob`` moves each formula's q with that rollout's solve rate: up where the policy solves
+            it, down where it does not (a reverse curriculum).
+The JSON line then also reports the share of the bank solved at least once during the timed updates (and, for
+reverse, the mean q and the share of formulas at q_max).
 Reference structure: src/learners/mappo_gnn_sat_learner.py:381-732, configs/MAPPO_CONFIG.yaml:27-48.
 """
 import argparse
@@ -32,19 +37,24 @@ import torch.distributed as dist
 sys.path.insert(0, str(Path(__file__).resolve().parent.parent))
 import marl_sat_b200 as M                                           # noqa: E402
 from marl_sat_b200 import synth                                     # noqa: E402
+from marl_sat_b200.curriculum import adapt_flip_prob                 # noqa: E402
 from marl_sat_b200.mappo import MAPPOTrainer, MLPActorCritic, PPOConfig    # noqa: E402
 
+Q_MAX = 0.5          # adapt_flip_prob's default ceiling: a start as random as the reference's draw
 
-def walksat_solvable(M, env, bank, max_flips, dev) -> torch.Tensor:
-    """bool [P]: the formulas one WalkSAT call (noise 0.5) solves from a reset of every bank formula."""
+
+def walksat_solvable(M, env, bank, max_flips, dev):
+    """bool [P]: the formulas one WalkSAT call (noise 0.5) solves from a reset of every bank formula, and int32 [P, n]
+    the searched assignments (row p is formula p; a solution where solved)."""
     P = bank.num_problems
     idx = torch.arange(P, dtype=torch.int32, device=dev)
     keys = M.env.as_u32_tensor(torch.stack([torch.zeros(P, dtype=torch.int64), torch.arange(P)], 1), dev)
     _, state = env.reset_from_bank(bank, idx, keys, want_obs=False)
-    solved = M.walksat(state, keys, max_flips).solved.cpu()
+    res = M.walksat(state, keys, max_flips)
+    solved = res.solved.cpu()
     if not bool(solved.any()):
         raise SystemExit(f"WalkSAT solved none of the {P} formulas in {max_flips} flips: nothing to train on")
-    return solved
+    return solved, res.state.variable_assignments
 
 
 def main():
@@ -61,8 +71,11 @@ def main():
     ap.add_argument("--hidden", type=int, default=128)
     ap.add_argument("--obs-int8", action="store_true",
                     help="int8 observations (MSAT_OBS_INT8): same values, a quarter of the bytes the policy reads")
-    ap.add_argument("--curriculum", choices=("none", "unsolved", "walksat"), default="none",
-                    help="problem draw of auto-reset: uniform, weighted by unsolved rate, or WalkSAT-solved formulas only")
+    ap.add_argument("--curriculum", choices=("none", "unsolved", "walksat", "reverse"), default="none",
+                    help="problem draw of auto-reset: uniform, weighted by unsolved rate, or WalkSAT-solved formulas "
+                         "only; reverse also starts episodes near the WalkSAT solutions")
+    ap.add_argument("--start-flip-prob", type=float, default=0.05,
+                    help="initial per-bit flip probability q of the reverse curriculum's starts")
     ap.add_argument("--walksat-flips", type=int, default=10000, help="flip budget of the walksat curriculum's labelling")
     ap.add_argument("--act-key-sampling", action="store_true",
                     help="draw actions on the device with each step's act_key (msat_sample_actions): trajectories "
@@ -82,10 +95,13 @@ def main():
     problems = synth.uniform_ksat_torch(args.problems, args.n, args.m, 3, seed=20261018 + 4, device=dev)
     bank = env.make_bank(problems, validate=False)
     vec = M.VecSATEnv(env, bank, args.envs, M.prng_key(42), world_size=world, rank=rank, compact_outputs=True)
-    labelled = None
-    if args.curriculum == "walksat":
-        labelled = walksat_solvable(M, env, bank, args.walksat_flips, dev)
+    labelled = solutions = flip_prob = None
+    if args.curriculum in ("walksat", "reverse"):
+        labelled, solutions = walksat_solvable(M, env, bank, args.walksat_flips, dev)
         vec.set_problem_weights(labelled)           # identical on every rank: same bank, same keys
+    if args.curriculum == "reverse":
+        flip_prob = torch.full((bank.num_problems,), float(args.start_flip_prob), dtype=torch.float64)
+        vec.set_start_states(solutions, flip_prob, has_start=labelled)
     vec.reset()
     torch.manual_seed(0)                       # identical initial weights on every rank
     net = MLPActorCritic(env, hidden=args.hidden)
@@ -106,6 +122,9 @@ def main():
             trainer.buf.problem_stats(totals)   # this rollout's counters, summed over the ranks, added to the totals
         if args.curriculum == "unsolved":
             vec.set_problem_weights(M.unsolved_weights(totals))
+        if args.curriculum == "reverse":              # this rollout's rates, identical on every rank
+            flip_prob = adapt_flip_prob(trainer.buf.problem_stats(), flip_prob)
+            vec.set_start_states(solutions, flip_prob, has_start=labelled)
         split += torch.tensor([last["rollout_ms"], last["gae_metrics_ms"], last["update_ms"]], dtype=torch.float64,
                               device=dev)
     torch.cuda.synchronize()
@@ -144,6 +163,10 @@ def main():
             "bank_share_solved_at_least_once": (None if args.curriculum == "none"
                                                 else float((totals[:, 1] > 0).double().mean())),
             "bank_share_walksat_solved": None if labelled is None else float(labelled.double().mean()),
+            "start_flip_prob_mean": (None if flip_prob is None
+                                     else float(flip_prob[labelled].mean())),
+            "start_share_at_q_max": (None if flip_prob is None
+                                     else float((flip_prob[labelled] >= Q_MAX).double().mean())),
         }))
     if world > 1:
         dist.barrier()

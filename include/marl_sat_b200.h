@@ -120,6 +120,48 @@ int msat_import_state(const msat_plan* plan, const void* bank, int32_t num_probl
                       const int32_t* step, const uint8_t* done,
                       uint32_t* state_out, int32_t* obs, int32_t num_envs, void* stream);
 
+/* Start states for reset episodes (a reverse curriculum: episodes start at or near a known solution, e.g. one
+ * msat_walksat found, and move further away as the policy succeeds).  Call it right after msat_reset or an
+ * auto-resetting step (msat_rollout_step, msat_rollout_step_gnn, msat_rollout_steps with
+ * num_steps = 1, msat_step with auto_reset) with the reset_key that call used: it
+ * rewrites, in place, the envs that restarted on a problem with a start state.
+ *
+ * Start-state contract (oracle/start_states.py restates it word for word).
+ *   - Env b is rewritten iff its state record has step == 0 and has_start[p] != 0, with p its problem index clamped
+ *     into [0, num_problems) as msat_reset clamps it.  step == 0 is what msat_reset and an auto-reset leave (and
+ *     msat_import_state given step 0); every env that did not restart has step >= 1.  Nothing is written for any
+ *     other env, not even its observation row.
+ *   - Key: K = split(reset_key, num_envs_global)[g] for the global env g = env_offset + b -- the key msat_env_keys
+ *     and the fused step derive -- and (ka, kb) = split(K).  randint reads only kb (env:162); the perturbation word
+ *     of variable v is u_v = threefry_2x32(ka, arange(n))[v] (randint's counter layout), so the flips are
+ *     independent of the reference draw and cost the same ceil(n/2) Threefry blocks.
+ *   - Assignment: bit v = (start bit v) XOR (u_v < flip_thr[p]); flip_thr = 0 reproduces the start exactly.
+ *     A flip probability q in [0, 1] is quantised on the host as flip_thr = min(round(q * 2^32), 2^32 - 1), so
+ *     every bit flips with probability flip_thr / 2^32: q = 1 misses a flip with probability 2^-32.
+ *   - State: clause status, num_unsatisfied and, on an MSAT_CLAUSES_INCREMENTAL plan, the 4-bit true-literal counts
+ *     are recomputed from the bank record as msat_import_state does; step, problem index and done stay 0 / p / 0.
+ *   - Outputs: obs (int32 or int8, following the plan) and the GNN inputs gnn_assignment int32[B,n] /
+ *     gnn_clause_features float[B,m,3] are rewritten for the rewritten envs only, equal to msat_get_obs and
+ *     msat_gnn_dynamic of the new state.  Any of them may be NULL.
+ *   - Each result depends only on (reset_key, num_envs_global, g, p, the tables), so any sharding reproduces the
+ *     single-device values.
+ *
+ *   state        uint32[B, state_words], read and written in place
+ *   start_words  uint32[num_problems, ceil(n/32)], packed like the state's assignment words (bit v % 32 of word
+ *                v / 32); bits past n are ignored
+ *   flip_thr     uint32[num_problems]
+ *   has_start    uint8[num_problems], NULL = every problem has a start
+ * MSAT_EINVAL: missing pointers while num_envs > 0, a negative count or offset, num_problems <= 0,
+ * env_offset + num_envs > num_envs_global.  MSAT_EALIGN as msat_import_state (bank 128 bytes, state and obs
+ * 16 bytes), the tables and GNN outputs 4 bytes.  MSAT_EUNSUPPORTED: num_envs_global > 2^30, or clause features
+ * with lits_per_clause > 15.  num_envs == 0 returns MSAT_OK without touching the device. */
+int msat_apply_start_states(const msat_plan* plan, const void* bank, int32_t num_problems,
+                            uint32_t* state, const uint32_t* reset_key,
+                            int32_t num_envs_global, int32_t env_offset,
+                            const uint32_t* start_words, const uint32_t* flip_thr, const uint8_t* has_start,
+                            int32_t* obs, int32_t* gnn_assignment, float* gnn_clause_features,
+                            int32_t num_envs, void* stream);
+
 /* Replaces `jax.vmap(SATEnv.step_env)` (env:225-284) and, with auto_reset != 0,
  * the reset-and-select of the rollout loop (learner:422-464) in the same launch.
  *   actions        int32 [B, A] (mode 0) or [B, A, V] (mode 1)

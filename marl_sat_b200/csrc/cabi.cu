@@ -297,6 +297,37 @@ int msat_import_state(const msat_plan* plan, const void* bank, int32_t P, const 
     return cuda_rc(launch_env(plan, MODE_IMPORT, a, (cudaStream_t)stream));
 }
 
+int msat_apply_start_states(const msat_plan* plan, const void* bank, int32_t P, uint32_t* state,
+                            const uint32_t* reset_key, int32_t Bg, int32_t env_offset, const uint32_t* start_words,
+                            const uint32_t* flip_thr, const uint8_t* has_start, int32_t* obs, int32_t* gnn_assignment,
+                            float* gnn_clause_features, int32_t B, void* stream) {
+    if (!plan || B < 0 || Bg < 0 || env_offset < 0 || P <= 0 || (long long)env_offset + B > Bg) return MSAT_EINVAL;
+    if (B > 0 && (!bank || !state || !reset_key || !start_words || !flip_thr)) return MSAT_EINVAL;
+    if (!aligned(bank, 128) || !aligned(state, 16) || !aligned(obs, 16) || !aligned(start_words, 4) ||
+        !aligned(flip_thr, 4) || !aligned(gnn_assignment, 4) || !aligned(gnn_clause_features, 4))
+        return MSAT_EALIGN;
+    if (Bg > (1 << 30)) return MSAT_EUNSUPPORTED;
+    if (gnn_clause_features && plan->d.k > 15) return MSAT_EUNSUPPORTED;   // 16-entry feature table
+    if (B == 0) return MSAT_OK;
+    EnvArgs a{};
+    a.bank = static_cast<const uint8_t*>(bank); a.P = P;
+    a.state_in = state; a.state_out = state; a.B = B;
+    a.Bg = (uint32_t)Bg; a.env_off = (uint32_t)env_offset; a.reset_key = reset_key;
+    a.start_words = start_words; a.flip_thr = flip_thr; a.has_start = has_start;
+    // observations and GNN inputs come from differently shaped launches; the rewrite depends only on the key and
+    // the tables, so the second launch selects the same envs and writes the same states again
+    cudaError_t e = cudaSuccess;
+    if (obs || !(gnn_assignment || gnn_clause_features)) {
+        a.obs = obs;
+        e = launch_env(plan, MODE_START, a, (cudaStream_t)stream);
+    }
+    if (e == cudaSuccess && (gnn_assignment || gnn_clause_features)) {
+        a.obs = nullptr; a.gnn_assign = gnn_assignment; a.gnn_cf = gnn_clause_features;
+        e = launch_env(plan, MODE_START, a, (cudaStream_t)stream);
+    }
+    return cuda_rc(e);
+}
+
 int msat_walksat(const msat_plan* plan, const void* bank, int32_t P, uint32_t* state, const uint32_t* keys,
                  int32_t max_flips, int32_t flip_offset, double noise, uint8_t* solved, int32_t* flips, int32_t B,
                  void* stream) {

@@ -108,10 +108,19 @@ struct EnvArgs {
     const int32_t* assign_in;
     const int32_t* step_in;
     const uint8_t* done_in;
+    // start states (msat_apply_start_states): per-problem packed start assignments uint32[P, aw], flip thresholds
+    // uint32[P] and flags uint8[P] (NULL = every problem has a start); the envs' reset key is derived from
+    // reset_key with the global env index (Bg, env_off)
+    const uint32_t* start_words;
+    const uint32_t* flip_thr;
+    const uint8_t* has_start;
+    const uint32_t* reset_key;
 };
 
 // MODE_IMPORT: the reset path with the assignment, step and done flag read from memory
-enum EnvMode { MODE_RESET = 0, MODE_STEP = 1, MODE_OBS = 2, MODE_IMPORT = 3 };
+// MODE_START: the reset path for the envs that just restarted (step == 0) on a problem with a start state, with the
+// assignment taken from that start and flipped by bits drawn from the env's reset key; every other env is left alone
+enum EnvMode { MODE_RESET = 0, MODE_STEP = 1, MODE_OBS = 2, MODE_IMPORT = 3, MODE_START = 4 };
 
 extern int g_gae_force_plain;   // gae.cu; msat_tune("gae_plain", 1)
 extern int g_gae_variant;       // gae.cu; msat_tune("gae_variant", v)

@@ -469,6 +469,31 @@ __device__ __forceinline__ void load_assign(const Dims& d, const int32_t* __rest
     }
 }
 
+// Start state (msat_apply_start_states) into zeroed assignment words: bit v = start bit v XOR (u_v < thr), where
+// u_v = threefry_2x32(ka, arange(n))[v] and (ka, kb) = split(key) -- the half of the key randint leaves unused
+// (threefry_assign reads kb), with randint's counter layout.  Start bits past n are dropped.  XOR commutes, so
+// the start words and the flips go in with atomics in any order.
+template <int GS>
+__device__ __forceinline__ void start_assign(const Dims& d, const uint32_t* __restrict__ start, uint32_t thr,
+                                             uint32_t k0, uint32_t k1, uint32_t* assign, int gt) {
+    for (int w = gt; w < d.aw; w += GS) {
+        const int tail = d.n - 32 * w;
+        const uint32_t word = start[w] & (tail >= 32 ? 0xFFFFFFFFu : (1u << tail) - 1u);
+        if (word) atomicXor(&assign[w], word);
+    }
+    uint32_t ka[2], kb[2];
+    split2(k0, k1, ka, kb);
+    const int half = (d.n + 1) >> 1;
+    for (int i = gt; i < half; i += GS) {
+        uint32_t x0 = (uint32_t)i;
+        uint32_t x1 = (half + i < d.n) ? (uint32_t)(half + i) : 0u;
+        threefry2x32(ka[0], ka[1], x0, x1);
+        if (x0 < thr) atomicXor(&assign[i >> 5], 1u << (i & 31));
+        const int v = half + i;
+        if (v < d.n && x1 < thr) atomicXor(&assign[v >> 5], 1u << (v & 31));
+    }
+}
+
 // Decode all agents' actions of env e (env:233-250) and call flip(v) once for every variable that flips; the flips
 // are simultaneous, so flip must commute (atomics).  has_pre: the caller already holds act[gt] (mode 0) in `pre`
 // (loaded early, next to the state record).
@@ -733,12 +758,15 @@ __device__ __forceinline__ void rng_advance(uint32_t& r0, uint32_t& r1) {
 // MULTI = K steps per launch (msat_rollout_steps); INCR = incremental clause update (step launches of a plan
 // with MSAT_CLAUSES_INCREMENTAL that write no observations).
 // MODE_IMPORT (msat_import_state) is the reset with the assignment, step and done flag taken from memory.
+// MODE_START (msat_apply_start_states) is the reset of the envs that just restarted on a problem with a start state,
+// in place, with the assignment built from that start (start_assign); the other groups leave after reading two words.
 // =====================================================================================
 template <int GS, int MODE, bool OBS, bool MULTI, bool INCR>
 __global__ void __launch_bounds__(kCtaThreads, (MULTI || !OBS) ? 4 : 8) env_kernel(const Dims d, const EnvArgs a) {
     extern __shared__ __align__(128) uint8_t smem_raw[];
     constexpr int NG = kCtaThreads / GS;
-    constexpr bool FRESH = MODE == MODE_RESET || MODE == MODE_IMPORT;    // builds a state instead of reading one
+    // builds a state instead of reading one
+    constexpr bool FRESH = MODE == MODE_RESET || MODE == MODE_IMPORT || MODE == MODE_START;
     const int gid = threadIdx.x / GS, gt = threadIdx.x % GS;
     const int e = blockIdx.x * NG + gid;
     const GroupLayout& L = a.L;
@@ -765,6 +793,14 @@ __global__ void __launch_bounds__(kCtaThreads, (MULTI || !OBS) ? 4 : 8) env_kern
         if (blockIdx.x == 0 && threadIdx.x < 10) a.chain_out[threadIdx.x] = s_chain[10 * (K - 1) + threadIdx.x];
     }
     if (e >= a.B) return;   // whole group leaves together
+    int start_pidx = 0;
+    if constexpr (MODE == MODE_START) {
+        // only an env that has just (re)started (step 0) on a problem with a start is rewritten; the group reads the
+        // same two words in every lane, so it leaves together
+        const uint32_t* tail = a.state_in + (size_t)e * d.state_words + d.aw;
+        start_pidx = clamp_problem((int)tail[ST_PIDX], a.P);
+        if (tail[ST_STEP] != 0u || (a.has_start && !a.has_start[start_pidx])) return;
+    }
 
     uint8_t* base = smem_raw + (size_t)gid * L.total;
     uint8_t* rec = base + L.rec;
@@ -825,13 +861,14 @@ __global__ void __launch_bounds__(kCtaThreads, (MULTI || !OBS) ? 4 : 8) env_kern
     // them in shared memory only after the last step, and a warp that read `step` from shared memory after
     // such a write would disagree with the others about `done` and wait at a group barrier nobody else reaches.
     // an imported step is stored verbatim: states exported after stepping past `done` carry step >= max_steps
-    int step_cur = (MODE == MODE_RESET) ? 0
+    int step_cur = (MODE == MODE_RESET || MODE == MODE_START) ? 0
                  : (MODE == MODE_IMPORT) ? (a.step_in ? a.step_in[e] : 0) : (int)st_tail[ST_STEP];
     int nunsat_prev = FRESH ? 0 : (int)st_tail[ST_NUNSAT];
-    uint32_t flags = (MODE == MODE_RESET) ? 0u
+    uint32_t flags = (MODE == MODE_RESET || MODE == MODE_START) ? 0u
                    : (MODE == MODE_IMPORT) ? ((a.done_in && a.done_in[e]) ? 1u : 0u) : st_tail[ST_FLAGS];
     int pidx;
-    if (FRESH) pidx = a.prob_idx[e];
+    if (MODE == MODE_START) pidx = start_pidx;
+    else if (FRESH) pidx = a.prob_idx[e];
     else pidx = (int)st_tail[ST_PIDX];
     pidx = clamp_problem(pidx, a.P);
     int loaded_pidx = -1;           // formula whose block sits in the record slot ...
@@ -882,6 +919,11 @@ __global__ void __launch_bounds__(kCtaThreads, (MULTI || !OBS) ? 4 : 8) env_kern
             threefry_assign<GS>(d, a.keys[2 * (size_t)e], a.keys[2 * (size_t)e + 1], st, gt);
         } else if (MODE == MODE_IMPORT) {
             load_assign<GS>(d, a.assign_in + (size_t)e * d.n, st, gt);
+        } else if (MODE == MODE_START) {
+            // the env's reset key, as msat_env_keys and the fused step derive it: split(reset_key, Bg)[env_off + e]
+            uint32_t key[2];
+            env_reset_key(a.reset_key[0], a.reset_key[1], a.Bg, a.env_off + (uint32_t)e, key);
+            start_assign<GS>(d, a.start_words + (size_t)pidx * d.aw, a.flip_thr[pidx], key[0], key[1], st, gt);
         } else if (MODE == MODE_STEP) {
             if (INCR) {
                 if (need_csr) {
@@ -1067,11 +1109,12 @@ static cudaError_t launch_env_gs(const msat_plan* plan, EnvMode mode, const EnvA
     // every instantiation a launch with this (GS, OBS) can select: the shared-memory opt-in below covers them all.
     // The single-step kernels sit at index `mode`, then the multi-step one, then the incremental clause update's
     // single- and multi-step kernels (step launches without observations on a plan that carries the counts).
-    constexpr int kFns = OBS ? 5 : 7;
-    const void* fns[7] = {(const void*)env_kernel<GS, MODE_RESET, OBS, false, false>,
+    constexpr int kFns = OBS ? 6 : 8;
+    const void* fns[8] = {(const void*)env_kernel<GS, MODE_RESET, OBS, false, false>,
                           (const void*)env_kernel<GS, MODE_STEP, OBS, false, false>,
                           (const void*)env_kernel<GS, MODE_OBS, OBS, false, false>,
                           (const void*)env_kernel<GS, MODE_IMPORT, OBS, false, false>,
+                          (const void*)env_kernel<GS, MODE_START, OBS, false, false>,
                           (const void*)env_kernel<GS, MODE_STEP, OBS, true, false>,
                           OBS ? nullptr : (const void*)env_kernel<GS, MODE_STEP, false, false, true>,
                           OBS ? nullptr : (const void*)env_kernel<GS, MODE_STEP, false, true, true>};
@@ -1092,7 +1135,7 @@ static cudaError_t launch_env_gs(const msat_plan* plan, EnvMode mode, const EnvA
             plan->prepared_devices.fetch_or(bit, std::memory_order_release);
         }
     }
-    const void* fn = fns[incr ? 5 + (int)multi : (multi ? 4 : (int)mode)];
+    const void* fn = fns[incr ? 6 + (int)multi : (multi ? 5 : (int)mode)];
     Dims d = plan->d;
     EnvArgs args = a;
     void* params[] = {&d, &args};

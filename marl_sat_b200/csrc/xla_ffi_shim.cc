@@ -271,6 +271,22 @@ ffi::Error Walksat(cudaStream_t s, int64_t plan, int64_t num_problems, int64_t m
                   "msat_walksat");
 }
 
+// start states after a reset / auto-resetting step, in place (state_in is aliased to state); the envs that restarted
+// on a problem with a start get it, with seeded flips, and their observations
+ffi::Error ApplyStartStates(cudaStream_t s, int64_t plan, int64_t num_problems, int64_t num_envs_global,
+                            int64_t env_offset, ffi::Buffer<ffi::U8> bank, ffi::Buffer<ffi::U32> state_in,
+                            ffi::Buffer<ffi::U32> reset_key, ffi::Buffer<ffi::U32> start_words,
+                            ffi::Buffer<ffi::U32> flip_thr, ffi::Buffer<ffi::U8> has_start,
+                            ffi::Buffer<ffi::S32> obs_in, ffi::ResultBuffer<ffi::U32> state,
+                            ffi::ResultBuffer<ffi::S32> obs) {
+    (void)state_in; (void)obs_in;      // aliased to the results (rows of envs without a new start stay as they are)
+    return status(msat_apply_start_states(plan_of(plan), bank.typed_data(), (int32_t)num_problems, state->typed_data(),
+                                          reset_key.typed_data(), (int32_t)num_envs_global, (int32_t)env_offset,
+                                          start_words.typed_data(), flip_thr.typed_data(), has_start.typed_data(),
+                                          obs->typed_data(), nullptr, nullptr, dim0(state->dimensions()), s),
+                  "msat_apply_start_states");
+}
+
 template <ffi::DataType T> using In = ffi::Buffer<T>;
 template <ffi::DataType T> using Out = ffi::Buffer<T>;
 using Stream = ffi::PlatformStream<cudaStream_t>;
@@ -356,3 +372,7 @@ XLA_FFI_DEFINE_HANDLER_SYMBOL(MsatWalksat, Walksat,
     ffi::Ffi::Bind().Ctx<Stream>().Attr<int64_t>("plan").Attr<int64_t>("num_problems").Attr<int64_t>("max_flips")
         .Attr<int64_t>("flip_offset").Attr<double>("noise").Arg<In<ffi::U8>>().Arg<In<ffi::U32>>().Arg<In<ffi::U32>>()
         .Ret<Out<ffi::U32>>().Ret<Out<ffi::U8>>().Ret<Out<ffi::S32>>());
+XLA_FFI_DEFINE_HANDLER_SYMBOL(MsatApplyStartStates, ApplyStartStates,
+    ffi::Ffi::Bind().Ctx<Stream>().Attr<int64_t>("plan").Attr<int64_t>("num_problems").Attr<int64_t>("num_envs_global")
+        .Attr<int64_t>("env_offset").Arg<In<ffi::U8>>().Arg<In<ffi::U32>>().Arg<In<ffi::U32>>().Arg<In<ffi::U32>>()
+        .Arg<In<ffi::U32>>().Arg<In<ffi::U8>>().Arg<In<ffi::S32>>().Ret<Out<ffi::U32>>().Ret<Out<ffi::S32>>());

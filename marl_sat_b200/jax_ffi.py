@@ -38,6 +38,7 @@ TARGETS = {
     "MsatAdvStats": "msat_adv_stats", "MsatAdvNormalize": "msat_adv_normalize", "MsatGnnStatic": "msat_gnn_static",
     "MsatGnnDynamic": "msat_gnn_dynamic", "MsatRolloutMetrics": "msat_rollout_metrics",
     "MsatFlipGains": "msat_flip_gains", "MsatEvalTrack": "msat_eval_track", "MsatWalksat": "msat_walksat",
+    "MsatApplyStartStates": "msat_apply_start_states",
 }
 _registered = False
 
@@ -95,6 +96,24 @@ def walksat(plan_handle: int, bank, num_problems: int, state, keys, max_flips: i
     return call(bank, state, jnp.asarray(keys, jnp.uint32), plan=np.int64(plan_handle),
                 num_problems=np.int64(num_problems), max_flips=np.int64(max_flips), flip_offset=np.int64(flip_offset),
                 noise=np.float64(noise))
+
+
+def apply_start_states(plan_handle: int, bank, num_problems: int, state, obs, reset_key, start_words, flip_thr,
+                       has_start=None, num_envs_global=None, env_offset: int = 0):
+    """Start states for the envs that just restarted (``msat_apply_start_states``; contract in
+    include/marl_sat_b200.h): call after ``reset`` or ``rollout_steps`` with the reset key that call used
+    (``chain[8:10]`` of ``rollout_steps``).  ``state`` and ``obs`` are donated (rows of other envs are kept);
+    ``start_words`` uint32 [P, ceil(n/32)], ``flip_thr`` uint32 [P] and ``has_start`` uint8 [P] (default all
+    ones) as ``curriculum.start_table`` returns them.  Returns ``(state, obs)``."""
+    register()
+    P = int(num_problems)
+    has_start = jnp.ones((P,), jnp.uint8) if has_start is None else jnp.asarray(has_start, jnp.uint8)
+    call = jffi.ffi_call("msat_apply_start_states", (_sds(state.shape, jnp.uint32), _sds(obs.shape, jnp.int32)),
+                         input_output_aliases={1: 0, 6: 1})
+    return call(bank, state, jnp.asarray(reset_key, jnp.uint32), jnp.asarray(start_words, jnp.uint32),
+                jnp.asarray(flip_thr, jnp.uint32), has_start, obs, plan=np.int64(plan_handle),
+                num_problems=np.int64(P), num_envs_global=np.int64(num_envs_global or state.shape[0]),
+                env_offset=np.int64(env_offset))
 
 
 def rollout_steps(plan_handle: int, dims, bank, num_problems: int, state, actions, rng, num_envs_global=None,

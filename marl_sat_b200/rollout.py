@@ -23,10 +23,11 @@ from __future__ import annotations
 import ctypes as C
 from typing import Dict, Optional
 
+import numpy as np
 import torch
 
 from . import _lib
-from .curriculum import problem_stats, problem_weights
+from .curriculum import StartTable, problem_stats, problem_weights, start_table
 from .env import ArrayLike, FormulaBank, SATEnv, SATState, _ptr, _stream_ptr, as_u32_tensor, obs_empty
 from .sampling import sample_actions
 
@@ -150,6 +151,8 @@ class VecSATEnv:
             self.out["gnn_clause_features"] = torch.empty((B, d.m, 3), dtype=torch.float32, device=dev)
         self._weights: Optional[torch.Tensor] = None        # quantised problem weights (host), None = uniform draw
         self._cum_weights: Optional[torch.Tensor] = None    # their inclusive prefix sums on the device
+        self._start: Optional[StartTable] = None             # start-state tables (host), None = random starts
+        self._start_dev: Optional[Dict[str, torch.Tensor]] = None   # their device copies, allocated once
 
     # ------------------------------------------------------------------ weighted problem draw
     @property
@@ -182,6 +185,59 @@ class VecSATEnv:
             raise ValueError(f"{what} draws problem indices inside its fused kernel and cannot apply problem weights; "
                              f"use step(), or set_problem_weights(None) first")
 
+    # ------------------------------------------------------------------ start states (reverse curriculum)
+    @property
+    def start_states(self) -> Optional[StartTable]:
+        """The tables of ``set_start_states`` (``curriculum.StartTable``, host), or None for random starts."""
+        return self._start
+
+    def set_start_states(self, assignments: Optional[ArrayLike], flip_prob=0.0,
+                         has_start: Optional[ArrayLike] = None) -> None:
+        """Start every reset episode of a problem with a start at that problem's stored assignment, each bit flipped
+        with probability ``flip_prob`` (a scalar or ``[P]``), instead of at the random draw (a reverse curriculum).
+        ``assignments`` ``[P, n]`` (nonzero = 1; e.g. WalkSAT solutions), ``has_start`` ``[P]`` (default every
+        problem); the tables are built by ``curriculum.start_table``.  While starts are set, ``reset`` and every
+        ``step`` end with ``msat_apply_start_states`` on that call's reset key, so only envs that just restarted are
+        rewritten, and each one's start depends only on the rng, its global index and the tables: sharded runs equal
+        the single-device run.  The device tables are allocated once and updated in place, so a captured CUDA graph
+        picks up new values without re-capture.  ``steps``, ``step_host`` and ``step_host_async`` raise
+        ``ValueError`` while starts are set.  ``None`` removes the extra launch."""
+        if assignments is None:
+            self._start = None
+            return
+        d = self.bank.plan.dims
+        shape = tuple(assignments.shape) if hasattr(assignments, "shape") else np.shape(assignments)
+        if tuple(shape) != (self.bank.num_problems, d.n):
+            raise ValueError(f"start assignments must be [{self.bank.num_problems}, {d.n}], got {tuple(shape)}")
+        self._install_starts(start_table(assignments, flip_prob, has_start))
+
+    def _install_starts(self, table: StartTable) -> None:
+        dev = self.state.device
+        if self._start_dev is None:
+            P, aw = table.words.shape
+            self._start_dev = {"words": torch.empty((P, aw), dtype=torch.int32, device=dev),
+                               "flip_thr": torch.empty((P,), dtype=torch.int32, device=dev),
+                               "has_start": torch.empty((P,), dtype=torch.uint8, device=dev)}
+        t = self._start_dev
+        t["words"].copy_(table.words)
+        t["flip_thr"].copy_(table.flip_thr.to(torch.int64).bitwise_and(0xFFFFFFFF).to(torch.int32))  # uint32 bits
+        t["has_start"].copy_(table.has_start)
+        self._start = StartTable(table.words.clone(), table.flip_thr.clone(), table.has_start.clone())
+
+    def _apply_starts(self, reset_key: torch.Tensor, obs: Optional[torch.Tensor],
+                      gnn: Optional[Dict[str, torch.Tensor]] = None) -> None:
+        t = self._start_dev
+        _lib.check(self.env._lib.msat_apply_start_states(
+            self.bank.plan.handle, _ptr(self.bank.data), self.bank.num_problems, _ptr(self.state), _ptr(reset_key),
+            self.num_envs_global, self.env_offset, _ptr(t["words"]), _ptr(t["flip_thr"]), _ptr(t["has_start"]),
+            _ptr(obs), _ptr(gnn["gnn_assignment"]) if gnn else None, _ptr(gnn["gnn_clause_features"]) if gnn else None,
+            self.num_envs, _stream_ptr(self.state.device)), "msat_apply_start_states")
+
+    def _require_random_starts(self, what: str) -> None:
+        if self._start is not None:
+            raise ValueError(f"{what} resets envs inside its fused kernel and cannot apply start states; "
+                             f"use step(), or set_start_states(None) first")
+
     # runner:289-295 -- key,_rng = split(key); idx = randint(_rng,...); reset_keys = split(_rng, B)
     def reset(self) -> Optional[torch.Tensor]:
         lib, dev = self.env._lib, self.state.device
@@ -192,12 +248,24 @@ class VecSATEnv:
                         self.new_problem_idx, self.reset_keys, None if self._weights is None else self._cum_weights)
         obs, _ = self.env.reset_from_bank(self.bank, self.new_problem_idx, self.reset_keys, state_out=self.state,
                                           obs_out=self.out["obs"], want_obs=self.out["obs"] is not None)
+        if self._start is not None:
+            self._apply_starts(rng, self.out["obs"])
         return obs
 
     def step(self, actions: torch.Tensor, out: Optional[Dict[str, torch.Tensor]] = None) -> Dict[str, torch.Tensor]:
         """One rollout step (learner:397-464) for this shard.  ``actions`` int32 ``[B, A]`` (mode 0) or
         ``[B, A, V]`` (mode 1) on the device.  Returns the output dict (obs of the state to continue
-        from; reward/done/info are the pre-reset values, learner:467-478)."""
+        from; reward/done/info are the pre-reset values, learner:467-478).  While start states are set, the envs
+        that restarted are then moved to their starts (``msat_apply_start_states`` with this step's reset key)."""
+        res = self._step(actions, out)
+        if self._start is not None:
+            if self.gnn_outputs:
+                self._apply_starts(self.keys.reset_key, None, self.out)
+            else:
+                self._apply_starts(self.keys.reset_key, res.get("obs"))
+        return res
+
+    def _step(self, actions: torch.Tensor, out: Optional[Dict[str, torch.Tensor]]) -> Dict[str, torch.Tensor]:
         weighted = self._weights is not None
         if self.gnn_outputs and not weighted:
             return self._step_gnn(actions)
@@ -318,6 +386,7 @@ class VecSATEnv:
         does not depend on the intermediate observations (replay, open-loop evaluation, launch-bound small
         batches).  Identical results to K calls of ``step``; ``out`` from ``alloc_multi_step_outputs``."""
         self._require_uniform("steps()")
+        self._require_random_starts("steps()")
         K = int(actions.shape[0])
         done, reward = out["done"], out["reward"]
         _lib.check(self.env._lib.msat_rollout_steps(
@@ -355,6 +424,7 @@ class VecSATEnv:
         With ``compact_outputs`` the per-agent reward / done values (identical for all agents, env:196,260)
         travel once per env; ``host_views`` expands them without copying."""
         self._require_uniform("step_host()")
+        self._require_random_starts("step_host()")
         out, dev = self.out, self.state.device
         if actions_dev is None:
             if not hasattr(self, "_actions_dev"):
@@ -405,6 +475,7 @@ class VecSATEnv:
         ``actions_host`` (pinned; default ``slot['host']['actions']``) must stay untouched until the step's
         kernel has run; read the results from ``slot['host']`` after ``host_wait(slot_idx)``."""
         self._require_uniform("step_host_async()")
+        self._require_random_starts("step_host_async()")
         host, dev = slot["host"], self.state.device
         acts = host["actions"] if actions_host is None else actions_host
         k, cur = self.keys, self.keys._cur
@@ -493,13 +564,17 @@ class VecSATEnv:
         chain (``RolloutKeys.chain``, 10 words), ``env_offset``, ``num_envs_global`` and a shape ``signature``.
         The packed layout never leaves the process, so the checkpoint loads into either clause-update mode, any
         observation dtype and any later library version.  While problem weights are set, their quantised values are
-        stored under ``problem_weights``.  Synchronises the stream."""
+        stored under ``problem_weights``, and while start states are set, their tables under ``start_states``
+        (``words``, ``flip_thr``, ``has_start``); the saved states are those after the starts were applied.
+        Synchronises the stream."""
         st = self.sat_state()
         sd = {"variable_assignments": st.variable_assignments.cpu(), "step": st.step.cpu(), "done": st.done.cpu(),
               "problem_idx": st.problem_idx.cpu(), "rng_chain": self.keys.chain.cpu().clone(),
               "env_offset": self.env_offset, "num_envs_global": self.num_envs_global, "signature": self._signature()}
         if self._weights is not None:
             sd["problem_weights"] = self._weights.clone()
+        if self._start is not None:
+            sd["start_states"] = dict(self._start._asdict())
         return sd
 
     def load_state_dict(self, sd: Dict) -> Optional[torch.Tensor]:
@@ -508,8 +583,8 @@ class VecSATEnv:
         reset keys depend only on (rng, global env index, global batch size) (DESIGN.md section 7), so a world-1
         checkpoint loads into every rank of a world-N run, and rank checkpoints joined with
         ``merge_state_dicts`` load into any world size, with the values of an uninterrupted single-device run.
-        The problem weights are restored too: those of the checkpoint, or the uniform draw for a checkpoint without
-        them.  Returns the policy input written by ``import_state``."""
+        The problem weights and start states are restored too: those of the checkpoint, or the uniform draw / random
+        starts for a checkpoint without them.  Returns the policy input written by ``import_state``."""
         sig = {k: int(v) for k, v in dict(sd["signature"]).items()}
         if sig != self._signature():
             raise ValueError(f"checkpoint signature {sig} does not match this env's {self._signature()}")
@@ -524,6 +599,11 @@ class VecSATEnv:
         q = None if weights is None else problem_weights(weights, self.bank.num_problems)
         if q is not None and not torch.equal(q, torch.as_tensor(weights, dtype=torch.int64)):
             raise ValueError("checkpoint problem_weights are not quantised weights (problem_weights)")
+        starts = _start_table_of(sd)
+        if starts is not None and (tuple(starts.words.shape) != (self.bank.num_problems, (self.env.num_vars + 31) // 32)
+                                   or tuple(starts.flip_thr.shape) != (self.bank.num_problems,)
+                                   or tuple(starts.has_start.shape) != (self.bank.num_problems,)):
+            raise ValueError("checkpoint start_states do not match this env's bank")
         rows_of = lambda name: torch.as_tensor(sd[name])[lo:lo + self.num_envs]
         obs = self.import_state(rows_of("problem_idx"), rows_of("variable_assignments"), rows_of("step"),
                                 rows_of("done"), validate=True)
@@ -532,13 +612,26 @@ class VecSATEnv:
             self._weights = None
         else:
             self._install_weights(q)
+        if starts is None:
+            self._start = None
+        else:
+            self._install_starts(starts)
         return obs
+
+
+def _start_table_of(sd: Dict) -> Optional[StartTable]:
+    t = sd.get("start_states")
+    if t is None:
+        return None
+    return StartTable(torch.as_tensor(t["words"], dtype=torch.int32), torch.as_tensor(t["flip_thr"], dtype=torch.int64),
+                      torch.as_tensor(t["has_start"], dtype=torch.uint8))
 
 
 def merge_state_dicts(dicts) -> Dict:
     """Join ``VecSATEnv.state_dict()`` checkpoints of adjacent shards of one run into one (rows in ``env_offset``
     order), e.g. every rank's, which then loads into any world size.  Shards must agree on the problem weights
-    (all without, or all with equal ``problem_weights``)."""
+    (all without, or all with equal ``problem_weights``) and on the start states (all without, or all with equal
+    ``start_states`` tables)."""
     dicts = sorted(dicts, key=lambda sd: int(sd["env_offset"]))
     first = dicts[0]
     end = int(first["env_offset"])
@@ -554,6 +647,9 @@ def merge_state_dicts(dicts) -> Dict:
         if (w is None) != (weights is None) or (w is not None and not torch.equal(torch.as_tensor(w),
                                                                                    torch.as_tensor(weights))):
             raise ValueError("shards have different problem weights")
+        st, st0 = _start_table_of(sd), _start_table_of(first)
+        if (st is None) != (st0 is None) or (st is not None and not all(torch.equal(x, y) for x, y in zip(st, st0))):
+            raise ValueError("shards have different start states")
         end += int(sd["variable_assignments"].shape[0])
     merged = {k: torch.cat([torch.as_tensor(sd[k]) for sd in dicts])
               for k in ("variable_assignments", "step", "done", "problem_idx")}
@@ -561,6 +657,9 @@ def merge_state_dicts(dicts) -> Dict:
                   num_envs_global=int(first["num_envs_global"]), signature=dict(first["signature"]))
     if weights is not None:
         merged["problem_weights"] = torch.as_tensor(weights).clone()
+    starts = _start_table_of(first)
+    if starts is not None:
+        merged["start_states"] = {k: v.clone() for k, v in starts._asdict().items()}
     return merged
 
 
