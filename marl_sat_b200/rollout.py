@@ -21,7 +21,7 @@ values of the single-device run (SURVEY.md section 8e).
 from __future__ import annotations
 
 import ctypes as C
-from typing import Dict, Optional
+from typing import Dict, Optional, Tuple
 
 import numpy as np
 import torch
@@ -58,6 +58,7 @@ class RolloutKeys:
         self._bufs = torch.zeros((2, 10), dtype=torch.int32, device=device)
         self._cur = 0
         self._bufs[0, :2] = as_u32_tensor(key, device).reshape(2)
+        self._buf_ptrs = (self._bufs[0].data_ptr(), self._bufs[1].data_ptr())   # _bufs is only ever updated in place
 
     @property
     def chain(self) -> torch.Tensor:
@@ -70,6 +71,13 @@ class RolloutKeys:
 
     def flip(self) -> None:
         self._cur = 1 - self._cur
+
+    def take_launch_ptrs(self) -> Tuple[int, int]:
+        """Device pointers of ``(chain, next_chain)`` -- the ``rng_in`` / ``chain_out`` of a launch that advances the
+        chain -- and ``flip``: the launch's chain becomes current.  ``flip`` again if the launch fails."""
+        cur = self._cur
+        self._cur = 1 - cur
+        return self._buf_ptrs[cur], self._buf_ptrs[1 - cur]
 
     @property
     def rng(self) -> torch.Tensor:
@@ -96,6 +104,34 @@ class RolloutKeys:
         _lib.check(self._lib.msat_rng_chain(_ptr(self.chain), _ptr(self.next_chain), _stream_ptr(self.device)),
                    "msat_rng_chain")
         self.flip()
+
+
+# Per-call arguments of a bound rollout launch: placeholders in the argument list that _BoundCall fills in on every call
+# (ctypes rejects one left unfilled).
+_ACTIONS, _RNG_IN, _CHAIN_OUT, _STREAM = object(), object(), object(), object()
+
+
+class _BoundCall:
+    """A rollout entry point with its argument list built once (``VecSATEnv._bind``).  A call fills the per-call
+    slots -- the action pointers it is given, the rng buffers of ``keys`` and the device's current stream (a graph
+    capture runs on a side stream) -- launches and advances ``keys``, or raises on an error code."""
+
+    def __init__(self, fn, name: str, args: list, keys: RolloutKeys, device: torch.device):
+        self.fn, self.name, self.args, self.keys, self.device = fn, name, args, keys, device
+        first = args.index(_ACTIONS)
+        self.actions = slice(first, first + args.count(_ACTIONS))
+        assert all(a is _ACTIONS for a in args[self.actions]), f"{name}: the action pointers must be adjacent"
+        self.rng_in, self.chain_out, self.stream = args.index(_RNG_IN), args.index(_CHAIN_OUT), args.index(_STREAM)
+
+    def __call__(self, *action_ptrs: int) -> None:
+        args = self.args
+        args[self.actions] = action_ptrs
+        args[self.rng_in], args[self.chain_out] = self.keys.take_launch_ptrs()
+        args[self.stream] = torch.cuda.current_stream(self.device).cuda_stream
+        rc = self.fn(*args)
+        if rc != 0:
+            self.keys.flip()
+            _lib.check(rc, self.name)
 
 
 def derive_env_keys(prob_key: Optional[torch.Tensor], reset_key: Optional[torch.Tensor], num_envs_global: int,
@@ -153,6 +189,10 @@ class VecSATEnv:
         self._cum_weights: Optional[torch.Tensor] = None    # their inclusive prefix sums on the device
         self._start: Optional[StartTable] = None             # start-state tables (host), None = random starts
         self._start_dev: Optional[Dict[str, torch.Tensor]] = None   # their device copies, allocated once
+        # bindings (_bind) cached with the buffers they were built over: at small per-GPU batches the ~80 µs kernel
+        # is short enough for per-call Python work to matter
+        self._fast_args = None   # step() on self.out: (binding, self.out["obs"])
+        self._host_args = None   # step_host: (binding, host["reward"], self.out["obs"])
 
     # ------------------------------------------------------------------ weighted problem draw
     @property
@@ -180,10 +220,14 @@ class VecSATEnv:
         self._cum_weights.copy_(torch.cumsum(q, 0))
         self._weights = q
 
-    def _require_uniform(self, what: str) -> None:
+    def _require_plain_resets(self, what: str) -> None:
+        """Refuse a fused entry point that resets envs itself while problem weights or start states are set."""
         if self._weights is not None:
             raise ValueError(f"{what} draws problem indices inside its fused kernel and cannot apply problem weights; "
                              f"use step(), or set_problem_weights(None) first")
+        if self._start is not None:
+            raise ValueError(f"{what} resets envs inside its fused kernel and cannot apply start states; "
+                             f"use step(), or set_start_states(None) first")
 
     # ------------------------------------------------------------------ start states (reverse curriculum)
     @property
@@ -233,11 +277,6 @@ class VecSATEnv:
             _ptr(obs), _ptr(gnn["gnn_assignment"]) if gnn else None, _ptr(gnn["gnn_clause_features"]) if gnn else None,
             self.num_envs, _stream_ptr(self.state.device)), "msat_apply_start_states")
 
-    def _require_random_starts(self, what: str) -> None:
-        if self._start is not None:
-            raise ValueError(f"{what} resets envs inside its fused kernel and cannot apply start states; "
-                             f"use step(), or set_start_states(None) first")
-
     # runner:289-295 -- key,_rng = split(key); idx = randint(_rng,...); reset_keys = split(_rng, B)
     def reset(self) -> Optional[torch.Tensor]:
         lib, dev = self.env._lib, self.state.device
@@ -255,8 +294,10 @@ class VecSATEnv:
     def step(self, actions: torch.Tensor, out: Optional[Dict[str, torch.Tensor]] = None) -> Dict[str, torch.Tensor]:
         """One rollout step (learner:397-464) for this shard.  ``actions`` int32 ``[B, A]`` (mode 0) or
         ``[B, A, V]`` (mode 1) on the device.  Returns the output dict (obs of the state to continue
-        from; reward/done/info are the pre-reset values, learner:467-478).  While start states are set, the envs
-        that restarted are then moved to their starts (``msat_apply_start_states`` with this step's reset key)."""
+        from; reward/done/info are the pre-reset values, learner:467-478).  With ``gnn_outputs`` the step emits the
+        dynamic GNN input into ``self.out`` instead of local observations (``msat_rollout_step_gnn``; combine with
+        ``features.static_graph(bank)`` for the full ``GNNInput``).  While start states are set, the envs that
+        restarted are then moved to their starts (``msat_apply_start_states`` with this step's reset key)."""
         res = self._step(actions, out)
         if self._start is not None:
             if self.gnn_outputs:
@@ -267,24 +308,18 @@ class VecSATEnv:
 
     def _step(self, actions: torch.Tensor, out: Optional[Dict[str, torch.Tensor]]) -> Dict[str, torch.Tensor]:
         weighted = self._weights is not None
-        if self.gnn_outputs and not weighted:
-            return self._step_gnn(actions)
-        if out is None and self.fused_keys and not weighted:
-            return self._step_fast(actions)
+        if not weighted and (self.gnn_outputs or self.fused_keys):
+            # one launch: rng chain + per-env key derivation + step + auto-reset; the GNN-input step ignores ``out``
+            if out is not None and not self.gnn_outputs:
+                self._bind("msat_rollout_step", out)(actions.data_ptr())
+                return out
+            call, obs = self._fast_args or (None, None)
+            if call is None or obs is not self.out["obs"]:
+                call = self._bind("msat_rollout_step_gnn" if self.gnn_outputs else "msat_rollout_step", self.out)
+                self._fast_args = (call, self.out["obs"])
+            call(actions.data_ptr())
+            return self.out
         out = self.out if out is None or self.gnn_outputs else out
-        if self.fused_keys and not weighted:
-            # one launch: rng chain + per-env key derivation + step + auto-reset (msat_rollout_step)
-            done, reward = out.get("done"), out.get("reward")
-            _lib.check(self.env._lib.msat_rollout_step(
-                self.bank.plan.handle, _ptr(self.bank.data), self.bank.num_problems, _ptr(self.state),
-                _ptr(self.state), _ptr(actions), _ptr(self.keys.chain), _ptr(self.keys.next_chain),
-                self.num_envs_global, self.env_offset, _ptr(out.get("obs")), _ptr(reward),
-                int(reward.shape[-1]) if reward is not None else 0, _ptr(done),
-                int(done.shape[-1]) if done is not None else 0, _ptr(out.get("solved")),
-                _ptr(out.get("num_unsatisfied")), _ptr(out.get("episode_step")), self.num_envs,
-                _stream_ptr(self.state.device)), "msat_rollout_step")
-            self.keys.flip()
-            return out
         # separate launches: rng chain, per-env problem indices (weighted while weights are set) and reset keys, step
         self.keys.advance()
         derive_env_keys(self.keys.prob_key, self.keys.reset_key, self.num_envs_global, self.env_offset, self.num_envs,
@@ -293,11 +328,50 @@ class VecSATEnv:
         self.env.step_into(self.bank, self.state, self.state, actions, dict(out, obs=None) if self.gnn_outputs else out,
                            auto_reset=True, new_problem_idx=self.new_problem_idx, reset_keys=self.reset_keys)
         if self.gnn_outputs:          # the GNN input of the state to continue from, as msat_rollout_step_gnn emits it
-            _lib.check(self.env._lib.msat_gnn_dynamic(
-                self.bank.plan.handle, _ptr(self.bank.data), self.bank.num_problems, _ptr(self.state), self.num_envs,
-                _ptr(out["gnn_assignment"]), _ptr(out["gnn_clause_features"]), _stream_ptr(self.state.device)),
-                "msat_gnn_dynamic")
+            self._gnn_dynamic()
         return out
+
+    def _gnn_dynamic(self) -> None:
+        """``msat_gnn_dynamic`` of the current state into ``self.out``'s GNN assignment and clause features."""
+        _lib.check(self.env._lib.msat_gnn_dynamic(
+            self.bank.plan.handle, _ptr(self.bank.data), self.bank.num_problems, _ptr(self.state), self.num_envs,
+            _ptr(self.out["gnn_assignment"]), _ptr(self.out["gnn_clause_features"]), _stream_ptr(self.state.device)),
+            "msat_gnn_dynamic")
+
+    def _bind(self, name: str, out: Dict[str, Optional[torch.Tensor]], host: Optional[Dict[str, torch.Tensor]] = None,
+              num_steps: int = 1, pipe_slot: Optional[Tuple[int, torch.Tensor]] = None) -> _BoundCall:
+        """The argument list of the rollout entry point ``name``, in the header's parameter order, bound to the device
+        outputs ``out``; ``host`` is the pinned result buffers of the host-buffer entry points, ``num_steps`` the K of
+        ``msat_rollout_steps`` and ``pipe_slot`` the ``(slot, actions_dev)`` of ``msat_rollout_step_host_async``.
+        Per-call slots, given to the returned call in this order: the action pointer (``actions``; ``actions_host``
+        and ``actions_dev`` for ``msat_rollout_step_host``; ``actions_host`` for ``msat_rollout_step_host_async``);
+        then ``rng_in``, ``chain_out`` and ``stream``, which the call fills in itself."""
+        s, obs = _ptr(self.state), _ptr(out.get("obs"))
+        reward, done = out.get("reward"), out.get("done")
+        chain = [_RNG_IN, _CHAIN_OUT, self.num_envs_global, self.env_offset]
+        results = [_ptr(reward), 0 if reward is None else int(reward.shape[-1]), _ptr(done),
+                   0 if done is None else int(done.shape[-1]), _ptr(out.get("solved")),
+                   _ptr(out.get("num_unsatisfied")), _ptr(out.get("episode_step"))]
+        if host is not None:
+            results += [_ptr(host[k]) for k in ("reward", "done", "solved", "num_unsatisfied", "episode_step")]
+        pipe = []
+        if name == "msat_rollout_step":
+            mid = [s, s, _ACTIONS, *chain, obs, *results]
+        elif name == "msat_rollout_step_gnn":
+            mid = [s, s, _ACTIONS, *chain, _ptr(out["gnn_assignment"]), _ptr(out["gnn_clause_features"]), *results]
+        elif name == "msat_rollout_steps":
+            mid = [s, s, _ACTIONS, num_steps, *chain, obs, _ptr(out.get("gnn_assignment")),
+                   _ptr(out.get("gnn_clause_features")), 1 if out.get("emit_every_step") else 0, *results,
+                   _ptr(out.get("newly_satisfied"))]
+        elif name == "msat_rollout_step_host":
+            mid = [s, _ACTIONS, _ACTIONS, *chain, obs, *results]
+        elif name == "msat_rollout_step_host_async":
+            slot_idx, actions_dev = pipe_slot
+            pipe = [self._pipe, int(slot_idx)]
+            mid = [s, _ACTIONS, _ptr(actions_dev), *chain, obs, *results]
+        args = [*pipe, self.bank.plan.handle, _ptr(self.bank.data), self.bank.num_problems, *mid, self.num_envs,
+                _STREAM]
+        return _BoundCall(getattr(self.env._lib, name), name, args, self.keys, self.state.device)
 
     def sample_actions(self, logits: torch.Tensor, actions: Optional[torch.Tensor] = None,
                        log_prob: Optional[torch.Tensor] = None):
@@ -318,44 +392,6 @@ class VecSATEnv:
         # the rng this env's next step advances: act_key = split(rng)[1] (msat_rng_chain's chain_out[2:4])
         return sample_actions(logits, self.keys.chain[0:2], self.num_envs_global * rows_per_env,
                               self.env_offset * rows_per_env, actions, log_prob)
-
-    def _step_gnn(self, actions: torch.Tensor) -> Dict[str, torch.Tensor]:
-        """Rollout step that emits the dynamic GNN input instead of local observations
-        (``msat_rollout_step_gnn``); combine with ``features.static_graph(bank)`` for the full ``GNNInput``."""
-        out = self.out
-        done, reward = out["done"], out["reward"]
-        _lib.check(self.env._lib.msat_rollout_step_gnn(
-            self.bank.plan.handle, _ptr(self.bank.data), self.bank.num_problems, _ptr(self.state), _ptr(self.state),
-            _ptr(actions), _ptr(self.keys.chain), _ptr(self.keys.next_chain), self.num_envs_global, self.env_offset,
-            _ptr(out["gnn_assignment"]), _ptr(out["gnn_clause_features"]), _ptr(reward), int(reward.shape[-1]),
-            _ptr(done), int(done.shape[-1]), _ptr(out["solved"]), _ptr(out["num_unsatisfied"]),
-            _ptr(out["episode_step"]), self.num_envs, _stream_ptr(self.state.device)), "msat_rollout_step_gnn")
-        self.keys.flip()
-        return out
-
-    def _step_fast(self, actions: torch.Tensor) -> Dict[str, torch.Tensor]:
-        """``step`` on the env's own output buffers with every constant argument bound once: at small
-        per-GPU batches the ~80 µs kernel is short enough for per-call Python work to matter."""
-        args = getattr(self, "_fast_args", None)
-        if args is None or args[-1] is not self.out["obs"]:
-            out, k = self.out, self.keys
-            done, reward = out["done"], out["reward"]
-            fixed = [self.bank.plan.handle, _ptr(self.bank.data), self.bank.num_problems, _ptr(self.state),
-                     _ptr(self.state), None, None, None, self.num_envs_global, self.env_offset, _ptr(out["obs"]),
-                     _ptr(reward), int(reward.shape[-1]), _ptr(done), int(done.shape[-1]), _ptr(out["solved"]),
-                     _ptr(out["num_unsatisfied"]), _ptr(out["episode_step"]), self.num_envs, None]
-            chains = (_ptr(k._bufs[0]), _ptr(k._bufs[1]))
-            args = self._fast_args = (fixed, chains, self.env._lib.msat_rollout_step, out["obs"])
-        fixed, chains, fn, _ = args
-        cur = self.keys._cur
-        fixed[5] = actions.data_ptr()
-        fixed[6], fixed[7] = chains[cur], chains[1 - cur]
-        fixed[19] = torch.cuda.current_stream(self.state.device).cuda_stream
-        rc = fn(*fixed)
-        if rc != 0:
-            _lib.check(rc, "msat_rollout_step")
-        self.keys._cur = 1 - cur
-        return self.out
 
     # ------------------------------------------------------------------ K fused steps
     def alloc_multi_step_outputs(self, num_steps: int, emit_every_step: bool = False) -> Dict[str, torch.Tensor]:
@@ -385,19 +421,8 @@ class VecSATEnv:
         """K rollout steps in ONE launch (``msat_rollout_steps``) for an action table ``[K, B, A(, V)]`` that
         does not depend on the intermediate observations (replay, open-loop evaluation, launch-bound small
         batches).  Identical results to K calls of ``step``; ``out`` from ``alloc_multi_step_outputs``."""
-        self._require_uniform("steps()")
-        self._require_random_starts("steps()")
-        K = int(actions.shape[0])
-        done, reward = out["done"], out["reward"]
-        _lib.check(self.env._lib.msat_rollout_steps(
-            self.bank.plan.handle, _ptr(self.bank.data), self.bank.num_problems, _ptr(self.state), _ptr(self.state),
-            _ptr(actions), K, _ptr(self.keys.chain), _ptr(self.keys.next_chain), self.num_envs_global,
-            self.env_offset, _ptr(out.get("obs")), _ptr(out.get("gnn_assignment")),
-            _ptr(out.get("gnn_clause_features")), 1 if out.get("emit_every_step") else 0, _ptr(reward),
-            int(reward.shape[-1]), _ptr(done), int(done.shape[-1]), _ptr(out["solved"]),
-            _ptr(out["num_unsatisfied"]), _ptr(out["episode_step"]), _ptr(out.get("newly_satisfied")),
-            self.num_envs, _stream_ptr(self.state.device)), "msat_rollout_steps")
-        self.keys.flip()
+        self._require_plain_resets("steps()")
+        self._bind("msat_rollout_steps", out, num_steps=int(actions.shape[0]))(actions.data_ptr())
         return out
 
     def set_episode_steps(self, steps: torch.Tensor) -> None:
@@ -423,32 +448,16 @@ class VecSATEnv:
         synchronised.  Observations stay in HBM (``self.out['obs']``) where the policy consumes them.
         With ``compact_outputs`` the per-agent reward / done values (identical for all agents, env:196,260)
         travel once per env; ``host_views`` expands them without copying."""
-        self._require_uniform("step_host()")
-        self._require_random_starts("step_host()")
-        out, dev = self.out, self.state.device
+        self._require_plain_resets("step_host()")
         if actions_dev is None:
             if not hasattr(self, "_actions_dev"):
-                self._actions_dev = torch.empty(host["actions"].shape, dtype=torch.int32, device=dev)
+                self._actions_dev = torch.empty(host["actions"].shape, dtype=torch.int32, device=self.state.device)
             actions_dev = self._actions_dev
-        bound = getattr(self, "_host_args", None)
-        if bound is None or bound[2] is not host["reward"] or bound[3] is not out["obs"]:
-            done, reward, k = out["done"], out["reward"], self.keys
-            fixed = [self.bank.plan.handle, _ptr(self.bank.data), self.bank.num_problems, _ptr(self.state),
-                     None, None, None, None, self.num_envs_global, self.env_offset, _ptr(out["obs"]), _ptr(reward),
-                     int(reward.shape[-1]), _ptr(done), int(done.shape[-1]), _ptr(out["solved"]),
-                     _ptr(out["num_unsatisfied"]), _ptr(out["episode_step"]), _ptr(host["reward"]), _ptr(host["done"]),
-                     _ptr(host["solved"]), _ptr(host["num_unsatisfied"]), _ptr(host["episode_step"]), self.num_envs,
-                     None]
-            bound = self._host_args = (fixed, (_ptr(k._bufs[0]), _ptr(k._bufs[1])), host["reward"], out["obs"])
-        fixed, chains = bound[0], bound[1]
-        cur = self.keys._cur
-        fixed[4], fixed[5] = host["actions"].data_ptr(), actions_dev.data_ptr()
-        fixed[6], fixed[7] = chains[cur], chains[1 - cur]
-        fixed[24] = torch.cuda.current_stream(dev).cuda_stream
-        rc = self.env._lib.msat_rollout_step_host(*fixed)
-        if rc != 0:
-            _lib.check(rc, "msat_rollout_step_host")
-        self.keys._cur = 1 - cur
+        call, reward, obs = self._host_args or (None, None, None)
+        if call is None or reward is not host["reward"] or obs is not self.out["obs"]:
+            call = self._bind("msat_rollout_step_host", self.out, host)
+            self._host_args = (call, host["reward"], self.out["obs"])
+        call(host["actions"].data_ptr(), actions_dev.data_ptr())
         return host
 
     def alloc_async_io(self, depth: int = 2):
@@ -474,33 +483,12 @@ class VecSATEnv:
         action upload, the fused step and the result download of this call overlap the neighbouring steps'.
         ``actions_host`` (pinned; default ``slot['host']['actions']``) must stay untouched until the step's
         kernel has run; read the results from ``slot['host']`` after ``host_wait(slot_idx)``."""
-        self._require_uniform("step_host_async()")
-        self._require_random_starts("step_host_async()")
-        host, dev = slot["host"], self.state.device
-        acts = host["actions"] if actions_host is None else actions_host
-        k, cur = self.keys, self.keys._cur
-        fixed = slot.get("_bound")
-        if fixed is None:
-            # the argument list of this slot, bound once (every buffer of a slot is fixed); per call only the
-            # action pointer, the two rng buffers and the stream change
-            out = slot["dev"]
-            done, reward = out["done"], out["reward"]
-            fixed = slot["_bound"] = [
-                self._pipe, int(slot_idx), self.bank.plan.handle, _ptr(self.bank.data), self.bank.num_problems,
-                _ptr(self.state), None, slot["actions_dev"].data_ptr(), None, None, self.num_envs_global,
-                self.env_offset, _ptr(out["obs"]), _ptr(reward), int(reward.shape[-1]), _ptr(done),
-                int(done.shape[-1]), _ptr(out["solved"]), _ptr(out["num_unsatisfied"]), _ptr(out["episode_step"]),
-                _ptr(host["reward"]), _ptr(host["done"]), _ptr(host["solved"]), _ptr(host["num_unsatisfied"]),
-                _ptr(host["episode_step"]), self.num_envs, None]
-            slot["_chains"] = (_ptr(k._bufs[0]), _ptr(k._bufs[1]))
-        chains = slot["_chains"]
-        fixed[6] = acts.data_ptr()
-        fixed[8], fixed[9] = chains[cur], chains[1 - cur]
-        fixed[26] = torch.cuda.current_stream(dev).cuda_stream
-        rc = self.env._lib.msat_rollout_step_host_async(*fixed)
-        if rc != 0:
-            _lib.check(rc, "msat_rollout_step_host_async")
-        self.keys._cur = 1 - cur
+        self._require_plain_resets("step_host_async()")
+        call = slot.get("_call")
+        if call is None:   # every buffer of a slot is fixed: bound on the slot's first step
+            call = slot["_call"] = self._bind("msat_rollout_step_host_async", slot["dev"], slot["host"],
+                                              pipe_slot=(slot_idx, slot["actions_dev"]))
+        call((slot["host"]["actions"] if actions_host is None else actions_host).data_ptr())
 
     def host_wait(self, slot_idx: int) -> None:
         """Block until the results of the step last enqueued on this slot are in its host buffers."""
@@ -547,10 +535,7 @@ class VecSATEnv:
         obs, _ = self.env.import_state(self.bank, problem_idx, variable_assignments, step, done, state_out=self.state,
                                        obs_out=out["obs"], want_obs=out["obs"] is not None, validate=validate)
         if self.gnn_outputs:
-            _lib.check(self.env._lib.msat_gnn_dynamic(
-                self.bank.plan.handle, _ptr(self.bank.data), self.bank.num_problems, _ptr(self.state), self.num_envs,
-                _ptr(out["gnn_assignment"]), _ptr(out["gnn_clause_features"]), _stream_ptr(self.state.device)),
-                "msat_gnn_dynamic")
+            self._gnn_dynamic()
         return obs
 
     def _signature(self) -> Dict[str, int]:
