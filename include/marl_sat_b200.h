@@ -260,7 +260,7 @@ int msat_export_state(const msat_plan* plan, const void* bank, int32_t num_probl
  * buffers that are adjacent in both address spaces are copied as one transfer; batches of 32768+ envs
  * are processed as four slices alternating between two internal streams so that the PCIe
  * copies overlap the kernel.  All device workspaces are caller-owned; observations stay on the device
- * (obs_dev). */
+ * (obs_dev).  This call and msat_rollout_step_host_async check the whole batch before they enqueue anything. */
 int msat_rollout_step_host(const msat_plan* plan, const void* bank, int32_t num_problems,
                            uint32_t* state, const int32_t* actions_host, int32_t* actions_dev,
                            const uint32_t* rng_in, uint32_t* chain_out,

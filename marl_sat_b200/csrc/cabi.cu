@@ -16,6 +16,9 @@ namespace {
 
 inline bool aligned(const void* p, size_t a) { return (reinterpret_cast<uintptr_t>(p) & (a - 1)) == 0; }
 inline int cuda_rc(cudaError_t e) { return e == cudaSuccess ? MSAT_OK : (int)e; }
+inline size_t actions_per_env(const Dims& d) { return (size_t)d.A * (d.action_mode == 0 ? 1 : d.V); }
+// GNN clause features come from a 16-entry table indexed by the true-literal count: k <= 15.
+inline bool clause_features_unsupported(const msat_plan* plan, const float* cf) { return cf && plan->d.k > 15; }
 constexpr int kMaxSmem = 227 * 1024;
 constexpr int kMaxPipeDepth = 4;
 
@@ -62,25 +65,122 @@ cudaError_t sync_pipe_for_current_device(SyncPipe** out) {
     return cudaSuccess;
 }
 
-// Device->host result copies of one batch slice; outputs that are adjacent in both address spaces (the Python
-// layer carves them out of one device block and one pinned block) travel as ONE copy.
-struct ResultBufs {
-    float* reward_dev; int32_t reward_cols; uint8_t* done_dev; int32_t done_cols; uint8_t* solved_dev;
-    int32_t* nunsat_dev; int32_t* estep_dev;
+// Every env entry point: a plan, B >= 0, P > 0 and, when B > 0, the bank and the caller's own required pointers.
+inline bool bad_env_call(const msat_plan* plan, const void* bank, int32_t P, int32_t B, bool missing) {
+    return !plan || B < 0 || P <= 0 || (B > 0 && (!bank || missing));
+}
+
+// bad_env_call, then bank (128 bytes), state and observation (16 bytes) alignment; fills the base of `a`.
+int env_args(EnvArgs& a, const msat_plan* plan, const void* bank, int32_t P, const uint32_t* state_in,
+             uint32_t* state_out, int32_t* obs, int32_t B, bool missing) {
+    if (bad_env_call(plan, bank, P, B, missing)) return MSAT_EINVAL;
+    if (!aligned(bank, 128) || !aligned(state_in, 16) || !aligned(state_out, 16) || !aligned(obs, 16))
+        return MSAT_EALIGN;
+    a = EnvArgs{};
+    a.bank = static_cast<const uint8_t*>(bank); a.P = P;
+    a.state_in = state_in; a.state_out = state_out; a.obs = obs; a.B = B;
+    return MSAT_OK;
+}
+
+// Per-step outputs of msat_step and the fused rollout steps, added to `a` with the plan's reward: reward
+// [B, reward_cols] and done [B, done_cols] need a positive column count, newly_satisfied the shaped reward.
+int step_outputs(EnvArgs& a, const msat_plan* plan, float* reward, int32_t reward_cols, uint8_t* done,
+                 int32_t done_cols, uint8_t* solved, int32_t* num_unsat, int32_t* episode_step, int32_t* newly_sat) {
+    if ((done && done_cols <= 0) || (reward && reward_cols <= 0)) return MSAT_EINVAL;
+    if (newly_sat && plan->reward_mode != MSAT_REWARD_SHAPED) return MSAT_EINVAL;
+    a.reward = reward; a.reward_cols = reward_cols; a.done = done; a.done_cols = done_cols;
+    a.solved = solved; a.num_unsat = num_unsat; a.episode_step = episode_step; a.newly_sat = newly_sat;
+    a.reward_mode = plan->reward_mode; a.r_gamma = plan->r_gamma; a.r_clause = plan->r_clause; a.r_sat = plan->r_sat;
+    a.reset_count = plan->reset_counter;
+    return MSAT_OK;
+}
+
+// A shard [off, off + B) inside a global batch of Bg envs, Bg at most 2^30.
+int shard_rule(int32_t Bg, int32_t off, int32_t B) {
+    if (Bg < 0 || off < 0 || B < 0 || (long long)off + B > Bg) return MSAT_EINVAL;
+    return Bg > (1 << 30) ? MSAT_EUNSUPPORTED : MSAT_OK;
+}
+
+// Checks of the fused rollout steps; on success `a` is the launch for the whole batch.
+int rollout_args(EnvArgs& a, const msat_plan* plan, const void* bank, int32_t P, const uint32_t* state_in,
+                 uint32_t* state_out, const int32_t* actions, int32_t K, const uint32_t* rng_in, uint32_t* chain_out,
+                 int32_t Bg, int32_t env_offset, int32_t* obs, int32_t* gnn_assign, float* gnn_cf,
+                 int32_t emit_every_step, float* reward, int32_t reward_cols, uint8_t* done, int32_t done_cols,
+                 uint8_t* solved, int32_t* num_unsat, int32_t* episode_step, int32_t* newly_sat, int32_t B) {
+    if (K < 1 || K > kMaxFusedSteps || !rng_in || !chain_out || Bg <= 0) return MSAT_EINVAL;
+    // the advanced chain is written while other CTAs still read rng_in: the buffers must not overlap
+    const uintptr_t r = reinterpret_cast<uintptr_t>(rng_in), c = reinterpret_cast<uintptr_t>(chain_out);
+    if (r + 8 > c && c + 40 > r) return MSAT_EINVAL;
+    int rc = env_args(a, plan, bank, P, state_in, state_out, obs, B, !state_in || !state_out || !actions);
+    if (rc == MSAT_OK) rc = step_outputs(a, plan, reward, reward_cols, done, done_cols, solved, num_unsat, episode_step,
+                                         newly_sat);
+    if (rc == MSAT_OK) rc = shard_rule(Bg, env_offset, B);
+    if (rc != MSAT_OK) return rc;
+    if (clause_features_unsupported(plan, gnn_cf)) return MSAT_EUNSUPPORTED;
+    a.actions = actions; a.num_steps = K; a.act_step_stride = (long long)B * actions_per_env(plan->d);
+    a.auto_reset = 1; a.rng_in = rng_in; a.chain_out = chain_out; a.Bg = (uint32_t)Bg; a.env_off = (uint32_t)env_offset;
+    a.gnn_assign = gnn_assign; a.gnn_cf = gnn_cf; a.emit_every_step = emit_every_step ? 1 : 0;
+    return MSAT_OK;
+}
+
+cudaError_t rollout_enqueue(const msat_plan* plan, const EnvArgs& a, cudaStream_t s) {
+    if (a.B > 0) return launch_env(plan, MODE_STEP, a, s);
+    cudaError_t e = cudaSuccess;   // an empty shard still advances the chain K times
+    for (int j = 0; j < a.num_steps && e == cudaSuccess; ++j)
+        e = launch_rng_chain(j == 0 ? a.rng_in : a.chain_out, a.chain_out, s);
+    return e;
+}
+
+// A rollout step with actions and results in host memory.  check() validates the whole batch before anything is
+// enqueued; after it, each stage of a slice [b0, b0 + bc) can fail only with a CUDA error.
+struct HostStep {
+    const msat_plan* plan;
+    const int32_t* actions_host; int32_t* actions_dev;
     float* reward_host; uint8_t* done_host; uint8_t* solved_host; int32_t* nunsat_host; int32_t* estep_host;
+    EnvArgs a{};                // the fused step of the whole batch
+    size_t act_per_env = 0, obs_env_bytes = 0;
+    int check(const void* bank, int32_t P, uint32_t* state, const uint32_t* rng_in, uint32_t* chain_out, int32_t Bg,
+              int32_t env_offset, int32_t* obs_dev, float* reward_dev, int32_t reward_cols, uint8_t* done_dev,
+              int32_t done_cols, uint8_t* solved_dev, int32_t* nunsat_dev, int32_t* estep_dev, int32_t B) {
+        if (!plan || !actions_host || !actions_dev || B < 0) return MSAT_EINVAL;
+        act_per_env = actions_per_env(plan->d);
+        obs_env_bytes = (size_t)plan->d.A * plan->d.D * (plan->obs_i8 ? 1 : 4);   // int8 plans: one byte per element
+        return rollout_args(a, plan, bank, P, state, state, actions_dev, 1, rng_in, chain_out, Bg, env_offset, obs_dev,
+                            nullptr, nullptr, 0, reward_dev, reward_cols, done_dev, done_cols, solved_dev, nunsat_dev,
+                            estep_dev, nullptr, B);
+    }
+    cudaError_t upload(int b0, int bc, cudaStream_t w) const {
+        const size_t off = b0 * act_per_env, bytes = bc * act_per_env * sizeof(int32_t);
+        if (bytes == 0) return cudaSuccess;
+        return cudaMemcpyAsync(actions_dev + off, actions_host + off, bytes, cudaMemcpyHostToDevice, w);
+    }
+    cudaError_t step(int b0, int bc, cudaStream_t w) const {
+        EnvArgs s = a;
+        s.B = bc; s.env_off += b0; s.actions += b0 * act_per_env; s.act_step_stride = (long long)bc * act_per_env;
+        s.state_in += (size_t)b0 * plan->d.state_words; s.state_out += (size_t)b0 * plan->d.state_words;
+        if (s.obs) s.obs = reinterpret_cast<int32_t*>(reinterpret_cast<char*>(s.obs) + b0 * obs_env_bytes);
+        auto at = [b0](auto* p, size_t per_env) { return p ? p + b0 * per_env : p; };
+        s.reward = at(s.reward, s.reward_cols); s.done = at(s.done, s.done_cols);
+        s.solved = at(s.solved, 1); s.num_unsat = at(s.num_unsat, 1); s.episode_step = at(s.episode_step, 1);
+        return rollout_enqueue(plan, s, w);
+    }
+    cudaError_t download(int b0, int bc, cudaStream_t w) const;
 };
-cudaError_t copy_results(const ResultBufs& r, int b0, int bc, cudaStream_t w) {
+
+// Outputs that are adjacent in both address spaces (the Python layer carves them out of one device block and
+// one pinned block) travel as ONE copy.
+cudaError_t HostStep::download(int b0, int bc, cudaStream_t w) const {
     struct Seg { const char* dev; char* host; size_t bytes; };
     Seg seg[5];
     int ns = 0;
     auto add = [&](const void* dv, void* hs, size_t off, size_t bytes) {
         if (dv && hs && bytes) seg[ns++] = Seg{static_cast<const char*>(dv) + off, static_cast<char*>(hs) + off, bytes};
     };
-    add(r.reward_dev, r.reward_host, (size_t)b0 * r.reward_cols * sizeof(float), (size_t)bc * r.reward_cols * sizeof(float));
-    add(r.nunsat_dev, r.nunsat_host, (size_t)b0 * 4, (size_t)bc * 4);
-    add(r.estep_dev, r.estep_host, (size_t)b0 * 4, (size_t)bc * 4);
-    add(r.done_dev, r.done_host, (size_t)b0 * r.done_cols, (size_t)bc * r.done_cols);
-    add(r.solved_dev, r.solved_host, (size_t)b0, (size_t)bc);
+    add(a.reward, reward_host, (size_t)b0 * a.reward_cols * sizeof(float), (size_t)bc * a.reward_cols * sizeof(float));
+    add(a.num_unsat, nunsat_host, (size_t)b0 * 4, (size_t)bc * 4);
+    add(a.episode_step, estep_host, (size_t)b0 * 4, (size_t)bc * 4);
+    add(a.done, done_host, (size_t)b0 * a.done_cols, (size_t)bc * a.done_cols);
+    add(a.solved, solved_host, (size_t)b0, (size_t)bc);
     for (int i = 1; i < ns; ++i)          // insertion sort by device address
         for (int j = i; j > 0 && seg[j].dev < seg[j - 1].dev; --j) { Seg t = seg[j]; seg[j] = seg[j - 1]; seg[j - 1] = t; }
     cudaError_t e = cudaSuccess;
@@ -92,13 +192,11 @@ cudaError_t copy_results(const ResultBufs& r, int b0, int bc, cudaStream_t w) {
     return e;
 }
 
-inline void fill_reward(EnvArgs& a, const msat_plan* plan, int32_t* newly) {
-    a.reward_mode = plan->reward_mode;
-    a.r_gamma = plan->r_gamma;
-    a.r_clause = plan->r_clause;
-    a.r_sat = plan->r_sat;
-    a.newly_sat = newly;
-    a.reset_count = plan->reset_counter;
+// Smallest group size from gs up to 256 whose CTA (plus the K key chains of a multi-step launch) fits; 0 if none.
+int fit_group_threads(int gs, const GroupLayout& L) {
+    for (; gs <= 256; gs *= 2)
+        if ((long long)L.total * (kCtaThreads / gs) + 40 * kMaxFusedSteps <= kMaxSmem) return gs;
+    return 0;
 }
 
 // Sizes that depend on the clause-update mode (d.cnt_words), group sizes and shared-memory layouts.
@@ -135,10 +233,8 @@ int finish_plan(msat_plan* p) {
     }
     if (gs != 16 && gs != 32 && gs != 64 && gs != 128 && gs != 256) return MSAT_EINVAL;
     const GroupLayout L = group_layout(d, true);
-    const int kChain = 40 * kMaxFusedSteps;      // room for the K key chains of a multi-step launch
-    // grow the group until one CTA's groups fit in shared memory
-    while (gs < 256 && (long long)L.total * (kCtaThreads / gs) + kChain > kMaxSmem) gs *= 2;
-    if ((long long)L.total * (kCtaThreads / gs) + kChain > kMaxSmem) return MSAT_EUNSUPPORTED;
+    gs = fit_group_threads(gs, L);
+    if (gs == 0) return MSAT_EUNSUPPORTED;
     p->group_threads = gs;
     p->layout_obs = L;
     p->layout_noobs = group_layout(d, false);
@@ -146,16 +242,24 @@ int finish_plan(msat_plan* p) {
     p->smem_bytes = L.total * (kCtaThreads / gs);
     // launches that write no observations (emit_obs off, GNN-input mode) have ~m clause evaluations of work per
     // env and stage only the literal block: one warp per env unless the caller pinned the group size or eight
-    // groups do not fit in shared memory
+    // groups do not fit in shared memory (half-warp groups only with observations)
     const GroupLayout Ln = p->layout_noobs;
-    int gn = p->requested_group_threads ? (gs < 32 ? 32 : gs) : 32;      // half-warp groups only with observations
-    while (gn < 256 && (long long)Ln.total * (kCtaThreads / gn) + kChain > kMaxSmem) gn *= 2;
-    if ((long long)Ln.total * (kCtaThreads / gn) + kChain > kMaxSmem) return MSAT_EUNSUPPORTED;
+    const int gn = fit_group_threads(p->requested_group_threads ? (gs < 32 ? 32 : gs) : 32, Ln);
+    if (gn == 0) return MSAT_EUNSUPPORTED;
     p->group_threads_noobs = gn;
     p->smem_bytes_noobs = Ln.total * (kCtaThreads / gn);
     p->compile_smem_bytes = 4 * (m + n) * d.agw + (d.cnt_words ? 4 * (n + 1) : 0);
     if (p->compile_smem_bytes > kMaxSmem) return MSAT_EUNSUPPORTED;
     return MSAT_OK;
+}
+
+// Sets an option finish_plan sizes the plan from; when the plan cannot take the value, nothing changes.
+int set_and_finish(msat_plan* p, int& option, int value) {
+    const int old = option;
+    option = value;
+    const int rc = finish_plan(p);
+    if (rc != MSAT_OK) { option = old; finish_plan(p); }
+    return rc;
 }
 
 }  // namespace
@@ -219,27 +323,13 @@ int msat_plan_set_reward(msat_plan* plan, int32_t mode, double gamma, double r_c
 
 int msat_plan_set_obs_dtype(msat_plan* plan, int32_t dtype) {
     if (!plan || (dtype != MSAT_OBS_INT32 && dtype != MSAT_OBS_INT8)) return MSAT_EINVAL;
-    const int old = plan->obs_i8;
-    plan->obs_i8 = dtype == MSAT_OBS_INT8;
-    const int rc = finish_plan(plan);          // the group size follows the store width
-    if (rc != MSAT_OK) {
-        plan->obs_i8 = old;
-        finish_plan(plan);
-    }
-    return rc;
+    return set_and_finish(plan, plan->obs_i8, dtype == MSAT_OBS_INT8);   // the group size follows the store width
 }
 
 int msat_plan_set_clause_update(msat_plan* plan, int32_t mode) {
     if (!plan || (mode != MSAT_CLAUSES_FULL && mode != MSAT_CLAUSES_INCREMENTAL)) return MSAT_EINVAL;
     if (mode == MSAT_CLAUSES_INCREMENTAL && plan->d.k > 15) return MSAT_EUNSUPPORTED;     // 4-bit counts
-    const int old = plan->d.cnt_words;
-    plan->d.cnt_words = mode == MSAT_CLAUSES_INCREMENTAL ? (plan->d.m + 7) / 8 : 0;
-    const int rc = finish_plan(plan);
-    if (rc != MSAT_OK) {
-        plan->d.cnt_words = old;
-        finish_plan(plan);
-    }
-    return rc;
+    return set_and_finish(plan, plan->d.cnt_words, mode == MSAT_CLAUSES_INCREMENTAL ? (plan->d.m + 7) / 8 : 0);
 }
 
 int msat_plan_set_reset_counter(msat_plan* plan, uint64_t* counter_dev) {
@@ -275,25 +365,20 @@ int msat_compile_bank(const msat_plan* plan, const int32_t* clauses, int32_t P, 
 
 int msat_reset(const msat_plan* plan, const void* bank, int32_t P, const int32_t* problem_idx, const uint32_t* keys,
                uint32_t* state, int32_t* obs, int32_t B, void* stream) {
-    if (!plan || B < 0 || P <= 0) return MSAT_EINVAL;
-    if (B > 0 && (!bank || !problem_idx || !keys || !state)) return MSAT_EINVAL;
-    if (!aligned(bank, 128) || !aligned(state, 16) || !aligned(obs, 16)) return MSAT_EALIGN;
-    EnvArgs a{};
-    a.bank = static_cast<const uint8_t*>(bank); a.P = P;
-    a.state_out = state; a.prob_idx = problem_idx; a.keys = keys; a.obs = obs; a.B = B;
+    EnvArgs a;
+    if (const int rc = env_args(a, plan, bank, P, nullptr, state, obs, B, !problem_idx || !keys || !state)) return rc;
+    a.prob_idx = problem_idx; a.keys = keys;
     return cuda_rc(launch_env(plan, MODE_RESET, a, (cudaStream_t)stream));
 }
 
 int msat_import_state(const msat_plan* plan, const void* bank, int32_t P, const int32_t* problem_idx,
                       const int32_t* variable_assignments, const int32_t* step, const uint8_t* done, uint32_t* state_out,
                       int32_t* obs, int32_t B, void* stream) {
-    if (!plan || B < 0 || P <= 0) return MSAT_EINVAL;
-    if (B > 0 && (!bank || !problem_idx || !variable_assignments || !state_out)) return MSAT_EINVAL;
-    if (!aligned(bank, 128) || !aligned(state_out, 16) || !aligned(obs, 16)) return MSAT_EALIGN;
-    EnvArgs a{};
-    a.bank = static_cast<const uint8_t*>(bank); a.P = P;
-    a.state_out = state_out; a.prob_idx = problem_idx; a.obs = obs; a.B = B;
-    a.assign_in = variable_assignments; a.step_in = step; a.done_in = done;
+    EnvArgs a;
+    if (const int rc = env_args(a, plan, bank, P, nullptr, state_out, obs, B,
+                                !problem_idx || !variable_assignments || !state_out))
+        return rc;
+    a.prob_idx = problem_idx; a.assign_in = variable_assignments; a.step_in = step; a.done_in = done;
     return cuda_rc(launch_env(plan, MODE_IMPORT, a, (cudaStream_t)stream));
 }
 
@@ -301,26 +386,21 @@ int msat_apply_start_states(const msat_plan* plan, const void* bank, int32_t P, 
                             const uint32_t* reset_key, int32_t Bg, int32_t env_offset, const uint32_t* start_words,
                             const uint32_t* flip_thr, const uint8_t* has_start, int32_t* obs, int32_t* gnn_assignment,
                             float* gnn_clause_features, int32_t B, void* stream) {
-    if (!plan || B < 0 || Bg < 0 || env_offset < 0 || P <= 0 || (long long)env_offset + B > Bg) return MSAT_EINVAL;
-    if (B > 0 && (!bank || !state || !reset_key || !start_words || !flip_thr)) return MSAT_EINVAL;
-    if (!aligned(bank, 128) || !aligned(state, 16) || !aligned(obs, 16) || !aligned(start_words, 4) ||
-        !aligned(flip_thr, 4) || !aligned(gnn_assignment, 4) || !aligned(gnn_clause_features, 4))
+    EnvArgs a;
+    int rc = env_args(a, plan, bank, P, state, state, obs, B, !state || !reset_key || !start_words || !flip_thr);
+    if (rc == MSAT_OK) rc = shard_rule(Bg, env_offset, B);
+    if (rc != MSAT_OK) return rc;
+    if (!aligned(start_words, 4) || !aligned(flip_thr, 4) || !aligned(gnn_assignment, 4) ||
+        !aligned(gnn_clause_features, 4))
         return MSAT_EALIGN;
-    if (Bg > (1 << 30)) return MSAT_EUNSUPPORTED;
-    if (gnn_clause_features && plan->d.k > 15) return MSAT_EUNSUPPORTED;   // 16-entry feature table
+    if (clause_features_unsupported(plan, gnn_clause_features)) return MSAT_EUNSUPPORTED;
     if (B == 0) return MSAT_OK;
-    EnvArgs a{};
-    a.bank = static_cast<const uint8_t*>(bank); a.P = P;
-    a.state_in = state; a.state_out = state; a.B = B;
     a.Bg = (uint32_t)Bg; a.env_off = (uint32_t)env_offset; a.reset_key = reset_key;
     a.start_words = start_words; a.flip_thr = flip_thr; a.has_start = has_start;
     // observations and GNN inputs come from differently shaped launches; the rewrite depends only on the key and
     // the tables, so the second launch selects the same envs and writes the same states again
     cudaError_t e = cudaSuccess;
-    if (obs || !(gnn_assignment || gnn_clause_features)) {
-        a.obs = obs;
-        e = launch_env(plan, MODE_START, a, (cudaStream_t)stream);
-    }
+    if (obs || !(gnn_assignment || gnn_clause_features)) e = launch_env(plan, MODE_START, a, (cudaStream_t)stream);
     if (e == cudaSuccess && (gnn_assignment || gnn_clause_features)) {
         a.obs = nullptr; a.gnn_assign = gnn_assignment; a.gnn_cf = gnn_clause_features;
         e = launch_env(plan, MODE_START, a, (cudaStream_t)stream);
@@ -331,10 +411,9 @@ int msat_apply_start_states(const msat_plan* plan, const void* bank, int32_t P, 
 int msat_walksat(const msat_plan* plan, const void* bank, int32_t P, uint32_t* state, const uint32_t* keys,
                  int32_t max_flips, int32_t flip_offset, double noise, uint8_t* solved, int32_t* flips, int32_t B,
                  void* stream) {
-    if (!plan || B < 0 || P <= 0) return MSAT_EINVAL;
+    if (bad_env_call(plan, bank, P, B, !state || !keys)) return MSAT_EINVAL;
     if (!(noise >= 0.0 && noise <= 1.0)) return MSAT_EINVAL;          // also NaN
     if (max_flips < 0 || flip_offset < 0 || (long long)flip_offset + max_flips > 2147483647LL) return MSAT_EINVAL;
-    if (B > 0 && (!bank || !state || !keys)) return MSAT_EINVAL;
     if (!aligned(bank, 128) || !aligned(state, 16)) return MSAT_EALIGN;
     if (walksat_warps(plan->d) == 0) return MSAT_EUNSUPPORTED;
     WalksatArgs a{};
@@ -349,63 +428,13 @@ int msat_step(const msat_plan* plan, const void* bank, int32_t P, const uint32_t
               const int32_t* actions, int32_t auto_reset, const int32_t* new_problem_idx, const uint32_t* reset_keys,
               int32_t* obs, float* reward, int32_t reward_cols, uint8_t* done, int32_t done_cols, uint8_t* solved,
               int32_t* num_unsatisfied, int32_t* episode_step, int32_t* newly_satisfied, int32_t B, void* stream) {
-    if (!plan || B < 0 || P <= 0 || (done && done_cols <= 0) || (reward && reward_cols <= 0)) return MSAT_EINVAL;
-    if (B > 0 && (!bank || !state_in || !state_out || !actions)) return MSAT_EINVAL;
-    if (auto_reset && B > 0 && (!new_problem_idx || !reset_keys)) return MSAT_EINVAL;
-    if (newly_satisfied && plan->reward_mode != MSAT_REWARD_SHAPED) return MSAT_EINVAL;
-    if (!aligned(bank, 128) || !aligned(state_in, 16) || !aligned(state_out, 16) || !aligned(obs, 16))
-        return MSAT_EALIGN;
-    EnvArgs a{};
-    a.bank = static_cast<const uint8_t*>(bank); a.P = P;
-    a.state_in = state_in; a.state_out = state_out; a.actions = actions;
-    a.auto_reset = auto_reset ? 1 : 0; a.prob_idx = new_problem_idx; a.keys = reset_keys;
-    a.obs = obs; a.reward = reward; a.reward_cols = reward_cols; a.done = done; a.done_cols = done_cols;
-    a.solved = solved;
-    a.num_unsat = num_unsatisfied; a.episode_step = episode_step; a.B = B;
-    fill_reward(a, plan, newly_satisfied);
-    return cuda_rc(launch_env(plan, MODE_STEP, a, (cudaStream_t)stream));
-}
-
-// Shared body of the fused rollout entry points: K >= 1 steps per launch, local observations or GNN inputs.
-static int rollout_launch(const msat_plan* plan, const void* bank, int32_t P, const uint32_t* state_in,
-                          uint32_t* state_out, const int32_t* actions, int32_t K, const uint32_t* rng_in,
-                          uint32_t* chain_out, int32_t Bg, int32_t env_offset, int32_t* obs, int32_t* gnn_assignment,
-                          float* gnn_clause_features, int32_t emit_every_step, float* reward, int32_t reward_cols,
-                          uint8_t* done, int32_t done_cols, uint8_t* solved, int32_t* num_unsatisfied,
-                          int32_t* episode_step, int32_t* newly_satisfied, int32_t B, void* stream) {
-    if (!plan || B < 0 || P <= 0 || (done && done_cols <= 0) || (reward && reward_cols <= 0)) return MSAT_EINVAL;
-    if (K < 1 || K > kMaxFusedSteps) return MSAT_EINVAL;
-    if (!rng_in || !chain_out || Bg <= 0 || env_offset < 0 || (long long)env_offset + B > Bg) return MSAT_EINVAL;
-    if (Bg > (1 << 30)) return MSAT_EUNSUPPORTED;
-    if (newly_satisfied && plan->reward_mode != MSAT_REWARD_SHAPED) return MSAT_EINVAL;
-    if (gnn_clause_features && plan->d.k > 15) return MSAT_EUNSUPPORTED;   // 16-entry feature table
-    {   // the advanced chain is written while other CTAs still read rng_in: the buffers must not overlap
-        const uintptr_t r = reinterpret_cast<uintptr_t>(rng_in), c = reinterpret_cast<uintptr_t>(chain_out);
-        if (r + 8 > c && c + 40 > r) return MSAT_EINVAL;
-    }
-    if (B > 0 && (!bank || !state_in || !state_out || !actions)) return MSAT_EINVAL;
-    if (!aligned(bank, 128) || !aligned(state_in, 16) || !aligned(state_out, 16) || !aligned(obs, 16))
-        return MSAT_EALIGN;
-    const Dims& d = plan->d;
-    EnvArgs a{};
-    a.bank = static_cast<const uint8_t*>(bank); a.P = P;
-    a.state_in = state_in; a.state_out = state_out; a.actions = actions;
-    a.auto_reset = 1; a.rng_in = rng_in; a.chain_out = chain_out; a.Bg = (uint32_t)Bg; a.env_off = (uint32_t)env_offset;
-    a.obs = obs; a.gnn_assign = gnn_assignment; a.gnn_cf = gnn_clause_features;
-    a.reward = reward; a.reward_cols = reward_cols; a.done = done; a.done_cols = done_cols;
-    a.solved = solved;
-    a.num_unsat = num_unsatisfied; a.episode_step = episode_step; a.B = B;
-    a.num_steps = K;
-    a.act_step_stride = (long long)B * d.A * (d.action_mode == 0 ? 1 : d.V);
-    a.emit_every_step = emit_every_step ? 1 : 0;
-    fill_reward(a, plan, newly_satisfied);
-    if (B == 0) {
-        // an empty shard still advances the chain K times
-        cudaError_t e = cudaSuccess;
-        for (int j = 0; j < K && e == cudaSuccess; ++j)
-            e = launch_rng_chain(j == 0 ? rng_in : chain_out, chain_out, (cudaStream_t)stream);
-        return cuda_rc(e);
-    }
+    EnvArgs a;
+    int rc = env_args(a, plan, bank, P, state_in, state_out, obs, B,
+                      !state_in || !state_out || !actions || (auto_reset && (!new_problem_idx || !reset_keys)));
+    if (rc == MSAT_OK) rc = step_outputs(a, plan, reward, reward_cols, done, done_cols, solved, num_unsatisfied,
+                                         episode_step, newly_satisfied);
+    if (rc != MSAT_OK) return rc;
+    a.actions = actions; a.auto_reset = auto_reset ? 1 : 0; a.prob_idx = new_problem_idx; a.keys = reset_keys;
     return cuda_rc(launch_env(plan, MODE_STEP, a, (cudaStream_t)stream));
 }
 
@@ -414,9 +443,9 @@ int msat_rollout_step(const msat_plan* plan, const void* bank, int32_t P, const 
                       int32_t Bg, int32_t env_offset, int32_t* obs, float* reward, int32_t reward_cols, uint8_t* done,
                       int32_t done_cols, uint8_t* solved, int32_t* num_unsatisfied, int32_t* episode_step, int32_t B,
                       void* stream) {
-    return rollout_launch(plan, bank, P, state_in, state_out, actions, 1, rng_in, chain_out, Bg, env_offset, obs,
-                          nullptr, nullptr, 0, reward, reward_cols, done, done_cols, solved, num_unsatisfied,
-                          episode_step, nullptr, B, stream);
+    return msat_rollout_steps(plan, bank, P, state_in, state_out, actions, 1, rng_in, chain_out, Bg, env_offset, obs,
+                              nullptr, nullptr, 0, reward, reward_cols, done, done_cols, solved, num_unsatisfied,
+                              episode_step, nullptr, B, stream);
 }
 
 int msat_rollout_step_gnn(const msat_plan* plan, const void* bank, int32_t P, const uint32_t* state_in,
@@ -424,9 +453,9 @@ int msat_rollout_step_gnn(const msat_plan* plan, const void* bank, int32_t P, co
                           int32_t Bg, int32_t env_offset, int32_t* assignment, float* clause_features, float* reward,
                           int32_t reward_cols, uint8_t* done, int32_t done_cols, uint8_t* solved,
                           int32_t* num_unsatisfied, int32_t* episode_step, int32_t B, void* stream) {
-    return rollout_launch(plan, bank, P, state_in, state_out, actions, 1, rng_in, chain_out, Bg, env_offset, nullptr,
-                          assignment, clause_features, 0, reward, reward_cols, done, done_cols, solved,
-                          num_unsatisfied, episode_step, nullptr, B, stream);
+    return msat_rollout_steps(plan, bank, P, state_in, state_out, actions, 1, rng_in, chain_out, Bg, env_offset,
+                              nullptr, assignment, clause_features, 0, reward, reward_cols, done, done_cols, solved,
+                              num_unsatisfied, episode_step, nullptr, B, stream);
 }
 
 int msat_rollout_steps(const msat_plan* plan, const void* bank, int32_t P, const uint32_t* state_in,
@@ -436,20 +465,18 @@ int msat_rollout_steps(const msat_plan* plan, const void* bank, int32_t P, const
                        uint8_t* done, int32_t done_cols, uint8_t* solved, int32_t* num_unsatisfied,
                        int32_t* episode_step, int32_t* newly_satisfied, int32_t B, void* stream) {
     if (obs && (gnn_assignment || gnn_clause_features)) return MSAT_EINVAL;   // one kind of policy input per launch
-    return rollout_launch(plan, bank, P, state_in, state_out, actions, num_steps, rng_in, chain_out, Bg, env_offset,
-                          obs, gnn_assignment, gnn_clause_features, emit_every_step, reward, reward_cols, done,
-                          done_cols, solved, num_unsatisfied, episode_step, newly_satisfied, B, stream);
+    EnvArgs a;
+    const int rc = rollout_args(a, plan, bank, P, state_in, state_out, actions, num_steps, rng_in, chain_out, Bg,
+                                env_offset, obs, gnn_assignment, gnn_clause_features, emit_every_step, reward,
+                                reward_cols, done, done_cols, solved, num_unsatisfied, episode_step, newly_satisfied, B);
+    return rc != MSAT_OK ? rc : cuda_rc(rollout_enqueue(plan, a, (cudaStream_t)stream));
 }
 
 int msat_get_obs(const msat_plan* plan, const void* bank, int32_t P, const uint32_t* state, int32_t* obs, int32_t B,
                  void* stream) {
-    if (!plan || B < 0 || P <= 0) return MSAT_EINVAL;
-    if (B > 0 && (!bank || !state || !obs)) return MSAT_EINVAL;
-    if (!aligned(bank, 128) || !aligned(state, 16) || !aligned(obs, 16)) return MSAT_EALIGN;
-    EnvArgs a{};
-    a.bank = static_cast<const uint8_t*>(bank); a.P = P;
-    a.state_in = state; a.obs = obs; a.B = B;
-    return cuda_rc(launch_env(plan, MODE_OBS, a, (cudaStream_t)stream));
+    EnvArgs a;
+    const int rc = env_args(a, plan, bank, P, state, nullptr, obs, B, !state || !obs);
+    return rc != MSAT_OK ? rc : cuda_rc(launch_env(plan, MODE_OBS, a, (cudaStream_t)stream));
 }
 
 int msat_export_state(const msat_plan* plan, const void* bank, int32_t P, const uint32_t* state, int32_t B,
@@ -457,8 +484,7 @@ int msat_export_state(const msat_plan* plan, const void* bank, int32_t P, const 
                       int32_t* step, uint8_t* done, int32_t* clauses, int32_t* agent_clause_masks,
                       int32_t* agent_neighbor_masks, int32_t* literal_to_agent_idx, int32_t* problem_idx,
                       void* stream) {
-    if (!plan || B < 0 || P <= 0) return MSAT_EINVAL;
-    if (B > 0 && (!bank || !state)) return MSAT_EINVAL;
+    if (bad_env_call(plan, bank, P, B, !state)) return MSAT_EINVAL;
     ExportArgs a{};
     a.bank = static_cast<const uint8_t*>(bank); a.P = P; a.state = state; a.B = B;
     a.assign = variable_assignments; a.sat = clauses_satisfied_status; a.num_unsat = num_unsatisfied;
@@ -474,67 +500,48 @@ int msat_rollout_step_host(const msat_plan* plan, const void* bank, int32_t P, u
                            int32_t* num_unsatisfied_dev, int32_t* episode_step_dev, float* reward_host,
                            uint8_t* done_host, uint8_t* solved_host, int32_t* num_unsatisfied_host,
                            int32_t* episode_step_host, int32_t B, void* stream) {
-    if (!plan || !actions_host || !actions_dev || B < 0) return MSAT_EINVAL;
+    HostStep h{plan, actions_host, actions_dev, reward_host, done_host, solved_host, num_unsatisfied_host,
+               episode_step_host};
+    if (const int rc = h.check(bank, P, state, rng_in, chain_out, Bg, env_offset, obs_dev, reward_dev, reward_cols,
+                               done_dev, done_cols, solved_dev, num_unsatisfied_dev, episode_step_dev, B))
+        return rc;
     cudaStream_t s = (cudaStream_t)stream;
-    const Dims& d = plan->d;
-    const size_t act_per_env = (size_t)d.A * (d.action_mode == 0 ? 1 : d.V);
-    const size_t obs_env_bytes = (size_t)d.A * d.D * (plan->obs_i8 ? 1u : 4u);   // int8 plans: one byte per element
-    const ResultBufs rb{reward_dev, reward_cols, done_dev, done_cols, solved_dev, num_unsatisfied_dev, episode_step_dev,
-                        reward_host, done_host, solved_host, num_unsatisfied_host, episode_step_host};
-
-    // One slice [b0, b0 + bc) of the batch on stream `w`: actions in, fused step, results out.
-    auto run_slice = [&](int b0, int bc, cudaStream_t w) -> int {
-        cudaError_t e = cudaSuccess;
-        if (bc > 0 && act_per_env)
-            e = cudaMemcpyAsync(actions_dev + b0 * act_per_env, actions_host + b0 * act_per_env,
-                                (size_t)bc * act_per_env * sizeof(int32_t), cudaMemcpyHostToDevice, w);
-        if (e != cudaSuccess) return (int)e;
-        uint32_t* st = state + (size_t)b0 * d.state_words;
-        int rc = msat_rollout_step(plan, bank, P, st, st, actions_dev + b0 * act_per_env, rng_in, chain_out, Bg,
-                                   env_offset + b0,
-                                   obs_dev ? reinterpret_cast<int32_t*>(reinterpret_cast<char*>(obs_dev) + b0 * obs_env_bytes)
-                                           : nullptr,
-                                   reward_dev ? reward_dev + (size_t)b0 * reward_cols : nullptr, reward_cols,
-                                   done_dev ? done_dev + (size_t)b0 * done_cols : nullptr, done_cols,
-                                   solved_dev ? solved_dev + b0 : nullptr,
-                                   num_unsatisfied_dev ? num_unsatisfied_dev + b0 : nullptr,
-                                   episode_step_dev ? episode_step_dev + b0 : nullptr, bc, (void*)w);
-        if (rc != MSAT_OK || bc == 0) return rc;
-        return (int)copy_results(rb, b0, bc, w);
+    auto run_slice = [&](int b0, int bc, cudaStream_t w) {
+        cudaError_t e = h.upload(b0, bc, w);
+        if (e == cudaSuccess) e = h.step(b0, bc, w);
+        if (e == cudaSuccess) e = h.download(b0, bc, w);
+        return e;
     };
-
     constexpr int kSlices = 4;
     if (B < 32768) {   // one slice on the caller's stream (slicing only pays when the kernel is long)
-        int rc = run_slice(0, B, s);
-        if (rc != MSAT_OK) return rc;
-        return cuda_rc(cudaStreamSynchronize(s));
+        const cudaError_t e = run_slice(0, B, s);
+        return cuda_rc(e != cudaSuccess ? e : cudaStreamSynchronize(s));
     }
     // Large batch: slices alternate between two internal streams so that the action upload of slice
     // i+1 and the result download of slice i-1 overlap the kernel of slice i (separate copy engines).
-    int rc = MSAT_OK;
+    cudaError_t e = cudaSuccess;
     {
         std::lock_guard<std::mutex> lock(g_pipe_mu);
         SyncPipe* pipe = nullptr;
-        cudaError_t e = sync_pipe_for_current_device(&pipe);
-        if (e != cudaSuccess) return (int)e;
-        e = cudaEventRecord(pipe->fork, s);
+        e = sync_pipe_for_current_device(&pipe);
+        if (e == cudaSuccess) e = cudaEventRecord(pipe->fork, s);
         for (int w = 0; w < 2 && e == cudaSuccess; ++w) e = cudaStreamWaitEvent(pipe->ws[w], pipe->fork, 0);
         if (e != cudaSuccess) return (int)e;
         const int per = (((B + kSlices - 1) / kSlices) + 63) & ~63;   // multiple of 64 envs keeps every slice aligned
-        for (int c = 0, b0 = 0; b0 < B && rc == MSAT_OK; ++c, b0 += per) {
+        for (int c = 0, b0 = 0; b0 < B && e == cudaSuccess; ++c, b0 += per) {
             const int bc = B - b0 < per ? B - b0 : per;
-            rc = run_slice(b0, bc, pipe->ws[c & 1]);
+            e = run_slice(b0, bc, pipe->ws[c & 1]);
         }
         // always join the internal streams back into the caller's stream -- also after a failed slice, so that
         // nothing enqueued so far is still running when the caller sees the error
         for (int w = 0; w < 2; ++w) {
             cudaError_t j = cudaEventRecord(pipe->join[w], pipe->ws[w]);
             if (j == cudaSuccess) j = cudaStreamWaitEvent(s, pipe->join[w], 0);
-            if (j != cudaSuccess && rc == MSAT_OK) rc = (int)j;
+            if (j != cudaSuccess && e == cudaSuccess) e = j;
         }
     }
     const cudaError_t se = cudaStreamSynchronize(s);
-    return rc != MSAT_OK ? rc : cuda_rc(se);
+    return cuda_rc(e != cudaSuccess ? e : se);
 }
 
 // ---- asynchronous host pipeline (double-buffered host I/O) -------------------------------------------------
@@ -586,36 +593,30 @@ int msat_rollout_step_host_async(msat_host_pipe* pipe, int32_t slot, const msat_
                                  int32_t* episode_step_dev, float* reward_host, uint8_t* done_host,
                                  uint8_t* solved_host, int32_t* num_unsatisfied_host, int32_t* episode_step_host,
                                  int32_t B, void* stream) {
-    if (!pipe || slot < 0 || slot >= pipe->depth || !plan || !actions_host || !actions_dev || B < 0) return MSAT_EINVAL;
+    if (!pipe || slot < 0 || slot >= pipe->depth) return MSAT_EINVAL;
+    HostStep h{plan, actions_host, actions_dev, reward_host, done_host, solved_host, num_unsatisfied_host,
+               episode_step_host};
+    if (const int rc = h.check(bank, P, state, rng_in, chain_out, Bg, env_offset, obs_dev, reward_dev, reward_cols,
+                               done_dev, done_cols, solved_dev, num_unsatisfied_dev, episode_step_dev, B))
+        return rc;
     cudaStream_t s = (cudaStream_t)stream;
-    const Dims& d = plan->d;
-    const size_t act_bytes = (size_t)B * d.A * (d.action_mode == 0 ? 1 : d.V) * sizeof(int32_t);
     cudaError_t e = cudaSuccess;
     // 1. upload this step's actions on the copy-in stream as soon as the kernel that last read this slot's
     //    device staging buffer has finished (it overlaps the kernels of the steps in between)
     if (pipe->kernel_valid[slot]) e = cudaStreamWaitEvent(pipe->s_in, pipe->ev_kernel[slot], 0);
-    if (e == cudaSuccess && act_bytes)
-        e = cudaMemcpyAsync(actions_dev, actions_host, act_bytes, cudaMemcpyHostToDevice, pipe->s_in);
+    if (e == cudaSuccess) e = h.upload(0, B, pipe->s_in);
     if (e == cudaSuccess) e = cudaEventRecord(pipe->ev_h2d[slot], pipe->s_in);
     // 2. the fused step on the caller's stream: after the upload, and after the previous download out of
     //    this slot's device result buffers
     if (e == cudaSuccess) e = cudaStreamWaitEvent(s, pipe->ev_h2d[slot], 0);
     if (e == cudaSuccess && pipe->d2h_valid[slot]) e = cudaStreamWaitEvent(s, pipe->ev_d2h[slot], 0);
+    if (e == cudaSuccess) e = h.step(0, B, s);
     if (e != cudaSuccess) return (int)e;
-    int rc = msat_rollout_step(plan, bank, P, state, state, actions_dev, rng_in, chain_out, Bg, env_offset, obs_dev,
-                               reward_dev, reward_cols, done_dev, done_cols, solved_dev, num_unsatisfied_dev,
-                               episode_step_dev, B, stream);
-    if (rc != MSAT_OK) return rc;
     e = cudaEventRecord(pipe->ev_kernel[slot], s);
     pipe->kernel_valid[slot] = e == cudaSuccess;
     // 3. results to the host on the copy-out stream; msat_host_wait(slot) blocks on ev_d2h
     if (e == cudaSuccess) e = cudaStreamWaitEvent(pipe->s_out, pipe->ev_kernel[slot], 0);
-    if (e == cudaSuccess && B > 0) {
-        const ResultBufs rb{reward_dev, reward_cols, done_dev, done_cols, solved_dev, num_unsatisfied_dev,
-                            episode_step_dev, reward_host, done_host, solved_host, num_unsatisfied_host,
-                            episode_step_host};
-        e = copy_results(rb, 0, B, pipe->s_out);
-    }
+    if (e == cudaSuccess) e = h.download(0, B, pipe->s_out);
     if (e == cudaSuccess) e = cudaEventRecord(pipe->ev_d2h[slot], pipe->s_out);
     pipe->d2h_valid[slot] = e == cudaSuccess;
     return cuda_rc(e);
@@ -652,10 +653,9 @@ int msat_rng_split2(const uint32_t* key_in, uint32_t* out, void* stream) {
 
 int msat_env_keys(const uint32_t* prob_key, const uint32_t* reset_key, int32_t Bg, int32_t off, int32_t Bl, int32_t P,
                   int32_t* problem_idx, uint32_t* reset_keys, void* stream) {
-    if (Bg < 0 || off < 0 || Bl < 0 || (long long)off + Bl > Bg) return MSAT_EINVAL;
+    if (const int rc = shard_rule(Bg, off, Bl)) return rc;
     if (problem_idx && (!prob_key || P <= 0)) return MSAT_EINVAL;
     if (reset_keys && !reset_key) return MSAT_EINVAL;
-    if (Bg > (1 << 30)) return MSAT_EUNSUPPORTED;
     return cuda_rc(launch_env_keys(prob_key, reset_key, Bg, off, Bl, P, problem_idx, reset_keys, nullptr,
                                    (cudaStream_t)stream));
 }
@@ -663,11 +663,10 @@ int msat_env_keys(const uint32_t* prob_key, const uint32_t* reset_key, int32_t B
 int msat_env_keys_weighted(const uint32_t* prob_key, const uint32_t* reset_key, int32_t Bg, int32_t off, int32_t Bl,
                            const int64_t* cum_weights, int32_t P, int32_t* problem_idx, uint32_t* reset_keys,
                            void* stream) {
-    if (Bg < 0 || off < 0 || Bl < 0 || (long long)off + Bl > Bg) return MSAT_EINVAL;
+    if (const int rc = shard_rule(Bg, off, Bl)) return rc;
     if (problem_idx && (!prob_key || !cum_weights || P <= 0)) return MSAT_EINVAL;
     if (reset_keys && !reset_key) return MSAT_EINVAL;
     if (!aligned(cum_weights, 8)) return MSAT_EALIGN;
-    if (Bg > (1 << 30)) return MSAT_EUNSUPPORTED;
     // without problem indices to draw, the call is msat_env_keys' reset-key half
     const long long* cum = problem_idx ? reinterpret_cast<const long long*>(cum_weights) : nullptr;
     return cuda_rc(launch_env_keys(prob_key, reset_key, Bg, off, Bl, P, problem_idx, reset_keys, cum,
@@ -729,7 +728,7 @@ int msat_gnn_static(const msat_plan* plan, const void* bank, int32_t P, float* s
 
 int msat_gnn_dynamic(const msat_plan* plan, const void* bank, int32_t P, const uint32_t* state, int32_t B,
                      int32_t* assignment, float* clause_features, void* stream) {
-    if (!plan || B < 0 || P <= 0 || (B > 0 && (!bank || !state))) return MSAT_EINVAL;
+    if (bad_env_call(plan, bank, P, B, !state)) return MSAT_EINVAL;
     return cuda_rc(launch_gnn_dynamic(plan, static_cast<const uint8_t*>(bank), P, state, B, assignment,
                                       clause_features, (cudaStream_t)stream));
 }
@@ -745,7 +744,7 @@ int msat_rollout_metrics(const float* reward, int64_t rs_t, int64_t rs_b, const 
 
 int msat_flip_gains(const msat_plan* plan, const void* bank, int32_t P, const uint32_t* state, int32_t B, double tau,
                     int32_t* delta_unsat, int32_t* greedy_labels, void* stream) {
-    if (!plan || B < 0 || P <= 0 || (B > 0 && (!bank || !state))) return MSAT_EINVAL;
+    if (bad_env_call(plan, bank, P, B, !state)) return MSAT_EINVAL;
     if (plan->d.n * (int)sizeof(int) > 48 * 1024) return MSAT_EUNSUPPORTED;
     return cuda_rc(launch_flip_gains(plan, static_cast<const uint8_t*>(bank), P, state, B, (float)tau, delta_unsat,
                                      greedy_labels, (cudaStream_t)stream));
